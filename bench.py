@@ -3,7 +3,7 @@
 workloads of the path as separately labelled lines.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                  [--workload proj|flow|builder|builder_fixed|proj5] [--scene room|iid]
+                  [--workload proj|flow|builder|builder_fixed|proj5] [--scene room|iid] [--dump-outputs DIR]
 
 Default (`--workload proj`, the line the driver reads): one "step" = one pass of the hot path
 (dm_orth_project_f32: fused projection + resolve) over one batch of 64 synthetic 480x640 depth frames
@@ -22,6 +22,8 @@ Other workloads (BASELINE.json configs 3, 4, 5; `--workload X` makes one of them
   proj5_job      config 5 as a job: 4096 / N frames per rank streamed from host memory in 64-frame chunks (class ids)
 N > 1: one process per GPU (torchrun; `python bench.py --gpus N` on its own re-launches itself that way), every
 rank works on its own environments, no collective on the data path (weak scaling).  Prints ONE JSON line on rank 0.
+--dump-outputs DIR: after the timed steps, rank 0 writes the arrays its last timed step returned as DIR/<name>.npy
+(see dump_outputs); the inputs depend on the arguments only, so two builds can be compared file by file.
 """
 import argparse
 import json
@@ -31,6 +33,8 @@ import subprocess
 import sys
 import threading
 import time
+
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the source tree, which may be read-only
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
@@ -203,6 +207,10 @@ class ProjWorkload:
     self.last = (depth, values, ids, pose)
     return self.out
 
+  def outputs(self):
+    top, mask, hgt = self.out
+    return {"topdown": top, "mask": mask, "height": hgt}
+
   def e2e_setup(self, float32=False):
     """Host-buffer leg.  Default: semantics as uint8 class ids (what a segmentation network emits and what the
     reference's object-map demo starts from, demos/object_map/run.py:117-124); float32=True: the one-hot float32
@@ -328,6 +336,9 @@ class FlowWorkload:
     self.t += 1
     return self.out
 
+  def outputs(self):
+    return {"grid": self.out}
+
   def e2e_setup(self):
     self.h_depth = self.depth.cpu().pin_memory()
     self.o_grid = torch.empty((self.B, 1, self.H, self.W, 2), dtype=torch.float32).pin_memory()
@@ -448,8 +459,14 @@ class BuilderWorkload:
       self.algo_bytes_total += 5 * (n_before + cells(local)) + 5 * cells(after)
     self.world_shape = list(after.mask.shape)
     self.t += 1
-    self.out = after
+    self.out, self.local = after, local
     return after
+
+  def outputs(self):
+    """The local map MapBuilder.step returned and the world map it merged that map into (height maps: C = 0)."""
+    w, l = self.out, self.local
+    return {"world_height": w.topdown_map, "world_mask": w.mask, "world_width_offset": w.proj.width_offset,
+            "world_height_offset": w.proj.height_offset, "local_height": l.topdown_map, "local_mask": l.mask}
 
   def reset_counters(self):
     self.algo_bytes_total = 0
@@ -588,6 +605,38 @@ def make_workload(args, key=None):
 
 # ================================================================================================
 
+DUMP_BYTES = 48 << 20  # all files of one --dump-outputs directory together
+
+
+def dump_positions(numel: int, k: int) -> np.ndarray:
+  """Sorted distinct flat positions, at most k of numel, of a dumped sample: seeded, so the same for the same shape."""
+  return np.unique(np.random.default_rng(0).integers(0, numel, size=k))
+
+
+def dump_outputs(arrays: dict, out_dir: str) -> None:
+  """Writes every array as out_dir/<name>.npy, float64 as float64 and anything else as float32 (masks as 0 / 1), with
+  finite numbers only: a floating-point array also gets out_dir/<name>_nonfinite.npy (0 finite, 1 +inf, -1 -inf,
+  2 NaN) and holds 0 where that is not 0, so the -inf fill of unobserved map cells and NaNs survive the dump.  An
+  array larger than its share of DUMP_BYTES is written as the 1-D sample of its flattened (row-major) elements at
+  dump_positions(numel, k)."""
+  os.makedirs(out_dir, exist_ok=True)
+  tensors = {name: torch.as_tensor(x).detach() for name, x in arrays.items()}
+  share = DUMP_BYTES // sum(2 if t.is_floating_point() else 1 for t in tensors.values())
+  for name, t in tensors.items():
+    floating = t.is_floating_point()
+    dtype = torch.float64 if t.dtype == torch.float64 else torch.float32
+    k = share // dtype.itemsize
+    if t.numel() > k:
+      t = t.reshape(-1)[torch.from_numpy(dump_positions(t.numel(), k)).to(t.device)]
+    t = t.to(dtype)
+    if floating:
+      flag = torch.zeros_like(t).masked_fill_(t == math.inf, 1).masked_fill_(t == -math.inf, -1)
+      flag.masked_fill_(t.isnan(), 2)
+      np.save(os.path.join(out_dir, name + "_nonfinite.npy"), flag.float().cpu().numpy())
+      t = t.masked_fill(flag != 0, 0)
+    np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+
+
 _RESULT_LINE = []
 
 
@@ -641,10 +690,7 @@ def run_reference(args):
     setup(threads)
     for _ in range(max(min(args.warmup, 3), 1)):
       wl.cpu_fn()
-    t0 = time.perf_counter()
-    wl.cpu_fn()
-    one = time.perf_counter() - t0
-    steps = max(3, min(args.steps, int(60.0 / max(one, 1e-3))))  # keep the whole run within minutes
+    steps = args.steps
     t0 = time.perf_counter()
     for _ in range(steps):
       wl.cpu_fn()
@@ -838,6 +884,8 @@ def run_ours(args):
   value = world * wl.units_per_step * args.steps / (ms_total * 1e-3)
   total_launches = int(sum_over_ranks(float(launches)))
   algo_bytes = wl.algo_bytes_total / args.steps if isinstance(wl, BuilderWorkload) else wl.algo_bytes_per_step
+  if args.dump_outputs and rank == 0:
+    dump_outputs(wl.outputs(), args.dump_outputs)
 
   # ---- e2e: HOST buffers through the public entry, copies inside the timed region
   # cheap steps (a MapBuilder step is < 1 ms) are timed over more of them: five would be one hiccup away from noise
@@ -927,7 +975,14 @@ def main():
   ap.add_argument("--e2e-steps", type=int, default=5)
   ap.add_argument("--no-cpu-baseline", action="store_true")
   ap.add_argument("--no-extra", action="store_true", help="skip the `extra` legs (other configs) of the default line")
+  ap.add_argument("--dump-outputs", metavar="DIR",
+                  help=f"write what the last timed step returned as DIR/<name>.npy (float32 / float64, at most "
+                       f"{DUMP_BYTES >> 20} MiB in all: larger outputs as a fixed seeded sample of their elements)")
   args = ap.parse_args()
+  if args.steps < 1:
+    ap.error("--steps must be at least 1")
+  if args.dump_outputs and args.impl != "ours":
+    ap.error("--dump-outputs writes the outputs of --impl ours")
   if args.gpus > 1 and args.impl == "ours" and "WORLD_SIZE" not in os.environ:
     # called directly with --gpus N: become the torchrun launch the driver would have made (one rank per GPU)
     import socket
