@@ -79,6 +79,11 @@ class DmMapRef(ctypes.Structure):
               ("width_offset", c_float), ("height_offset", c_float), ("box", c_void_p), ("plane_box", c_void_p)]
 
 
+class DmValueMapRef(ctypes.Structure):
+  _fields_ = [("topdown", c_void_p), ("height", c_void_p), ("mask", c_void_p), ("h", c_int32), ("w", c_int32),
+              ("width_offset", c_float), ("height_offset", c_float), ("box", c_void_p), ("plane_box", c_void_p)]
+
+
 class DmMergeShape(ctypes.Structure):
   _fields_ = [("n_valid", c_int64), ("map_height", c_int32), ("map_width", c_int32),
               ("width_offset", c_float), ("height_offset", c_float)]
@@ -135,6 +140,13 @@ _SIGNATURES = {
   "dm_builder_merge": (ctypes.c_int, [c_void_p, POINTER(DmMapRef), c_void_p]),
   "dm_builder_step_fixed": (ctypes.c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                            POINTER(DmMapRef), c_void_p]),
+  "dm_builder_create_values": (ctypes.c_int, [POINTER(DmBuilderCfg), c_int32, c_int32, POINTER(c_void_p)]),
+  "dm_builder_plot_values": (ctypes.c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                            c_void_p, c_void_p, c_void_p, POINTER(DmValueMapRef), POINTER(DmMergeShape),
+                                            c_void_p, c_void_p, c_void_p, c_int64, c_void_p]),
+  "dm_builder_merge_values": (ctypes.c_int, [c_void_p, POINTER(DmValueMapRef), c_void_p]),
+  "dm_builder_step_fixed_values": (ctypes.c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                                  c_void_p, c_void_p, c_void_p, POINTER(DmValueMapRef), c_void_p]),
   "dm_transform_points_f32": (ctypes.c_int, [c_void_p, c_void_p, c_int32, c_int32, c_int64, c_void_p, c_void_p]),
   "dm_image_camera_f32": (ctypes.c_int, [c_void_p, c_int64, c_float, c_float, c_float, c_float, c_int32, c_int32,
                                          c_int32, c_void_p, c_void_p]),

@@ -154,6 +154,7 @@ extern "C" int32_t dm_sizeof_struct(int32_t id) {
     case 8: return sizeof(DmMapRef);
     case 9: return sizeof(DmMergeShape);
     case 10: return sizeof(DmPoseCfg);
+    case 11: return sizeof(DmValueMapRef);
     default: return -1;
   }
 }

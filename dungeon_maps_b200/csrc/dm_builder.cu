@@ -26,7 +26,9 @@ constexpr int kFuseWords = 2 * kStepWords + 2;           // per sample: two step
 using namespace dm;
 
 struct DmBuilder {
-  DmBuilderCfg cfg;
+  DmBuilderCfg cfg;      // value builders: cfg.proj.C channels, want_height set
+  int C = 0;             // 0: height maps (dm_builder_create); >= 1: value maps (dm_builder_create_values)
+  int labels = 0;        // value maps from class ids (dm_orth_project_labels_f32) instead of float planes
   int device = 0;
   DmPoseCfg pose;      // the constants of the yaw / pitch steps, fused as the projection's rotations are
   int fused_fuse = 0;  // DmStep.fused of the local map's local → global step in the merge
@@ -45,6 +47,7 @@ struct DmBuilder {
   int n_src = 0;
   cudaEvent_t ev_bbox = nullptr;     // the bounding box has reached the host
   float* prefilled_top = nullptr;    // canvases dm_builder_plot_prefill filled while the host waited for the box
+  float* prefilled_height = nullptr;  // (value maps: dm_builder_plot_values)
   uint8_t* prefilled_mask = nullptr;
   int64_t prefilled_cells = 0;
 };
@@ -63,17 +66,45 @@ static void builder_free(DmBuilder* h) {
   delete h;
 }
 
+static bool cfg_ok(const DmBuilderCfg* cfg, DmBuilder** out) {
+  if (!cfg || !out || cfg->b <= 0) return false;
+  if (cfg->proj.H <= 0 || cfg->proj.W <= 0 || cfg->proj.Mh <= 0 || cfg->proj.Mw <= 0) return false;
+  return cfg->merge_reduction == 0 || cfg->merge_reduction == 1;
+}
+
+static int builder_create(const DmBuilderCfg* cfg, int C, int labels, int32_t device, DmBuilder** out);
+
 extern "C" int dm_builder_create(const DmBuilderCfg* cfg, int32_t device, DmBuilder** out) {
   DM_TRACE();
-  if (!cfg || !out || cfg->b <= 0 || cfg->proj.C != 0) return DM_EINVAL;
-  if (cfg->proj.H <= 0 || cfg->proj.W <= 0 || cfg->proj.Mh <= 0 || cfg->proj.Mw <= 0) return DM_EINVAL;
-  if (cfg->merge_reduction != 0 && cfg->merge_reduction != 1) return DM_EINVAL;
+  if (!cfg_ok(cfg, out) || cfg->proj.C != 0) return DM_EINVAL;
+  return builder_create(cfg, 0, 0, device, out);
+}
+
+// MapBuilder.step(value_map=) / step(label_map=, num_classes=): the same step for C-channel value maps with their
+// height planes (maps.py:335-349, 2258-2271).  Every argument is checked before the first CUDA call.
+extern "C" int dm_builder_create_values(const DmBuilderCfg* cfg, int32_t labels, int32_t device, DmBuilder** out) {
+  DM_TRACE();
+  if (!cfg_ok(cfg, out) || cfg->proj.C < 1 || (labels && cfg->proj.C > 63)) return DM_EINVAL;
+  if (cfg->proj.reduction != 0 && cfg->proj.reduction != 1) return DM_EINVAL;
+  return builder_create(cfg, cfg->proj.C, labels ? 1 : 0, device, out);
+}
+
+static int builder_create(const DmBuilderCfg* cfg, int C, int labels, int32_t device, DmBuilder** out) {
+  DmProjCfg pc = cfg->proj;
+  pc.want_height = C > 0 ? 1 : 0;  // value maps: the local map's (b, 1, Mh, Mw) height plane too
+  const size_t ws_bytes = labels ? dm_orth_project_labels_workspace_bytes(&pc, cfg->b)
+                                 : dm_orth_project_workspace_bytes(&pc, cfg->b);
+  if (ws_bytes == 0) return DM_EINVAL;
   DmBuilder* h = new (std::nothrow) DmBuilder();
   if (!h) return DM_EINVAL;
   h->cfg = *cfg;
+  h->cfg.proj = pc;
+  h->C = C;
+  h->labels = labels;
   h->device = device;
   const long long n_proj = (long long)cfg->proj.H * cfg->proj.W;            // points one bmm rotates (utils.py:329)
-  const long long n_fuse = (long long)cfg->proj.Mh * cfg->proj.Mw;          // C * h * w points of the local map
+  // C * h * w points of the local map (_fuse_source: local_to_global(pose, C * h * w)); a height map has one plane
+  const long long n_fuse = (long long)(C > 0 ? C : 1) * cfg->proj.Mh * cfg->proj.Mw;
   memset(&h->pose, 0, sizeof(h->pose));
   memcpy(h->pose.pitch_R, cfg->pitch_R, sizeof(cfg->pitch_R));
   memcpy(h->pose.yaw_skew, cfg->yaw_skew, sizeof(cfg->yaw_skew));
@@ -97,8 +128,7 @@ extern "C" int dm_builder_create(const DmBuilderCfg* cfg, int32_t device, DmBuil
   }
   DM_TRY(cudaMalloc(reinterpret_cast<void**>(&h->d_bbox), 5 * sizeof(int64_t)));
   DM_TRY(cudaHostAlloc(reinterpret_cast<void**>(&h->h_bbox), 5 * sizeof(int64_t), cudaHostAllocDefault));
-  h->ws_bytes = dm_orth_project_workspace_bytes(&cfg->proj, cfg->b);
-  if (h->ws_bytes == 0 && rc == DM_OK) rc = DM_EINVAL;
+  h->ws_bytes = ws_bytes;
   DM_TRY(cudaMalloc(&h->ws, h->ws_bytes));
   DM_TRY(cudaMemset(h->ws, 0, h->ws_bytes));
 #undef DM_TRY
@@ -114,8 +144,9 @@ extern "C" void dm_builder_destroy(DmBuilder* h) { builder_free(h); }
 
 // Packs one step's parameter blocks into a pinned slot and queues their upload; returns the slot's device base.
 //   [DmProjSample x b | local fuse params (steps (b,2), woff (b), hoff (b)) | world fuse params (same layout)]
+// world_off: the world map's (width_offset, height_offset), NULL without a world map
 static int upload_params(DmBuilder* h, const float* pose, const float* sin_yaw, const float* cos_yaw,
-                         const DmMapRef* world, cudaStream_t stream, char** d_base, int* fast_steps) {
+                         const float* world_off, cudaStream_t stream, char** d_base, int* fast_steps) {
   const DmBuilderCfg& c = h->cfg;
   const int b = c.b;
   const unsigned slot = h->next++ % kParamSlots;
@@ -150,8 +181,8 @@ static int upload_params(DmBuilder* h, const float* pose, const float* sin_yaw, 
     lhoff[i] = c.height_offset;
     put_step(wsteps + (size_t)i * 2 * kStepWords, DM_STEP_NONE, nullptr, nullptr, 0);
     put_step(wsteps + (size_t)i * 2 * kStepWords + kStepWords, DM_STEP_NONE, nullptr, nullptr, 0);
-    wwoff[i] = world ? world->width_offset : 0.0f;
-    whoff[i] = world ? world->height_offset : 0.0f;
+    wwoff[i] = world_off ? world_off[0] : 0.0f;
+    whoff[i] = world_off ? world_off[1] : 0.0f;
   }
   DM_CUDA_OK(cudaMemcpyAsync(h->d_params[slot], h->h_params[slot], h->param_bytes, cudaMemcpyHostToDevice, stream));
   DM_CUDA_OK(cudaEventRecord(h->ev[slot], stream));
@@ -160,7 +191,11 @@ static int upload_params(DmBuilder* h, const float* pose, const float* sin_yaw, 
   return DM_OK;
 }
 
-static void make_sources(DmBuilder* h, char* d_base, float* local_topdown, uint8_t* local_mask, const DmMapRef* world) {
+// The fuse sources of a step: the old world map (NULL: none) first, then the local map.  A height builder's maps are
+// their own height maps (world->height unused); a value builder's local map has one height plane for all C channels
+// (the stride-0 expand of maps.py:349), its world map C planes of its own (maps.py:2258-2271).
+static void make_sources(DmBuilder* h, char* d_base, float* local_topdown, uint8_t* local_mask, float* local_height,
+                         const DmValueMapRef* world) {
   const DmBuilderCfg& c = h->cfg;
   const int b = c.b;
   float* w = reinterpret_cast<float*>(d_base);
@@ -173,15 +208,27 @@ static void make_sources(DmBuilder* h, char* d_base, float* local_topdown, uint8
   h->n_src = 0;
   if (world) {  // fuse_topdown_maps(world, new): the world map first (maps.py:2471-2508)
     DmFuseSource& s = h->src[h->n_src++];
-    s.height = world->topdown; s.values = nullptr; s.mask = world->mask;
-    s.height_bstride = (int64_t)world->h * world->w; s.height_cstride = s.height_bstride;
+    const int64_t plane = (int64_t)world->h * world->w;
+    if (h->C == 0) {
+      s.height = world->topdown; s.values = nullptr;
+      s.height_bstride = plane; s.height_cstride = plane;
+    } else {
+      s.height = world->height; s.values = world->topdown;
+      s.height_bstride = plane * h->C; s.height_cstride = plane;
+    }
+    s.mask = world->mask;
     s.h = world->h; s.w = world->w; s.flip_h = c.proj.flip_h; s.map_res = c.proj.map_res;
     s.width_offset = wwoff; s.height_offset = whoff; s.steps = reinterpret_cast<const DmStep*>(wsteps);
     s.plane_box = world->plane_box;
   }
   DmFuseSource& s = h->src[h->n_src++];
-  s.height = local_topdown; s.values = nullptr; s.mask = local_mask;
-  s.height_bstride = (int64_t)c.proj.Mh * c.proj.Mw; s.height_cstride = s.height_bstride;
+  s.mask = local_mask;
+  s.height_bstride = (int64_t)c.proj.Mh * c.proj.Mw;
+  if (h->C == 0) {
+    s.height = local_topdown; s.values = nullptr; s.height_cstride = s.height_bstride;
+  } else {
+    s.height = local_height; s.values = local_topdown; s.height_cstride = 0;
+  }
   s.h = c.proj.Mh; s.w = c.proj.Mw; s.flip_h = c.proj.flip_h; s.map_res = c.proj.map_res;
   s.width_offset = lwoff; s.height_offset = lhoff; s.steps = reinterpret_cast<const DmStep*>(lsteps);
   s.plane_box = nullptr;
@@ -206,17 +253,24 @@ extern "C" int dm_builder_plot_prefill(DmBuilder* h, const float* depth, const f
                                        const DmMapRef* world, DmMergeShape* shape, float* prefill_topdown,
                                        uint8_t* prefill_mask, int64_t prefill_cells, void* stream_) {
   DM_TRACE();
-  if (!h || !depth || !pose || !sin_yaw || !cos_yaw || !local_topdown || !local_mask) return DM_EINVAL;
+  if (!h || h->C != 0 || !depth || !pose || !sin_yaw || !cos_yaw || !local_topdown || !local_mask) return DM_EINVAL;
   if (world && (!world->topdown || !world->mask || world->h <= 0 || world->w <= 0)) return DM_EINVAL;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   char* d_base = nullptr;
   int fast = 0;
-  int rc = upload_params(h, pose, sin_yaw, cos_yaw, world, stream, &d_base, &fast);
+  const float world_off[2] = {world ? world->width_offset : 0.0f, world ? world->height_offset : 0.0f};
+  int rc = upload_params(h, pose, sin_yaw, cos_yaw, world ? world_off : nullptr, stream, &d_base, &fast);
   if (rc != DM_OK) return rc;
   DmProjCfg pc = h->cfg.proj;
   pc.fast_steps = fast;
   pc.want_height = 0;  // C == 0: the topdown map is the height map (maps.py:333-334)
-  make_sources(h, d_base, local_topdown, local_mask, world);
+  DmValueMapRef wv = {};
+  if (world) {
+    wv.topdown = world->topdown; wv.mask = world->mask; wv.h = world->h; wv.w = world->w;
+    wv.width_offset = world->width_offset; wv.height_offset = world->height_offset;
+    wv.box = world->box; wv.plane_box = world->plane_box;
+  }
+  make_sources(h, d_base, local_topdown, local_mask, nullptr, world ? &wv : nullptr);
   // pass 1 (maps.py:2146-2179): a world map that carries the box its own scatter pass tracked only seeds the reduction
   const bool seeded = world && world->box;
   // the projection's resolve pass and pass 1 over the local map it writes are ONE kernel (dm_fuse.cu:
@@ -275,7 +329,8 @@ extern "C" int dm_builder_plot_wait(DmBuilder* h, DmMergeShape* shape) {
 
 extern "C" int dm_builder_merge(DmBuilder* h, const DmMapRef* out, void* stream_) {
   DM_TRACE();
-  if (!h || !out || !out->topdown || !out->mask || out->h <= 0 || out->w <= 0 || h->n_src <= 0) return DM_EINVAL;
+  if (!h || h->C != 0 || !out || !out->topdown || !out->mask || out->h <= 0 || out->w <= 0 || h->n_src <= 0)
+    return DM_EINVAL;
   const DmBuilderCfg& c = h->cfg;
   DmFuseTarget tgt;
   tgt.Mh = out->h; tgt.Mw = out->w; tgt.flip_h = c.proj.flip_h; tgt.map_res = c.proj.map_res;
@@ -301,7 +356,7 @@ extern "C" int dm_builder_step_fixed(DmBuilder* h, const float* depth, const flo
                                      const float* cos_yaw, float* local_topdown, uint8_t* local_mask,
                                      const DmMapRef* canvas, void* stream_) {
   DM_TRACE();
-  if (!h || !depth || !pose || !sin_yaw || !cos_yaw || !local_topdown || !local_mask) return DM_EINVAL;
+  if (!h || h->C != 0 || !depth || !pose || !sin_yaw || !cos_yaw || !local_topdown || !local_mask) return DM_EINVAL;
   if (!canvas || !canvas->topdown || !canvas->mask || canvas->h <= 0 || canvas->w <= 0) return DM_EINVAL;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   char* d_base = nullptr;
@@ -314,13 +369,129 @@ extern "C" int dm_builder_step_fixed(DmBuilder* h, const float* depth, const flo
   rc = dm_orth_project_f32(depth, nullptr, nullptr, reinterpret_cast<const DmProjSample*>(d_base), &pc, h->cfg.b,
                            local_topdown, local_mask, nullptr, h->ws, h->ws_bytes, stream);
   if (rc != DM_OK) return rc;
-  make_sources(h, d_base, local_topdown, local_mask, nullptr);
+  make_sources(h, d_base, local_topdown, local_mask, nullptr, nullptr);
   const DmBuilderCfg& c = h->cfg;
   DmFuseTarget tgt;
   tgt.Mh = canvas->h; tgt.Mw = canvas->w; tgt.flip_h = c.proj.flip_h; tgt.map_res = c.proj.map_res;
   tgt.width_offset = canvas->width_offset; tgt.height_offset = canvas->height_offset;
   tgt.fill_value = c.merge_fill_value; tgt.reduction = c.merge_reduction;
   rc = dm_fuse_inplace_f32(h->src, 1, c.b, 1, &tgt, canvas->topdown, canvas->mask, nullptr, stream);
+  h->n_src = 0;
+  return rc;
+}
+
+// ---- value maps (dm_builder_create_values) ----------------------------------------------------------------------
+
+// orth_project(value_map= / label_map=, get_height_map=True) of the step: local map, mask and its one height plane.
+static int project_values(DmBuilder* h, const float* depth, const float* values, const uint8_t* labels, char* d_base,
+                          int fast, float* topdown, uint8_t* mask, float* height, cudaStream_t stream) {
+  DmProjCfg pc = h->cfg.proj;
+  pc.fast_steps = fast;
+  const DmProjSample* samples = reinterpret_cast<const DmProjSample*>(d_base);
+  if (h->labels)
+    return dm_orth_project_labels_f32(depth, labels, nullptr, samples, &pc, h->cfg.b, topdown, mask, height, h->ws,
+                                      h->ws_bytes, stream);
+  return dm_orth_project_f32(depth, values, nullptr, samples, &pc, h->cfg.b, topdown, mask, height, h->ws, h->ws_bytes,
+                             stream);
+}
+
+static bool value_inputs_ok(const DmBuilder* h, const float* depth, const float* values, const uint8_t* labels,
+                            const float* pose, const float* sin_yaw, const float* cos_yaw, const float* local_topdown,
+                            const uint8_t* local_mask, const float* local_height) {
+  if (!h || h->C == 0 || !depth || !pose || !sin_yaw || !cos_yaw || !local_topdown || !local_mask || !local_height)
+    return false;
+  return h->labels ? (labels && !values) : (values && !labels);
+}
+
+static bool value_map_ok(const DmValueMapRef* m) {
+  return m->topdown && m->height && m->mask && m->h > 0 && m->w > 0;
+}
+
+extern "C" int dm_builder_plot_values(DmBuilder* h, const float* depth, const float* values, const uint8_t* labels,
+                                      const float* pose, const float* sin_yaw, const float* cos_yaw,
+                                      float* local_topdown, uint8_t* local_mask, float* local_height,
+                                      const DmValueMapRef* world, DmMergeShape* shape, float* prefill_topdown,
+                                      float* prefill_height, uint8_t* prefill_mask, int64_t prefill_cells,
+                                      void* stream_) {
+  DM_TRACE();
+  if (!value_inputs_ok(h, depth, values, labels, pose, sin_yaw, cos_yaw, local_topdown, local_mask, local_height))
+    return DM_EINVAL;
+  if (world && !value_map_ok(world)) return DM_EINVAL;
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  char* d_base = nullptr;
+  int fast = 0;
+  const float world_off[2] = {world ? world->width_offset : 0.0f, world ? world->height_offset : 0.0f};
+  int rc = upload_params(h, pose, sin_yaw, cos_yaw, world ? world_off : nullptr, stream, &d_base, &fast);
+  if (rc != DM_OK) return rc;
+  rc = project_values(h, depth, values, labels, d_base, fast, local_topdown, local_mask, local_height, stream);
+  if (rc != DM_OK) return rc;
+  make_sources(h, d_base, local_topdown, local_mask, local_height, world);
+  // pass 1 (maps.py:2146-2179): a tracked world map only seeds the box; the local map is scanned
+  const bool seeded = world && world->box;
+  const DmFuseSource* scan = seeded ? &h->src[h->n_src - 1] : h->src;
+  rc = dm_fuse_bbox_seeded_i64(scan, seeded ? 1 : h->n_src, h->cfg.b, h->C, h->cfg.proj.map_res,
+                               seeded ? world->box : nullptr, h->d_bbox, stream);
+  if (rc != DM_OK) return rc;
+  DM_CUDA_OK(cudaMemcpyAsync(h->h_bbox, h->d_bbox, 5 * sizeof(int64_t), cudaMemcpyDeviceToHost, stream));
+  DM_CUDA_OK(cudaEventRecord(h->ev_bbox, stream));
+  h->prefilled_top = nullptr; h->prefilled_height = nullptr; h->prefilled_mask = nullptr; h->prefilled_cells = 0;
+  prefill_cells &= ~(int64_t)15;
+  if (prefill_topdown && prefill_height && prefill_mask && prefill_cells > 0) {
+    rc = dm_fuse_canvas_init_f32(prefill_topdown, prefill_mask, prefill_height, prefill_cells, h->cfg.merge_fill_value,
+                                 stream);
+    if (rc != DM_OK) return rc;
+    h->prefilled_top = prefill_topdown; h->prefilled_height = prefill_height; h->prefilled_mask = prefill_mask;
+    h->prefilled_cells = prefill_cells;
+  }
+  return shape ? dm_builder_plot_wait(h, shape) : DM_OK;
+}
+
+extern "C" int dm_builder_merge_values(DmBuilder* h, const DmValueMapRef* out, void* stream_) {
+  DM_TRACE();
+  if (!h || h->C == 0 || !out || !value_map_ok(out) || h->n_src <= 0) return DM_EINVAL;
+  const DmBuilderCfg& c = h->cfg;
+  DmFuseTarget tgt;
+  tgt.Mh = out->h; tgt.Mw = out->w; tgt.flip_h = c.proj.flip_h; tgt.map_res = c.proj.map_res;
+  tgt.width_offset = out->width_offset; tgt.height_offset = out->height_offset;
+  tgt.fill_value = c.merge_fill_value; tgt.reduction = c.merge_reduction;
+  const int64_t n_cells = (int64_t)c.b * h->C * out->h * out->w;  // 64-bit: b * C * h * w passes 2^31 at scale
+  const bool prefilled = out->topdown == h->prefilled_top && out->height == h->prefilled_height &&
+                         out->mask == h->prefilled_mask && h->prefilled_cells > 0;
+  if (prefilled && n_cells > h->prefilled_cells) {
+    const int64_t p = h->prefilled_cells;
+    const int rf = dm_fuse_canvas_init_f32(out->topdown + p, out->mask + p, out->height + p, n_cells - p,
+                                           c.merge_fill_value, stream_);
+    if (rf != DM_OK) return rf;
+  }
+  const int rc = fuse_scatter_track(h->src, h->n_src, c.b, h->C, &tgt, out->topdown, out->mask, out->height, out->box,
+                                    out->plane_box, prefilled ? 1 : 0, stream_);
+  h->prefilled_top = nullptr; h->prefilled_height = nullptr; h->prefilled_mask = nullptr; h->prefilled_cells = 0;
+  h->n_src = 0;
+  return rc;
+}
+
+extern "C" int dm_builder_step_fixed_values(DmBuilder* h, const float* depth, const float* values,
+                                            const uint8_t* labels, const float* pose, const float* sin_yaw,
+                                            const float* cos_yaw, float* local_topdown, uint8_t* local_mask,
+                                            float* local_height, const DmValueMapRef* canvas, void* stream_) {
+  DM_TRACE();
+  if (!value_inputs_ok(h, depth, values, labels, pose, sin_yaw, cos_yaw, local_topdown, local_mask, local_height))
+    return DM_EINVAL;
+  if (!canvas || !value_map_ok(canvas)) return DM_EINVAL;
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  char* d_base = nullptr;
+  int fast = 0;
+  int rc = upload_params(h, pose, sin_yaw, cos_yaw, nullptr, stream, &d_base, &fast);
+  if (rc != DM_OK) return rc;
+  rc = project_values(h, depth, values, labels, d_base, fast, local_topdown, local_mask, local_height, stream);
+  if (rc != DM_OK) return rc;
+  make_sources(h, d_base, local_topdown, local_mask, local_height, nullptr);
+  const DmBuilderCfg& c = h->cfg;
+  DmFuseTarget tgt;
+  tgt.Mh = canvas->h; tgt.Mw = canvas->w; tgt.flip_h = c.proj.flip_h; tgt.map_res = c.proj.map_res;
+  tgt.width_offset = canvas->width_offset; tgt.height_offset = canvas->height_offset;
+  tgt.fill_value = c.merge_fill_value; tgt.reduction = c.merge_reduction;
+  rc = dm_fuse_inplace_f32(h->src, 1, c.b, h->C, &tgt, canvas->topdown, canvas->mask, canvas->height, stream);
   h->n_src = 0;
   return rc;
 }

@@ -1106,10 +1106,11 @@ class _NativeBuilder():
 
   def __init__(self, proj: MapProjector, key: tuple, dev: torch.device):
     (b, H, W, _, plot_global, woff, hoff, Mw, Mh, pitch, camh, res, _, _, tdmin, tdmax, thmax, clip, flip, fill,
-     red) = key
+     red, kind, C) = key
+    self.handle = None
     cfg = nat.DmBuilderCfg()
     p = cfg.proj
-    p.H, p.W, p.C, p.Mh, p.Mw = H, W, 0, Mh, Mw
+    p.H, p.W, p.C, p.Mh, p.Mw = H, W, C, Mh, Mw
     k = proj.cam_params
     p.fx, p.fy, p.cx, p.cy = k.fx, k.fy, k.cx, k.cy
     p.map_res = res
@@ -1134,14 +1135,22 @@ class _NativeBuilder():
     self._lib = nat.lib()
     handle = nat.ctypes.c_void_p()
     with torch.cuda.device(dev):
-      nat.check(self._lib.dm_builder_create(cfg, dev.index, nat.ctypes.byref(handle)), "dm_builder_create")
+      if kind == "height":
+        nat.check(self._lib.dm_builder_create(cfg, dev.index, nat.ctypes.byref(handle)), "dm_builder_create")
+      else:
+        nat.check(self._lib.dm_builder_create_values(cfg, int(kind == "labels"), dev.index, nat.ctypes.byref(handle)),
+                  "dm_builder_create_values")
     self.handle = handle
+
+  def close(self):
+    """Destroys the handle (dm_builder_destroy synchronises with the work it queued)."""
+    if self.handle:
+      self._lib.dm_builder_destroy(self.handle)
+      self.handle = None
 
   def __del__(self):
     try:
-      if self.handle:
-        self._lib.dm_builder_destroy(self.handle)
-        self.handle = None
+      self.close()
     except Exception:
       pass
 
@@ -1155,14 +1164,19 @@ class MapBuilder():
     SURVEY.md §8f-2): global canvases of that size are allocated at the first merge, the world origin sits
     at their centre, and every merge max-merges the new map's cells into them with one kernel launch —
     no bounding box, no host sync, no reallocation.  Points that fall outside the canvas are dropped.
-    `native_step`: height-map steps of a global-frame builder (value_map / valid_map None, CenterMode.none, device
-    depth tensors) run with their host side in C (dm_builder_*, csrc/dm_builder.cu) — same kernels, same results,
-    two library calls per step instead of ~1000 interpreter calls; anything else takes the general path."""
+    `native_step`: steps of a global-frame builder (valid_map None, CenterMode.none, device depth tensors; height
+    maps, CUDA float32 `value_map=` planes or CUDA `label_map=` class ids, reduction max / min) run with their host
+    side in C (dm_builder_*, csrc/dm_builder.cu) — same kernels, same results, two library calls per step instead of
+    ~1000 interpreter calls; anything else takes the general path.  Memory: while the host waits for the bounding box,
+    the C step fills canvases of the old world map's size class (values, heights and mask for value maps: up to
+    1.25 x the old map).  They become the new map.  When the new map outgrows them, they are released before the new
+    map's canvases are taken, so the step holds at most the old map plus one canvas set of the new map's size class,
+    as the general path does."""
     self._proj = map_projector
     self._world_map = world_map if world_map is not None else TopdownMap(map_projector=self.proj.clone())
     self._fixed = None if fixed_canvas is None else (int(fixed_canvas[0]), int(fixed_canvas[1]))
     self._native = bool(native_step)
-    self._handles: Dict[tuple, "_NativeBuilder"] = {}
+    self._handles: Dict[tuple, "_NativeBuilder"] = {}  # least recently used first, at most _MAX_HANDLES
 
   @property
   def proj(self) -> MapProjector:
@@ -1188,8 +1202,8 @@ class MapBuilder():
            **kwargs: Dict[str, Any]) -> TopdownMap:
     """Plot the frame's local map and (by default) merge it into the world map
     (maps.py:2357-2406).  Returns the local map."""
-    if self._native and merge and not keep_pose and value_map is None and valid_map is None:
-      done = self._native_step(depth_map, cam_pose, center_mode, kwargs)
+    if self._native and merge and not keep_pose and valid_map is None:
+      done = self._native_step(depth_map, value_map, cam_pose, center_mode, kwargs)
       if done is not None:
         return done
     topdown_map = self.plot(depth_map=depth_map, value_map=value_map, valid_map=valid_map, cam_pose=cam_pose,
@@ -1235,15 +1249,56 @@ class MapBuilder():
 
   # ---- the step with its host side in C (csrc/dm_builder.cu) ----------------------------------------------------
 
-  _NATIVE_KW = frozenset(("to_global", "width_offset", "height_offset", "map_width", "map_height"))
+  _NATIVE_KW = frozenset(("to_global", "width_offset", "height_offset", "map_width", "map_height", "label_map",
+                          "num_classes"))
+  _MAX_HANDLES = 4  # a value-map handle owns a projection workspace of C planes: keep the few recently used ones
 
-  def _native_step(self, depth_map, cam_pose, center_mode, kwargs) -> Optional[TopdownMap]:
+  def _native_handle(self, key: tuple, dev: torch.device) -> "_NativeBuilder":
+    """The handle of `key`, created on first use; the least recently used one beyond _MAX_HANDLES is destroyed."""
+    nb = self._handles.pop(key, None)
+    if nb is None:
+      nb = _NativeBuilder(self.proj, key, dev)
+    self._handles[key] = nb
+    while len(self._handles) > self._MAX_HANDLES:
+      self._handles.pop(next(iter(self._handles))).close()
+    return nb
+
+  @staticmethod
+  def _native_values(depth_map, value_map, kwargs):
+    """(kind, C, values, labels) of a step the C step can take, or None: kind "height" (C = 0), "values" (a CUDA
+    float32 contiguous (b, C, H, W) value_map) or "labels" (a CUDA integer (b, 1, H, W) label_map, 1..63 classes).
+    Argument errors are left to the general path, which reports them."""
+    label_map, num_classes = kwargs.get("label_map"), kwargs.get("num_classes")
+    b, _, H, W = depth_map.shape
+    if label_map is not None:
+      if (value_map is not None or num_classes is None or not torch.is_tensor(label_map) or not label_map.is_cuda
+          or label_map.device != depth_map.device or label_map.dtype.is_floating_point or label_map.dtype is torch.bool
+          or tuple(label_map.shape) != (b, 1, H, W) or not 1 <= int(num_classes) <= 63):
+        return None
+      C = int(num_classes)
+      return "labels", C, None, _label_ids(label_map, C, depth_map.device)
+    if num_classes is not None:
+      return None
+    if value_map is None:
+      return "height", 0, None, None
+    if (not torch.is_tensor(value_map) or value_map.device != depth_map.device or value_map.dtype is not torch.float32
+        or value_map.dim() != 4 or value_map.shape[0] != b or value_map.shape[1] < 1
+        or tuple(value_map.shape[2:]) != (H, W) or not value_map.is_contiguous()):
+      return None
+    return "values", int(value_map.shape[1]), value_map, None
+
+  def _native_step(self, depth_map, value_map, cam_pose, center_mode, kwargs) -> Optional[TopdownMap]:
     """MapBuilder.step for the case dm_builder_* covers; None when the call needs the general path."""
     proj = self.proj
     if (CenterMode(center_mode) is not CenterMode.none or not set(kwargs) <= self._NATIVE_KW or not proj.to_global
         or not torch.is_tensor(depth_map) or not depth_map.is_cuda or depth_map.dtype is not torch.float32
         or depth_map.dim() != 4 or depth_map.shape[1] != 1 or not depth_map.is_contiguous()):
       return None
+    inputs = self._native_values(depth_map, value_map, kwargs)
+    if inputs is None:
+      return None
+    kind, C, values, labels = inputs
+    kwargs = {k: v for k, v in kwargs.items() if k not in ("label_map", "num_classes")}
     get_kw = lambda name: get(kwargs.get(name), getattr(proj, name))
     scalars = [proj.cam_pitch, proj.cam_height, proj.map_res, get_kw("width_offset"), get_kw("height_offset"),
                get_kw("map_width"), get_kw("map_height")]
@@ -1259,7 +1314,7 @@ class MapBuilder():
       return None
     world = self._world_map
     have_world = world is not None and not world.is_empty
-    if have_world and not self._native_world_ok(world, b, dev):
+    if have_world and not self._native_world_ok(world, b, dev, C):
       return None
     cam_pose = get(cam_pose, proj.cam_pose, np.array([0., 0., 0.], dtype=np.float32))
     plot_global = bool(get_kw("to_global"))
@@ -1268,10 +1323,10 @@ class MapBuilder():
     fill = proj.fill_value
     key = (b, H, W, dev.index, plot_global, woff, hoff, Mw, Mh, float(proj.cam_pitch), float(proj.cam_height),
            float(proj.map_res), proj.hfov, proj.vfov, proj.trunc_depth_min, proj.trunc_depth_max,
-           proj.trunc_height_max, proj.clip_border, bool(proj.flip_h), fill, red)
-    nb = self._handles.get(key)
-    if nb is None:
-      nb = self._handles[key] = _NativeBuilder(proj, key, dev)
+           proj.trunc_height_max, proj.clip_border, bool(proj.flip_h), fill, red, kind, C)
+    nb = self._native_handle(key, dev)
+    if C > 0:
+      return self._native_value_step(nb, depth_map, values, labels, C, cam_pose, kwargs, have_world, woff, hoff, Mw, Mh)
     pose = prm.per_sample(cam_pose, b, (3,), "cam_pose").contiguous()
     # utils.py:325-326 with the reference's own torch-CPU ops (the last ulp of sin / cos matters)
     sin, cos = prm.yaw_sin_cos(pose)
@@ -1369,18 +1424,122 @@ class MapBuilder():
     self._world_map = merged
     return local
 
-  def _native_world_ok(self, world: TopdownMap, b: int, dev: torch.device) -> bool:
-    """The world map is one the C step can take as it is: a contiguous (b, 1, h, w) float32 height map + bool mask on
+  def _native_value_step(self, nb: "_NativeBuilder", depth_map, values, labels, C: int, cam_pose, kwargs,
+                         have_world: bool, woff: float, hoff: float, Mw: int, Mh: int) -> TopdownMap:
+    """_native_step for value maps (dm_builder_plot_values / _merge_values / _step_fixed_values): the same sequence as
+    the height-map step with (b, C, h, w) maps, their height planes, and (b * C, 4) plane boxes."""
+    proj, world = self.proj, self._world_map
+    dev = depth_map.device
+    b = depth_map.shape[0]
+    cam_pose = get(cam_pose, proj.cam_pose, np.array([0., 0., 0.], dtype=np.float32))
+    pose = prm.per_sample(cam_pose, b, (3,), "cam_pose").contiguous()
+    sin, cos = prm.yaw_sin_cos(pose)  # utils.py:325-326 with the reference's own torch-CPU ops
+    local_top = torch.empty((b, C, Mh, Mw), dtype=torch.float32, device=dev)
+    local_mask = torch.empty((b, C, Mh, Mw), dtype=torch.bool, device=dev)
+    local_height = torch.empty((b, 1, Mh, Mw), dtype=torch.float32, device=dev)
+    lib = nat.lib()
+    stream = nat.stream_ptr(dev)
+    inputs = (depth_map.data_ptr(), nat.ptr(values), nat.ptr(labels), pose.data_ptr(), sin.data_ptr(), cos.data_ptr(),
+              local_top.data_ptr(), local_mask.data_ptr(), local_height.data_ptr())
+    def make_local():
+      """The local map as plot() describes it: the height map is the stride-0 expand orth_project returns."""
+      local_kw = {k: v for k, v in kwargs.items() if k in _CTOR_ARGS}
+      local_kw["width_offset"] = torch.tensor([woff], dtype=torch.float32)
+      local_kw["height_offset"] = torch.tensor([hoff], dtype=torch.float32)
+      return TopdownMap(topdown_map=local_top, mask=local_mask, height_map=torch.broadcast_to(local_height, local_top.shape),
+                        map_projector=proj.clone(cam_pose=cam_pose, **local_kw), is_height_map=False)
+    target = proj.clone(cam_pose=cam_pose)
+    fill = nb.fill
+    with torch.cuda.device(dev):
+      if self._fixed is not None:
+        Hc, Wc = self._fixed
+        if not have_world:
+          topdown = torch.empty((b, C, Hc, Wc), dtype=torch.float32, device=dev)
+          mask = torch.empty((b, C, Hc, Wc), dtype=torch.bool, device=dev)
+          height = torch.empty_like(topdown)
+          nat.check(lib.dm_fuse_canvas_init_f32(topdown.data_ptr(), mask.data_ptr(), height.data_ptr(), topdown.numel(),
+                                                fill, stream), "dm_fuse_canvas_init_f32")
+        else:
+          topdown, mask, height = world.topdown_map, world.mask, world.height_map
+        canvas = nat.DmValueMapRef(topdown.data_ptr(), height.data_ptr(), mask.data_ptr(), Hc, Wc, Wc / 2., Hc / 2.,
+                                   None, None)
+        nat.check(lib.dm_builder_step_fixed_values(nb.handle, *inputs, canvas, stream), "dm_builder_step_fixed_values")
+        self._world_map = TopdownMap(
+          topdown_map=topdown, mask=mask, height_map=height, is_height_map=False,
+          map_projector=target.clone(to_global=True, width_offset=Wc / 2., height_offset=Hc / 2., map_width=Wc,
+                                     map_height=Hc))
+        return make_local()
+      wref = None
+      if have_world:
+        box = world._tracked_box.box if _tracked_box_valid(world, target, dev) else None
+        tb = getattr(world, "_tracked_box", None)
+        planes = None
+        if (tb is not None and tb.plane_box is not None and world.mask is tb.mask
+            and tb.mask._version == tb.mask_version and tb.plane_box.device == dev):
+          planes = tb.plane_box
+        wref = nat.DmValueMapRef(world.topdown_map.data_ptr(), world.height_map.data_ptr(), world.mask.data_ptr(),
+                                 world.mask.shape[-2], world.mask.shape[-1], float(world.proj.width_offset),
+                                 float(world.proj.height_offset), nat.ptr(box), nat.ptr(planes))
+      shape = nat.DmMergeShape()
+      track = fill == fill
+      next_box = torch.empty((5,), dtype=torch.int64, device=dev) if track else None
+      next_planes = torch.empty((b * C, 4), dtype=torch.int32, device=dev) if track else None
+      spec = None  # canvases of the old map's size class, filled while the host waits for the box (see _native_step)
+      if have_world and world.mask.numel() >= (1 << 18):
+        cap = _canvas_cap(world.mask.numel())
+        spec = (torch.empty((cap,), dtype=torch.float32, device=dev), torch.empty((cap,), dtype=torch.float32, device=dev),
+                torch.empty((cap,), dtype=torch.bool, device=dev))
+      n_guess = 0 if spec is None else min(spec[0].numel(), world.mask.numel() + world.mask.numel() // 50 + 4096)
+      nat.check(lib.dm_builder_plot_values(nb.handle, *inputs, wref, None, *[nat.ptr(t) for t in (spec or (None,) * 3)],
+                                           n_guess, stream), "dm_builder_plot_values")
+      local = make_local()
+      nat.check(lib.dm_builder_plot_wait(nb.handle, shape), "dm_builder_plot_wait")
+      if shape.n_valid == 0:  # maps.py:2217-2225
+        self._world_map = TopdownMap(topdown_map=local.topdown_map, mask=local.mask, height_map=local.height_map,
+                                     map_projector=target)
+        return local
+      mh, mw = shape.map_height, shape.map_width
+      n_new = b * C * mh * mw
+      if spec is not None and (1 << 18) <= n_new <= spec[0].numel():
+        topdown, height, mask = (t[:n_new].view(b, C, mh, mw) for t in spec)
+      else:
+        # the map outgrew the guess: the speculative canvases go back to the allocator BEFORE the new ones are taken,
+        # so that three C-channel canvases of the old class are not held next to the old map and the new one
+        # (the prefill queued on them is ordered before any later use of their blocks on this stream)
+        spec = None
+        topdown = _alloc_canvas((b, C, mh, mw), torch.float32, dev)
+        height = _alloc_canvas((b, C, mh, mw), torch.float32, dev)
+        mask = _alloc_canvas((b, C, mh, mw), torch.bool, dev)
+      spec = None
+      out = nat.DmValueMapRef(topdown.data_ptr(), height.data_ptr(), mask.data_ptr(), mh, mw, shape.width_offset,
+                              shape.height_offset, nat.ptr(next_box), nat.ptr(next_planes))
+      nat.check(lib.dm_builder_merge_values(nb.handle, out, stream), "dm_builder_merge_values")
+    new_proj = target.clone(width_offset=torch.tensor([shape.width_offset], dtype=torch.float32),
+                            height_offset=torch.tensor([shape.height_offset], dtype=torch.float32),
+                            map_width=mw, map_height=mh)
+    merged = TopdownMap(topdown_map=topdown, mask=mask, height_map=height, map_projector=new_proj, is_height_map=False)
+    if track:
+      merged._tracked_box = _TrackedBox(next_box, mask, new_proj, next_planes)
+    self._world_map = merged
+    return local
+
+  def _native_world_ok(self, world: TopdownMap, b: int, dev: torch.device, C: int = 0) -> bool:
+    """The world map is one the C step can take as it is: a contiguous (b, 1, h, w) float32 height map + bool mask
+    (C = 0), or a contiguous (b, C, h, w) float32 value map with (b, C, h, w) height planes + bool mask (C >= 1), on
     `dev`, in the global frame, with this builder's resolution / flip and scalar offsets."""
     p, proj = world.proj, self.proj
     top, mask = world.topdown_map, world.mask
-    if not (world.is_height_map and p is not None and p.to_global and torch.is_tensor(top) and torch.is_tensor(mask)):
+    if not (bool(world.is_height_map) == (C == 0) and p is not None and p.to_global and torch.is_tensor(top)
+            and torch.is_tensor(mask)):
       return False
     if self._fixed is not None and tuple(top.shape[-2:]) != self._fixed:
       return False
-    ok_t = lambda t, dt: (t.device == dev and t.dtype is dt and t.dim() == 4 and t.shape[0] == b and t.shape[1] == 1
-                          and t.is_contiguous())
+    ok_t = lambda t, dt: (t.device == dev and t.dtype is dt and t.dim() == 4 and t.shape[0] == b
+                          and t.shape[1] == max(C, 1) and t.is_contiguous())
     if not (ok_t(top, torch.float32) and ok_t(mask, torch.bool) and top.shape == mask.shape):
+      return False
+    hm = world.height_map
+    if C > 0 and not (torch.is_tensor(hm) and ok_t(hm, torch.float32) and hm.shape == top.shape):
       return False
     def one(v):
       if v is None:

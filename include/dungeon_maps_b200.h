@@ -308,8 +308,8 @@ int dm_pack_flow_samples(const DmPoseCfg* cfg, const float* pose, const float* s
 typedef struct DmBuilder DmBuilder; /* opaque */
 
 typedef struct DmBuilderCfg {
-  DmProjCfg proj;          /* projection of the local maps (maps.py:2447-2458); C must be 0; fast_steps, want_height
-                              are derived */
+  DmProjCfg proj;          /* projection of the local maps (maps.py:2447-2458); C: 0 for dm_builder_create, the
+                              channel count for dm_builder_create_values; fast_steps, want_height are derived */
   int32_t b;               /* environments */
   int32_t plot_to_global;  /* the local maps are plotted in the global frame (to_global of the plot call) */
   float pitch_R[9];        /* DmStep.R of camera_to_local_space: rotation about x by cam_pitch, built on the host by
@@ -370,6 +370,43 @@ int dm_builder_step_fixed(DmBuilder* builder, const float* depth, const float* p
                           const float* cos_yaw, float* local_topdown, uint8_t* local_mask, const DmMapRef* canvas,
                           void* stream);
 
+/* The same step for value maps: MapBuilder.step(value_map=) with float planes, or step(label_map=, num_classes=) with
+ * class ids (the one_hot planes of the reference's object-map loop, never materialised).  World maps carry C height
+ * planes of their own (maps.py:2258-2271); the local map has one, shared by its C channels (maps.py:349).  Results are
+ * those of dm_orth_project_f32 / dm_orth_project_labels_f32 (want_height) + dm_fuse_bbox_seeded_i64 +
+ * dm_fuse_scatter_track_f32 / dm_fuse_inplace_f32 called one by one. */
+typedef struct DmValueMapRef {
+  float* topdown;     /* (b, C, h, w) f32 values */
+  float* height;      /* (b, C, h, w) f32 height planes */
+  uint8_t* mask;      /* (b, C, h, w) u8 */
+  int32_t h, w;
+  float width_offset, height_offset;
+  int64_t* box;       /* as DmMapRef.box */
+  int32_t* plane_box; /* device, (b * C, 4) int32: as DmMapRef.plane_box, one rectangle per (sample, channel) */
+} DmValueMapRef;
+
+/* cfg->proj.C = C channels: 1..63 with labels != 0 (class ids), >= 1 otherwise (float planes).  Reductions max / min
+ * (proj.reduction and merge_reduction).  DM_EINVAL for anything else, before any CUDA call.  The handle owns the
+ * workspace of the projection entry it uses.  Destroy with dm_builder_destroy. */
+int dm_builder_create_values(const DmBuilderCfg* cfg, int32_t labels, int32_t device, DmBuilder** out);
+/* dm_builder_plot_prefill for value maps.  Input: values (b, C, H, W) f32 (labels NULL) or labels (b, 1, H, W) u8
+ * (values NULL), as the handle was created.  Output: local_topdown / local_mask (b, C, Mh, Mw), local_height
+ * (b, 1, Mh, Mw).  world may be NULL.  The prefill covers three canvases of prefill_cells elements each:
+ * prefill_topdown = fill, prefill_height = -inf, prefill_mask = 0.  shape NULL: wait with dm_builder_plot_wait. */
+int dm_builder_plot_values(DmBuilder* builder, const float* depth, const float* values, const uint8_t* labels,
+                           const float* pose, const float* sin_yaw, const float* cos_yaw, float* local_topdown,
+                           uint8_t* local_mask, float* local_height, const DmValueMapRef* world, DmMergeShape* shape,
+                           float* prefill_topdown, float* prefill_height, uint8_t* prefill_mask, int64_t prefill_cells,
+                           void* stream);
+/* dm_builder_merge for value maps: fills `out` (the tail beyond a prefill) and scatters the world map and the local map
+ * of the preceding dm_builder_plot_values into it; out->box / out->plane_box (may be NULL) receive the tracked boxes. */
+int dm_builder_merge_values(DmBuilder* builder, const DmValueMapRef* out, void* stream);
+/* dm_builder_step_fixed for value maps: plot, then merge in place into the (b, C, Hc, Wc) canvases and their height
+ * planes; no host sync. */
+int dm_builder_step_fixed_values(DmBuilder* builder, const float* depth, const float* values, const uint8_t* labels,
+                                 const float* pose, const float* sin_yaw, const float* cos_yaw, float* local_topdown,
+                                 uint8_t* local_mask, float* local_height, const DmValueMapRef* canvas, void* stream);
+
 /* ---- materialising primitives (the reference's public L0/L1 functions) ------ */
 
 /* points (b, n, 3) f32 → out (b, n, 3): applies steps[b][n_steps] in order.
@@ -427,7 +464,7 @@ int dm_crop_nearest_u8(const uint8_t* image, const float* center, int32_t b, int
 int dm_abi_version(void);
 /* sizeof() of a struct of this header as the library was compiled, for bindings to check their mirror against:
  * 0 DmStep, 1 DmProjSample, 2 DmProjCfg, 3 DmFlowSample, 4 DmFlowCfg, 5 DmFuseSource, 6 DmFuseTarget,
- * 7 DmBuilderCfg, 8 DmMapRef, 9 DmMergeShape, 10 DmPoseCfg; -1 for an unknown id. */
+ * 7 DmBuilderCfg, 8 DmMapRef, 9 DmMergeShape, 10 DmPoseCfg, 11 DmValueMapRef; -1 for an unknown id. */
 int32_t dm_sizeof_struct(int32_t id);
 const char* dm_build_info(void);
 /* Number of kernel launches issued by this library since load (bench "gpu_launches"). */
