@@ -126,6 +126,8 @@ _SIGNATURES = {
   "dm_fuse_inplace_f32": (ctypes.c_int, [POINTER(DmFuseSource), c_int32, c_int32, c_int32, POINTER(DmFuseTarget),
                                          c_void_p, c_void_p, c_void_p, c_void_p]),
   "dm_fuse_canvas_init_f32": (ctypes.c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_float, c_void_p]),
+  "dm_fuse_clear_envs_f32": (ctypes.c_int, [c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_void_p,
+                                            POINTER(DmFuseTarget), c_void_p, c_void_p, c_void_p]),
   "dm_pack_proj_samples": (ctypes.c_int, [POINTER(DmPoseCfg), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int32,
                                           c_int32, c_void_p, POINTER(c_int32)]),
   "dm_pack_flow_samples": (ctypes.c_int, [POINTER(DmPoseCfg), c_void_p, c_void_p, c_void_p, c_int32, c_void_p]),

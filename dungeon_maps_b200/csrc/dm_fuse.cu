@@ -397,24 +397,54 @@ hmap_resolve_bbox_kernel(uint32_t* __restrict__ acc, unsigned long long slot_wor
   }
 }
 
-// Fresh canvases: topdown = fill (utils.py:472-473), height = -inf (maps.py:2268), mask = false.
+// Fresh canvases: topdown = fill (utils.py:472-473), height = -inf (maps.py:2268), mask = false, over cells [0, n) of
+// one span (a whole batch of canvases, or one plane of it) by thread `tid` of `nth`.
 // Consecutive lanes store consecutive 16-byte words (a thread owning 64 contiguous bytes made every warp
-// store touch 32 different lines: 45 % of DRAM peak in ncu); unaligned bases / the tail take the scalar loop.
-__global__ void __launch_bounds__(kFuseThreads)
-fuse_fill_kernel(float* __restrict__ topdown, float* __restrict__ height, uint8_t* __restrict__ mask, long long n,
-                 float fill, int vec_ok) {
-  const long long n16 = vec_ok ? n / 16 : 0;
-  const long long tid = (long long)blockIdx.x * kFuseThreads + threadIdx.x, nth = (long long)gridDim.x * kFuseThreads;
+// store touch 32 different lines: 45 % of DRAM peak in ncu).  vec_ok: the three arrays' bases are 16-byte aligned, so
+// a cell whose mask byte is 16-byte aligned is aligned in the float arrays too; the head up to the mask's first such
+// cell (a plane of h * w cells starts anywhere), the tail, and spans without vec_ok take the scalar loop.
+__device__ __forceinline__ void fill_span(float* __restrict__ topdown, float* __restrict__ height,
+                                          uint8_t* __restrict__ mask, long long n, float fill, int vec_ok,
+                                          long long tid, long long nth) {
+  long long head = vec_ok ? (long long)((16 - (reinterpret_cast<uintptr_t>(mask) & 15)) & 15) : n;
+  if (head > n) head = n;
+  const long long n16 = (n - head) / 16;
+  float* t = topdown + head;
+  float* h = height ? height + head : nullptr;
+  uint8_t* m = mask + head;
   const float4 f4 = make_float4(fill, fill, fill, fill);
   const float4 h4 = make_float4(-INFINITY, -INFINITY, -INFINITY, -INFINITY);
-  for (long long i = tid; i < n16 * 4; i += nth) st_stream_f4(topdown + i * 4, f4);
-  if (height)
-    for (long long i = tid; i < n16 * 4; i += nth) st_stream_f4(height + i * 4, h4);
-  for (long long i = tid; i < n16; i += nth) *reinterpret_cast<uint4*>(mask + i * 16) = make_uint4(0u, 0u, 0u, 0u);
-  for (long long i = n16 * 16 + tid; i < n; i += nth) {
+  for (long long i = tid; i < n16 * 4; i += nth) st_stream_f4(t + i * 4, f4);
+  if (h)
+    for (long long i = tid; i < n16 * 4; i += nth) st_stream_f4(h + i * 4, h4);
+  for (long long i = tid; i < n16; i += nth) *reinterpret_cast<uint4*>(m + i * 16) = make_uint4(0u, 0u, 0u, 0u);
+  auto one = [&](long long i) {
     topdown[i] = fill;
     if (height) height[i] = -INFINITY;
     mask[i] = 0;
+  };
+  for (long long i = tid; i < head; i += nth) one(i);
+  for (long long i = head + n16 * 16 + tid; i < n; i += nth) one(i);
+}
+
+__global__ void __launch_bounds__(kFuseThreads)
+fuse_fill_kernel(float* __restrict__ topdown, float* __restrict__ height, uint8_t* __restrict__ mask, long long n,
+                 float fill, int vec_ok) {
+  fill_span(topdown, height, mask, n, fill, vec_ok, (long long)blockIdx.x * kFuseThreads + threadIdx.x,
+            (long long)gridDim.x * kFuseThreads);
+}
+
+// MapBuilder.reset_envs: every plane of a sample with done[sample] set gets what fuse_fill_kernel writes, whole (the
+// height planes of a value map hold heights at cells whose mask is 0, so the tracked rectangle is not enough); a block
+// of another sample's plane leaves at once.  grid = (blocks per plane, planes folded into y).
+__global__ void __launch_bounds__(kFuseThreads)
+fuse_clear_kernel(float* __restrict__ topdown, float* __restrict__ height, uint8_t* __restrict__ mask,
+                  const uint8_t* __restrict__ done, int planes, int C, long long M, float fill, int vec_ok) {
+  for (int plane = blockIdx.y; plane < planes; plane += gridDim.y) {
+    if (!__ldg(done + plane / C)) continue;
+    const long long o = (long long)plane * M;
+    fill_span(topdown + o, height ? height + o : nullptr, mask + o, M, fill, vec_ok,
+              (long long)blockIdx.x * kFuseThreads + threadIdx.x, (long long)gridDim.x * kFuseThreads);
   }
 }
 
@@ -485,6 +515,24 @@ __device__ __forceinline__ bool plane_shift(const DmFuseSource& src, const Plane
   *dx_out = dx;
   *dz_out = dz;
   return __syncthreads_and(ok) != 0;
+}
+
+// min_x, max_x, min_z, max_z that pass 1 (fuse_bbox_kernel: source_point + quantize_f with zero offsets) finds for a
+// global-frame map in `tgt`'s frame whose valid cells span columns cmin..cmax and rows rmin..rmax (whole numbers held
+// in floats).  Every float step is weakly monotone in the column and in the (flipped) row, so the extreme cells give
+// the extremes.  Shared by the scatter pass, which tracks the box of the map it writes, and the box rebuild of
+// dm_fuse_clear_envs_f32: the same float operations by construction.
+__device__ __forceinline__ void tracked_box(const DmFuseTarget& tgt, float cmin, float cmax, float rmin, float rmax,
+                                            long long* q) {
+  // rows: the dequantised z falls with the row when the map is flipped (maps.py:1081-1083)
+  const float zlo = tgt.flip_h ? __fsub_rn((float)(tgt.Mh - 1), rmax) : rmin;
+  const float zhi = tgt.flip_h ? __fsub_rn((float)(tgt.Mh - 1), rmin) : rmax;
+  auto deq = [&](float bin, float off) { return __fmul_rn(__fsub_rn(bin, off), tgt.map_res); };
+  float qx0, qx1, qz0, qz1;
+  quantize_f(deq(cmin, tgt.width_offset), deq(zlo, tgt.height_offset), 0.0f, 0.0f, tgt.map_res, 0, 0, &qx0, &qz0);
+  quantize_f(deq(cmax, tgt.width_offset), deq(zhi, tgt.height_offset), 0.0f, 0.0f, tgt.map_res, 0, 0, &qx1, &qz1);
+  q[0] = f2i64(qx0); q[1] = f2i64(qx1);
+  q[2] = f2i64(qz0); q[3] = f2i64(qz1);
 }
 
 __global__ void fuse_plane_box_init(int* box, int planes) {
@@ -606,17 +654,56 @@ fuse_scatter_kernel(const __grid_constant__ DmFuseSource src, int planes, int C,
     block_reduce_box(cmin, cmax, rmin, rmax);
     if (threadIdx.x == 0) {
       if (cmin <= cmax) {
-        // rows: the dequantised z falls with the row when the map is flipped (maps.py:1081-1083)
-        const float zlo = tgt.flip_h ? __fsub_rn((float)(tgt.Mh - 1), rmax) : rmin;
-        const float zhi = tgt.flip_h ? __fsub_rn((float)(tgt.Mh - 1), rmin) : rmax;
-        auto deq = [&](float bin, float off) { return __fmul_rn(__fsub_rn(bin, off), tgt.map_res); };
-        float qx0, qx1, qz0, qz1;
-        quantize_f(deq(cmin, tgt.width_offset), deq(zlo, tgt.height_offset), 0.0f, 0.0f, tgt.map_res, 0, 0, &qx0, &qz0);
-        quantize_f(deq(cmax, tgt.width_offset), deq(zhi, tgt.height_offset), 0.0f, 0.0f, tgt.map_res, 0, 0, &qx1, &qz1);
-        atomicMin(next_bbox + 0, f2i64(qx0)); atomicMax(next_bbox + 1, f2i64(qx1));
-        atomicMin(next_bbox + 2, f2i64(qz0)); atomicMax(next_bbox + 3, f2i64(qz1));
+        long long q[4];
+        tracked_box(tgt, cmin, cmax, rmin, rmax, q);
+        atomicMin(next_bbox + 0, q[0]); atomicMax(next_bbox + 1, q[1]);
+        atomicMin(next_bbox + 2, q[2]); atomicMax(next_bbox + 3, q[3]);
         atomicAdd(reinterpret_cast<unsigned long long*>(next_bbox + 4), 1ull);
       }
+    }
+  }
+}
+
+// dm_fuse_clear_envs_f32's rectangles and box, one block: the rectangles of the cleared planes become empty
+// (fuse_plane_box_init's sentinel), the others stay, and `box` (may be NULL) becomes what the scatter pass would have
+// left for a map holding only the surviving planes: tracked_box() of their extremes, counting the non-empty planes
+// (zero iff no valid cell is left).  With nothing cleared it stays as it is.
+__global__ void __launch_bounds__(kScanThreads)
+fuse_clear_boxes_kernel(const uint8_t* __restrict__ done, int planes, int C, const DmFuseTarget tgt,
+                        int* __restrict__ plane_box, long long* __restrict__ box) {
+  __shared__ unsigned int s_cnt;
+  if (threadIdx.x == 0) s_cnt = 0;
+  __syncthreads();
+  float cmin = INFINITY, cmax = -INFINITY, rmin = INFINITY, rmax = -INFINITY;
+  unsigned int cnt = 0;
+  int cleared = 0;
+  for (int p = threadIdx.x; p < planes; p += kScanThreads) {
+    int4* pb = reinterpret_cast<int4*>(plane_box) + p;  // rmin, rmax, cmin, cmax
+    if (__ldg(done + p / C)) {
+      *pb = make_int4(0x7fffffff, -1, 0x7fffffff, -1);
+      cleared = 1;
+      continue;
+    }
+    const int4 bx = *pb;
+    if (bx.y < bx.x || bx.w < bx.z) continue;  // no valid cell
+    rmin = fminf(rmin, (float)bx.x); rmax = fmaxf(rmax, (float)bx.y);
+    cmin = fminf(cmin, (float)bx.z); cmax = fmaxf(cmax, (float)bx.w);
+    ++cnt;
+  }
+  if (!box) return;  // block-uniform
+  if (!__syncthreads_or(cleared)) return;  // nothing cleared: the box stays as the scatter pass left it, count included
+  if (cnt) atomicAdd(&s_cnt, cnt);
+  block_reduce_box(cmin, cmax, rmin, rmax);  // its barriers order the count's atomics before thread 0 reads it
+  if (threadIdx.x == 0) {
+    if (s_cnt) {
+      long long q[4];
+      tracked_box(tgt, cmin, cmax, rmin, rmax, q);
+      for (int i = 0; i < 4; ++i) box[i] = q[i];
+      box[4] = s_cnt;
+    } else {  // what fuse_bbox_init starts from
+      box[0] = 0x7fffffffffffffffLL; box[1] = (long long)0x8000000000000000ULL;
+      box[2] = 0x7fffffffffffffffLL; box[3] = (long long)0x8000000000000000ULL;
+      box[4] = 0;
     }
   }
 }
@@ -913,5 +1000,39 @@ extern "C" int dm_fuse_canvas_init_f32(float* topdown, uint8_t* mask, float* hei
                      (!height || reinterpret_cast<uintptr_t>(height) % 16 == 0);
   fuse_fill_kernel<<<grid_for((n + 3) / 4), kFuseThreads, 0, stream>>>(topdown, height, mask, n, fill_value, vec_ok);
   DM_LAUNCHED();
+  return DM_OK;
+}
+
+/* MapBuilder.reset_envs: the planes of the samples with done[s] set become fresh canvas, their tracked rectangles empty,
+ * and the tracked box is rebuilt from the surviving rectangles.  `done` is read on the device only. */
+extern "C" int dm_fuse_clear_envs_f32(float* topdown, float* height, uint8_t* mask, int32_t b, int32_t C,
+                                      const uint8_t* done, const DmFuseTarget* map, int32_t* plane_box, int64_t* box,
+                                      void* stream_) {
+  DM_TRACE();
+  if (!topdown || !mask || !done || !map || b <= 0 || C <= 0 || map->Mh <= 0 || map->Mw <= 0) return DM_EINVAL;
+  if ((long long)b * C >= (1ll << 31) || (long long)map->Mh * map->Mw >= (1ll << 31)) return DM_EINVAL;
+  if (map->reduction < 0 || map->reduction > 4) return DM_EINVAL;
+  if (box && !plane_box) return DM_EINVAL;  // the box is rebuilt from the rectangles
+  // tracking assumes "mask = beats fill"
+  if ((box || plane_box) && (!(map->fill_value == map->fill_value) || map->reduction >= 2)) return DM_EINVAL;
+  if (reinterpret_cast<uintptr_t>(plane_box) % 16 != 0) return DM_EINVAL;
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  const int planes = b * C;
+  const long long M = (long long)map->Mh * map->Mw;
+  const int vec_ok = reinterpret_cast<uintptr_t>(topdown) % 16 == 0 && reinterpret_cast<uintptr_t>(mask) % 16 == 0 &&
+                     (!height || reinterpret_cast<uintptr_t>(height) % 16 == 0);
+  // a block stores 1024 cells per round: a few rounds per block, and at most two blocks per SM for one plane (the
+  // blocks of planes that are not cleared cost a launch slot each)
+  long long gx = (M + 4095) / 4096;
+  if (gx > 2ll * sm_count()) gx = 2ll * sm_count();
+  const unsigned gy = planes < 65535 ? (unsigned)planes : 65535u;
+  fuse_clear_kernel<<<dim3((unsigned)gx, gy), kFuseThreads, 0, stream>>>(topdown, height, mask, done, planes, C, M,
+                                                                         map->fill_value, vec_ok);
+  DM_LAUNCHED();
+  if (plane_box) {
+    fuse_clear_boxes_kernel<<<1, kScanThreads, 0, stream>>>(done, planes, C, *map, plane_box,
+                                                            reinterpret_cast<long long*>(box));
+    DM_LAUNCHED();
+  }
   return DM_OK;
 }

@@ -1177,6 +1177,9 @@ class MapBuilder():
     self._fixed = None if fixed_canvas is None else (int(fixed_canvas[0]), int(fixed_canvas[1]))
     self._native = bool(native_step)
     self._handles: Dict[tuple, "_NativeBuilder"] = {}  # least recently used first, at most _MAX_HANDLES
+    # the mask of the world map when its canvases are the builder's own (a merge allocated them), else None:
+    # reset_envs writes into those only
+    self._owned: Optional[torch.Tensor] = None
 
   @property
   def proj(self) -> MapProjector:
@@ -1191,10 +1194,91 @@ class MapBuilder():
             center_mode: CenterMode = CenterMode.none, **kwargs):
     """Forget the world map; if a frame is given, plot and merge it (maps.py:2312-2355)."""
     self._world_map = TopdownMap(map_projector=self.proj.clone())
+    self._owned = None
     if depth_map is None:
       return None
     return self.step(depth_map=depth_map, value_map=value_map, valid_map=valid_map, cam_pose=cam_pose,
                      center_mode=center_mode, **kwargs)
+
+  def reset_envs(self, done, fill_value: Optional[float] = None) -> None:
+    """Forget the world map of every environment i with done[i] set and keep the others bit for bit (not in the
+    reference, whose MapBuilder is not batched): a vectorised loop whose episodes end at different steps keeps one
+    batched builder.
+
+    `done`: (b,) bools, b the world map's batch.  A CUDA bool tensor on the world map's device is read by the kernel
+    only (no host sync); a CPU tensor, numpy array or list is uploaded.  ValueError for another length, another dtype
+    or another CUDA device.
+
+    Every plane of a done environment becomes what a fresh canvas holds: `get(fill_value, proj.fill_value, NINF)`
+    (merge's fill rule), heights -inf (value maps; a height map's heights are its values and get the fill), mask False.
+    Shape, offsets and projector stay; the next merge sizes the canvas from the cells that are left, as every merge
+    does, so the map may shrink.  The per-plane rectangles and the bounding box the world map carries are kept up to
+    date on the device, so the next step still starts from the box instead of scanning the world map.
+
+    In place when the canvases are the builder's own: a world map a merge allocated, or a fixed canvas the builder
+    allocated.  A world map that shares tensors with the caller (one passed to the constructor, or a local map that a
+    merge adopted because nothing was valid before) is replaced by a cleared copy; the caller's tensors stay as they
+    were.  With no world map yet there is nothing to do."""
+    world = self._world_map
+    if world is None or world.is_empty:
+      return
+    in_place = world.mask is self._owned
+    top, mask, hm = world.topdown_map, world.mask, world.height_map
+    dev = mask.device if in_place else _pick_device(self.proj.device, mask, top)
+    b, C = utils.to_4D_image(mask).shape[:2]
+    done_dev = self._done_flags(done, b, dev)
+    fill = get(fill_value, self.proj.fill_value, NINF)
+    red = utils._reduction_code(self.proj.reduction, fused=False)
+    proj = world.proj if world.proj is not None else self.proj
+    tb = getattr(world, "_tracked_box", None)
+    planes = box = None
+    if (tb is not None and tb.plane_box is not None and tb.mask is mask and tb.mask._version == tb.mask_version
+        and tb.plane_box.device == dev and tuple(tb.plane_box.shape) == (b * C, 4)):
+      planes = tb.plane_box
+      box = tb.box if _tracked_box_valid(world, proj, dev) else None
+    track = planes is not None and fill == fill and red < 2   # the rectangles assume "mask = beats the merge's fill"
+    if not in_place:
+      copy = lambda t, dt: utils.to_4D_image(t).to(device=dev, dtype=dt).clone(memory_format=torch.contiguous_format)
+      top, mask = copy(top, torch.float32), copy(mask, torch.bool)
+      hm = top if world.is_height_map else copy(hm, torch.float32)
+      if track:
+        planes, box = planes.clone(), None if box is None else box.clone()
+    tgt = nat.DmFuseTarget()
+    tgt.Mh, tgt.Mw = mask.shape[-2], mask.shape[-1]
+    tgt.flip_h, tgt.map_res = bool(proj.flip_h), float(proj.map_res)
+    if track and box is not None:
+      tgt.width_offset, tgt.height_offset = float(proj.width_offset), float(proj.height_offset)
+    tgt.fill_value, tgt.reduction = fill, red
+    with torch.cuda.device(dev):
+      rc = nat.lib().dm_fuse_clear_envs_f32(top.data_ptr(), None if world.is_height_map else hm.data_ptr(),
+                                            mask.data_ptr(), b, C, done_dev.data_ptr(), tgt,
+                                            nat.ptr(planes) if track else None, nat.ptr(box) if track else None,
+                                            nat.stream_ptr(dev))
+    nat.check(rc, "dm_fuse_clear_envs_f32")
+    if not in_place:
+      world = TopdownMap(topdown_map=top, mask=mask, height_map=hm, map_projector=world.proj,
+                         is_height_map=world.is_height_map)
+      self._world_map, self._owned = world, mask
+    if track:
+      world._tracked_box = _TrackedBox(box, mask, proj, planes)
+    elif in_place and tb is not None:
+      world._tracked_box = None   # rectangles that the clear did not update no longer describe the mask
+
+  @staticmethod
+  def _done_flags(done, b: int, dev: torch.device):
+    """reset_envs' `done` as a device buffer of b bytes (0 / 1); a CUDA tensor is used as it is, unread."""
+    if torch.is_tensor(done):
+      if done.dtype is not torch.bool or tuple(done.shape) != (b,):
+        raise ValueError(f"done must be a ({b},) bool tensor, got {done.dtype} {tuple(done.shape)}")
+      if done.is_cuda:
+        if done.device != dev:
+          raise ValueError(f"done is on {done.device}, the world map on {dev}")
+        return done.contiguous()
+      return prm.upload(done.detach(), dev)
+    flags = np.asarray(done)
+    if flags.dtype != np.bool_ or flags.shape != (b,):
+      raise ValueError(f"done must be {b} bools, got {flags.dtype} {flags.shape}")
+    return prm.upload(torch.from_numpy(np.ascontiguousarray(flags)), dev)
 
   def step(self, depth_map: np.ndarray, value_map: Optional[np.ndarray] = None,
            valid_map: Optional[np.ndarray] = None, cam_pose: Optional[np.ndarray] = None,
@@ -1236,15 +1320,19 @@ class MapBuilder():
     (maps.py:2471-2508)."""
     if self._world_map is None:
       self._world_map = TopdownMap(map_projector=self.proj.clone())
-    cam_pose = self._world_map.proj.cam_pose if keep_pose else topdown_map.proj.cam_pose
+    old = self._world_map
+    cam_pose = old.proj.cam_pose if keep_pose else topdown_map.proj.cam_pose
     if self._fixed is not None:
-      self._world_map = merge_into_canvas(self._world_map, topdown_map, canvas_shape=self._fixed,
+      self._world_map = merge_into_canvas(old, topdown_map, canvas_shape=self._fixed,
                                           map_projector=self.proj.clone(cam_pose=cam_pose),
                                           fill_value=fill_value, reduction=reduction)
-      return self._world_map
-    self._world_map = fuse_topdown_maps(self._world_map, topdown_map,
-                                        map_projector=self.proj.clone(cam_pose=cam_pose),
-                                        fill_value=fill_value, reduction=reduction)
+    else:
+      self._world_map = fuse_topdown_maps(old, topdown_map, map_projector=self.proj.clone(cam_pose=cam_pose),
+                                          fill_value=fill_value, reduction=reduction)
+    # both merges return either canvases they allocated, or the tensors of one of the two maps they were given
+    mask = self._world_map.mask
+    fresh = mask is not None and mask is not topdown_map.mask and mask is not old.mask
+    self._owned = mask if fresh or (mask is old.mask and mask is self._owned) else None
     return self._world_map
 
   # ---- the step with its host side in C (csrc/dm_builder.cu) ----------------------------------------------------
@@ -1351,6 +1439,7 @@ class MapBuilder():
           mask = torch.empty((b, 1, Hc, Wc), dtype=torch.bool, device=dev)
           nat.check(lib.dm_fuse_canvas_init_f32(topdown.data_ptr(), mask.data_ptr(), None, topdown.numel(),
                                                 get(fill, NINF), stream), "dm_fuse_canvas_init_f32")
+          self._owned = mask
         else:
           topdown, mask = world.topdown_map, world.mask
         canvas = nat.DmMapRef(topdown.data_ptr(), mask.data_ptr(), Hc, Wc, Wc / 2., Hc / 2., None, None)
@@ -1399,6 +1488,7 @@ class MapBuilder():
       if shape.n_valid == 0:  # maps.py:2217-2225
         self._world_map = TopdownMap(topdown_map=local.topdown_map, mask=local.mask, height_map=local.height_map,
                                      map_projector=target)
+        self._owned = None
         return local
       mh, mw = shape.map_height, shape.map_width
       n_new = b * mh * mw
@@ -1421,7 +1511,7 @@ class MapBuilder():
       merged._tracked_box = _TrackedBox(next_box, mask, new_proj, next_planes)
     # (the scatter pass still reads the old world map and the local map on the stream: torch's caching allocator
     # hands freed blocks to later work of the same stream only, so dropping the old map here is safe)
-    self._world_map = merged
+    self._world_map, self._owned = merged, mask
     return local
 
   def _native_value_step(self, nb: "_NativeBuilder", depth_map, values, labels, C: int, cam_pose, kwargs,
@@ -1459,6 +1549,7 @@ class MapBuilder():
           height = torch.empty_like(topdown)
           nat.check(lib.dm_fuse_canvas_init_f32(topdown.data_ptr(), mask.data_ptr(), height.data_ptr(), topdown.numel(),
                                                 fill, stream), "dm_fuse_canvas_init_f32")
+          self._owned = mask
         else:
           topdown, mask, height = world.topdown_map, world.mask, world.height_map
         canvas = nat.DmValueMapRef(topdown.data_ptr(), height.data_ptr(), mask.data_ptr(), Hc, Wc, Wc / 2., Hc / 2.,
@@ -1497,6 +1588,7 @@ class MapBuilder():
       if shape.n_valid == 0:  # maps.py:2217-2225
         self._world_map = TopdownMap(topdown_map=local.topdown_map, mask=local.mask, height_map=local.height_map,
                                      map_projector=target)
+        self._owned = None
         return local
       mh, mw = shape.map_height, shape.map_width
       n_new = b * C * mh * mw
@@ -1520,7 +1612,7 @@ class MapBuilder():
     merged = TopdownMap(topdown_map=topdown, mask=mask, height_map=height, map_projector=new_proj, is_height_map=False)
     if track:
       merged._tracked_box = _TrackedBox(next_box, mask, new_proj, next_planes)
-    self._world_map = merged
+    self._world_map, self._owned = merged, mask
     return local
 
   def _native_world_ok(self, world: TopdownMap, b: int, dev: torch.device, C: int = 0) -> bool:

@@ -274,6 +274,20 @@ int dm_fuse_inplace_f32(const DmFuseSource* sources, int32_t n_sources, int32_t 
  * n = b*C*Mh*Mw cells. */
 int dm_fuse_canvas_init_f32(float* topdown, uint8_t* mask, float* height, int64_t n, float fill_value,
                             void* stream);
+/* Clears the samples of a batched map that are done (MapBuilder.reset_envs), in place, on the device:
+ *   topdown (b, C, Mh, Mw) f32, height (b, C, Mh, Mw) f32 (NULL for height maps), mask (b, C, Mh, Mw) u8;
+ *   done (b,) u8 device, read by the kernels only: every plane of a sample with done[s] != 0 gets fill_value / -inf / 0,
+ *   whole; the other planes are not touched.
+ *   map: Mh, Mw, flip_h, map_res, width_offset, height_offset, fill_value and reduction of the map.
+ *   plane_box (optional, (b*C, 4) int32 device, 16-byte aligned, as dm_fuse_scatter_track_f32 left it): the cleared
+ *   planes' rectangles become empty (max < min), the others stay.
+ *   box (optional, 5 x int64 device; requires plane_box): rebuilt from the surviving rectangles, what
+ *   dm_fuse_bbox_i64 finds for the cleared map; its count is the number of non-empty planes (zero iff no valid cell).
+ *   With no sample done, plane_box and box are left as they are.
+ * DM_EINVAL for null tensors, b <= 0, C <= 0, a box without plane_box, and a box or plane_box with a NaN fill_value or
+ * reduction >= 2.  No host synchronisation, no copy. */
+int dm_fuse_clear_envs_f32(float* topdown, float* height, uint8_t* mask, int32_t b, int32_t C, const uint8_t* done,
+                           const DmFuseTarget* map, int32_t* plane_box, int64_t* box, void* stream);
 
 /* ---- per-sample parameter blocks packed on the host, in C ------------------------------------------------------
  * What the kernels need per sample derives from a pose (x, z, yaw) and per-call constants.  These two functions are
