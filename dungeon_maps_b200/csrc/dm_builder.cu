@@ -142,23 +142,28 @@ static int builder_create(const DmBuilderCfg* cfg, int C, int labels, int32_t de
 
 extern "C" void dm_builder_destroy(DmBuilder* h) { builder_free(h); }
 
+// The packed parameter slot of a step, on the host and on the device:
+//   [DmProjSample x b | local map's fuse params | world map's fuse params]
+// and a source's fuse params are its steps (b, 2), width offsets (b) and height offsets (b).
+struct FuseParams {
+  float *steps, *woff, *hoff;
+};
+
+static FuseParams fuse_params(char* slot, int b, int source) {  // source 0: the local map, 1: the world map
+  float* p = reinterpret_cast<float*>(slot) + (size_t)b * (kSampleWords + source * kFuseWords);
+  return {p, p + (size_t)b * 2 * kStepWords, p + (size_t)b * (2 * kStepWords + 1)};
+}
+
 // Packs one step's parameter blocks into a pinned slot and queues their upload; returns the slot's device base.
-//   [DmProjSample x b | local fuse params (steps (b,2), woff (b), hoff (b)) | world fuse params (same layout)]
-// world_off: the world map's (width_offset, height_offset), NULL without a world map
+// world: the world map whose offsets the merge uses, NULL without a world map
 static int upload_params(DmBuilder* h, const float* pose, const float* sin_yaw, const float* cos_yaw,
-                         const float* world_off, cudaStream_t stream, char** d_base, int* fast_steps) {
+                         const DmValueMapRef* world, cudaStream_t stream, char** d_base, int* fast_steps) {
   const DmBuilderCfg& c = h->cfg;
   const int b = c.b;
   const unsigned slot = h->next++ % kParamSlots;
   DM_CUDA_OK(cudaEventSynchronize(h->ev[slot]));  // the copy that last read this slot has run (it was queued long ago)
-  float* w = reinterpret_cast<float*>(h->h_params[slot]);
-  float* samples = w;
-  float* lsteps = w + (size_t)b * kSampleWords;
-  float* lwoff = lsteps + (size_t)b * 2 * kStepWords;
-  float* lhoff = lwoff + b;
-  float* wsteps = lhoff + b;
-  float* wwoff = wsteps + (size_t)b * 2 * kStepWords;
-  float* whoff = wwoff + b;
+  float* samples = reinterpret_cast<float*>(h->h_params[slot]);
+  const FuseParams lp = fuse_params(h->h_params[slot], b, 0), wp = fuse_params(h->h_params[slot], b, 1);
   int fast = h->local_fast ? (c.plot_to_global ? 2 : 1) : 0;
   for (int i = 0; i < b; ++i) {
     float Ry[9];
@@ -174,15 +179,15 @@ static int upload_params(DmBuilder* h, const float* pose, const float* sin_yaw, 
     if (fast == 2 && !yaw_step_is_fast(Ry)) fast = 0;
     // the local map as a source of the merge (maps.py:2059-2060): local → global with its own pose, unless it was
     // plotted in the global frame; the target is global (maps.py:2116-2117: no second step)
-    put_step(lsteps + (size_t)i * 2 * kStepWords, c.plot_to_global ? DM_STEP_NONE : DM_STEP_ROT_THEN_ADD, Ry, ty,
+    put_step(lp.steps + (size_t)i * 2 * kStepWords, c.plot_to_global ? DM_STEP_NONE : DM_STEP_ROT_THEN_ADD, Ry, ty,
              h->fused_fuse);
-    put_step(lsteps + (size_t)i * 2 * kStepWords + kStepWords, DM_STEP_NONE, nullptr, nullptr, 0);
-    lwoff[i] = c.width_offset;
-    lhoff[i] = c.height_offset;
-    put_step(wsteps + (size_t)i * 2 * kStepWords, DM_STEP_NONE, nullptr, nullptr, 0);
-    put_step(wsteps + (size_t)i * 2 * kStepWords + kStepWords, DM_STEP_NONE, nullptr, nullptr, 0);
-    wwoff[i] = world_off ? world_off[0] : 0.0f;
-    whoff[i] = world_off ? world_off[1] : 0.0f;
+    put_step(lp.steps + (size_t)i * 2 * kStepWords + kStepWords, DM_STEP_NONE, nullptr, nullptr, 0);
+    lp.woff[i] = c.width_offset;
+    lp.hoff[i] = c.height_offset;
+    put_step(wp.steps + (size_t)i * 2 * kStepWords, DM_STEP_NONE, nullptr, nullptr, 0);
+    put_step(wp.steps + (size_t)i * 2 * kStepWords + kStepWords, DM_STEP_NONE, nullptr, nullptr, 0);
+    wp.woff[i] = world ? world->width_offset : 0.0f;
+    wp.hoff[i] = world ? world->height_offset : 0.0f;
   }
   DM_CUDA_OK(cudaMemcpyAsync(h->d_params[slot], h->h_params[slot], h->param_bytes, cudaMemcpyHostToDevice, stream));
   DM_CUDA_OK(cudaEventRecord(h->ev[slot], stream));
@@ -197,14 +202,7 @@ static int upload_params(DmBuilder* h, const float* pose, const float* sin_yaw, 
 static void make_sources(DmBuilder* h, char* d_base, float* local_topdown, uint8_t* local_mask, float* local_height,
                          const DmValueMapRef* world) {
   const DmBuilderCfg& c = h->cfg;
-  const int b = c.b;
-  float* w = reinterpret_cast<float*>(d_base);
-  float* lsteps = w + (size_t)b * kSampleWords;
-  float* lwoff = lsteps + (size_t)b * 2 * kStepWords;
-  float* lhoff = lwoff + b;
-  float* wsteps = lhoff + b;
-  float* wwoff = wsteps + (size_t)b * 2 * kStepWords;
-  float* whoff = wwoff + b;
+  const FuseParams lp = fuse_params(d_base, c.b, 0), wp = fuse_params(d_base, c.b, 1);
   h->n_src = 0;
   if (world) {  // fuse_topdown_maps(world, new): the world map first (maps.py:2471-2508)
     DmFuseSource& s = h->src[h->n_src++];
@@ -218,7 +216,7 @@ static void make_sources(DmBuilder* h, char* d_base, float* local_topdown, uint8
     }
     s.mask = world->mask;
     s.h = world->h; s.w = world->w; s.flip_h = c.proj.flip_h; s.map_res = c.proj.map_res;
-    s.width_offset = wwoff; s.height_offset = whoff; s.steps = reinterpret_cast<const DmStep*>(wsteps);
+    s.width_offset = wp.woff; s.height_offset = wp.hoff; s.steps = reinterpret_cast<const DmStep*>(wp.steps);
     s.plane_box = world->plane_box;
   }
   DmFuseSource& s = h->src[h->n_src++];
@@ -230,9 +228,144 @@ static void make_sources(DmBuilder* h, char* d_base, float* local_topdown, uint8
     s.height = local_height; s.values = local_topdown; s.height_cstride = 0;
   }
   s.h = c.proj.Mh; s.w = c.proj.Mw; s.flip_h = c.proj.flip_h; s.map_res = c.proj.map_res;
-  s.width_offset = lwoff; s.height_offset = lhoff; s.steps = reinterpret_cast<const DmStep*>(lsteps);
+  s.width_offset = lp.woff; s.height_offset = lp.hoff; s.steps = reinterpret_cast<const DmStep*>(lp.steps);
   s.plane_box = nullptr;
 }
+
+// A height map as the shared code takes it: its topdown map is its height map (height NULL).
+static DmValueMapRef value_ref(const DmMapRef& m) {
+  DmValueMapRef v = {};
+  v.topdown = m.topdown; v.height = nullptr; v.mask = m.mask; v.h = m.h; v.w = m.w;
+  v.width_offset = m.width_offset; v.height_offset = m.height_offset;
+  v.box = m.box; v.plane_box = m.plane_box;
+  return v;
+}
+
+static DmFuseTarget fuse_target(const DmBuilder* h, const DmValueMapRef& m) {
+  const DmBuilderCfg& c = h->cfg;
+  DmFuseTarget t;
+  t.Mh = m.h; t.Mw = m.w; t.flip_h = c.proj.flip_h; t.map_res = c.proj.map_res;
+  t.width_offset = m.width_offset; t.height_offset = m.height_offset;
+  t.fill_value = c.merge_fill_value; t.reduction = c.merge_reduction;
+  return t;
+}
+
+// orth_project(get_height_map=True) of the step: local map and mask; value maps also their one height plane.
+static int project_values(DmBuilder* h, const float* depth, const float* values, const uint8_t* labels, char* d_base,
+                          int fast, float* topdown, uint8_t* mask, float* height, cudaStream_t stream) {
+  DmProjCfg pc = h->cfg.proj;
+  pc.fast_steps = fast;
+  const DmProjSample* samples = reinterpret_cast<const DmProjSample*>(d_base);
+  if (h->labels)
+    return dm_orth_project_labels_f32(depth, labels, nullptr, samples, &pc, h->cfg.b, topdown, mask, height, h->ws,
+                                      h->ws_bytes, stream);
+  return dm_orth_project_f32(depth, values, nullptr, samples, &pc, h->cfg.b, topdown, mask, height, h->ws, h->ws_bytes,
+                             stream);
+}
+
+// The first half of a step for both kinds of handle (height maps: values, labels, local_height and every height NULL):
+// projection, bounding box of world ∪ local, its copy to the host, and the fill of the canvases the caller guessed.
+static int builder_plot(DmBuilder* h, const float* depth, const float* values, const uint8_t* labels, const float* pose,
+                        const float* sin_yaw, const float* cos_yaw, float* local_topdown, uint8_t* local_mask,
+                        float* local_height, const DmValueMapRef* world, DmMergeShape* shape, float* prefill_topdown,
+                        float* prefill_height, uint8_t* prefill_mask, int64_t prefill_cells, cudaStream_t stream) {
+  char* d_base = nullptr;
+  int fast = 0;
+  int rc = upload_params(h, pose, sin_yaw, cos_yaw, world, stream, &d_base, &fast);
+  if (rc != DM_OK) return rc;
+  make_sources(h, d_base, local_topdown, local_mask, local_height, world);
+  // pass 1 (maps.py:2146-2179): a world map that carries the box its own scatter pass tracked only seeds the reduction
+  const bool seeded = world && world->box;
+  bool fused = false;
+  if (h->C == 0) {
+    // the projection's resolve pass and pass 1 over the local map it writes are ONE kernel (dm_fuse.cu:
+    // hmap_resolve_bbox_kernel) whenever the depth-only projection can hand over its key planes
+    DmProjCfg pc = h->cfg.proj;
+    pc.fast_steps = fast;
+    uint32_t* planes = nullptr;
+    unsigned long long slot_words = 0;
+    rc = hmap_project_keys(depth, nullptr, reinterpret_cast<const DmProjSample*>(d_base), &pc, h->cfg.b, h->ws,
+                           h->ws_bytes, stream, &planes, &slot_words);
+    if (rc != DM_OK && rc != DM_EINVAL) return rc;
+    fused = rc == DM_OK;
+    if (fused) {
+      rc = hmap_resolve_with_bbox(planes, slot_words, &pc, h->cfg.b, local_topdown, local_mask, &h->src[h->n_src - 1],
+                                  h->cfg.proj.map_res, seeded ? world->box : nullptr, h->d_bbox, stream);
+      if (rc != DM_OK) return rc;
+      if (world && !seeded) {  // an untracked world map is scanned as before
+        rc = fuse_bbox_accumulate(h->src, 1, h->cfg.b, 1, h->cfg.proj.map_res, h->d_bbox, stream);
+        if (rc != DM_OK) return rc;
+      }
+    }
+  }
+  if (!fused) {  // value maps, and height maps of more than 64 frames or with the height-map path switched off
+    rc = project_values(h, depth, values, labels, d_base, fast, local_topdown, local_mask, local_height, stream);
+    if (rc != DM_OK) return rc;
+    const DmFuseSource* scan = seeded ? &h->src[h->n_src - 1] : h->src;
+    rc = dm_fuse_bbox_seeded_i64(scan, seeded ? 1 : h->n_src, h->cfg.b, h->C > 0 ? h->C : 1, h->cfg.proj.map_res,
+                                 seeded ? world->box : nullptr, h->d_bbox, stream);
+    if (rc != DM_OK) return rc;
+  }
+  DM_CUDA_OK(cudaMemcpyAsync(h->h_bbox, h->d_bbox, 5 * sizeof(int64_t), cudaMemcpyDeviceToHost, stream));
+  DM_CUDA_OK(cudaEventRecord(h->ev_bbox, stream));
+  h->prefilled_top = nullptr; h->prefilled_height = nullptr; h->prefilled_mask = nullptr; h->prefilled_cells = 0;
+  prefill_cells &= ~(int64_t)15;
+  if (prefill_topdown && prefill_mask && (h->C == 0 || prefill_height) && prefill_cells > 0) {
+    rc = dm_fuse_canvas_init_f32(prefill_topdown, prefill_mask, prefill_height, prefill_cells, h->cfg.merge_fill_value,
+                                 stream);
+    if (rc != DM_OK) return rc;
+    h->prefilled_top = prefill_topdown; h->prefilled_height = prefill_height; h->prefilled_mask = prefill_mask;
+    h->prefilled_cells = prefill_cells;
+  }
+  return shape ? dm_builder_plot_wait(h, shape) : DM_OK;  // shape == NULL: the caller waits later (dm_builder_plot_wait)
+}
+
+// The second half: fills `out` and scatters the sources builder_plot left into it.
+static int builder_merge(DmBuilder* h, const DmValueMapRef& out, void* stream) {
+  const DmBuilderCfg& c = h->cfg;
+  const int planes = h->C > 0 ? h->C : 1;
+  const DmFuseTarget tgt = fuse_target(h, out);
+  // the prefill covers the first prefilled_cells cells (a multiple of 16: the tail below starts 16-byte aligned) of the
+  // canvases the caller guessed; a map that outgrew the guess gets its tail filled here
+  const int64_t n_cells = (int64_t)c.b * planes * out.h * out.w;  // 64-bit: b * C * h * w passes 2^31 at scale
+  const bool prefilled = out.topdown == h->prefilled_top && out.height == h->prefilled_height &&
+                         out.mask == h->prefilled_mask && h->prefilled_cells > 0;
+  if (prefilled && n_cells > h->prefilled_cells) {
+    const int64_t p = h->prefilled_cells;
+    const int rf = dm_fuse_canvas_init_f32(out.topdown + p, out.mask + p, out.height ? out.height + p : nullptr,
+                                           n_cells - p, c.merge_fill_value, stream);
+    if (rf != DM_OK) return rf;
+  }
+  const int rc = fuse_scatter_track(h->src, h->n_src, c.b, planes, &tgt, out.topdown, out.mask, out.height, out.box,
+                                    out.plane_box, prefilled ? 1 : 0, stream);
+  h->prefilled_top = nullptr; h->prefilled_height = nullptr; h->prefilled_mask = nullptr; h->prefilled_cells = 0;
+  h->n_src = 0;
+  return rc;
+}
+
+// The fixed-canvas step: plot, then merge in place.  For a height handle project_values is the depth-only projection
+// (want_height 0, values and labels NULL).
+static int builder_step_fixed(DmBuilder* h, const float* depth, const float* values, const uint8_t* labels,
+                              const float* pose, const float* sin_yaw, const float* cos_yaw, float* local_topdown,
+                              uint8_t* local_mask, float* local_height, const DmValueMapRef& canvas,
+                              cudaStream_t stream) {
+  char* d_base = nullptr;
+  int fast = 0;
+  int rc = upload_params(h, pose, sin_yaw, cos_yaw, nullptr, stream, &d_base, &fast);
+  if (rc != DM_OK) return rc;
+  rc = project_values(h, depth, values, labels, d_base, fast, local_topdown, local_mask, local_height, stream);
+  if (rc != DM_OK) return rc;
+  make_sources(h, d_base, local_topdown, local_mask, local_height, nullptr);
+  const DmFuseTarget tgt = fuse_target(h, canvas);
+  rc = dm_fuse_inplace_f32(h->src, 1, h->cfg.b, h->C > 0 ? h->C : 1, &tgt, canvas.topdown, canvas.mask, canvas.height,
+                           stream);
+  h->n_src = 0;
+  return rc;
+}
+
+// ---- height maps (dm_builder_create) ------------------------------------------------------------------------------
+
+static bool height_map_ok(const DmMapRef* m) { return m->topdown && m->mask && m->h > 0 && m->w > 0; }
 
 extern "C" int dm_builder_plot(DmBuilder* h, const float* depth, const float* pose, const float* sin_yaw,
                                const float* cos_yaw, float* local_topdown, uint8_t* local_mask, const DmMapRef* world,
@@ -254,60 +387,11 @@ extern "C" int dm_builder_plot_prefill(DmBuilder* h, const float* depth, const f
                                        uint8_t* prefill_mask, int64_t prefill_cells, void* stream_) {
   DM_TRACE();
   if (!h || h->C != 0 || !depth || !pose || !sin_yaw || !cos_yaw || !local_topdown || !local_mask) return DM_EINVAL;
-  if (world && (!world->topdown || !world->mask || world->h <= 0 || world->w <= 0)) return DM_EINVAL;
-  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  char* d_base = nullptr;
-  int fast = 0;
-  const float world_off[2] = {world ? world->width_offset : 0.0f, world ? world->height_offset : 0.0f};
-  int rc = upload_params(h, pose, sin_yaw, cos_yaw, world ? world_off : nullptr, stream, &d_base, &fast);
-  if (rc != DM_OK) return rc;
-  DmProjCfg pc = h->cfg.proj;
-  pc.fast_steps = fast;
-  pc.want_height = 0;  // C == 0: the topdown map is the height map (maps.py:333-334)
-  DmValueMapRef wv = {};
-  if (world) {
-    wv.topdown = world->topdown; wv.mask = world->mask; wv.h = world->h; wv.w = world->w;
-    wv.width_offset = world->width_offset; wv.height_offset = world->height_offset;
-    wv.box = world->box; wv.plane_box = world->plane_box;
-  }
-  make_sources(h, d_base, local_topdown, local_mask, nullptr, world ? &wv : nullptr);
-  // pass 1 (maps.py:2146-2179): a world map that carries the box its own scatter pass tracked only seeds the reduction
-  const bool seeded = world && world->box;
-  // the projection's resolve pass and pass 1 over the local map it writes are ONE kernel (dm_fuse.cu:
-  // hmap_resolve_bbox_kernel) whenever the depth-only projection can hand over its key planes
-  uint32_t* planes = nullptr;
-  unsigned long long slot_words = 0;
-  rc = hmap_project_keys(depth, nullptr, reinterpret_cast<const DmProjSample*>(d_base), &pc, h->cfg.b, h->ws, h->ws_bytes,
-                         stream, &planes, &slot_words);
-  if (rc == DM_OK) {
-    rc = hmap_resolve_with_bbox(planes, slot_words, &pc, h->cfg.b, local_topdown, local_mask, &h->src[h->n_src - 1],
-                                h->cfg.proj.map_res, seeded ? world->box : nullptr, h->d_bbox, stream);
-    if (rc != DM_OK) return rc;
-    if (world && !seeded) {  // an untracked world map is scanned as before
-      rc = fuse_bbox_accumulate(h->src, 1, h->cfg.b, 1, h->cfg.proj.map_res, h->d_bbox, stream);
-      if (rc != DM_OK) return rc;
-    }
-  } else if (rc == DM_EINVAL) {  // more than 64 frames, or the height-map path is switched off: the unfused sequence
-    rc = dm_orth_project_f32(depth, nullptr, nullptr, reinterpret_cast<const DmProjSample*>(d_base), &pc, h->cfg.b,
-                             local_topdown, local_mask, nullptr, h->ws, h->ws_bytes, stream);
-    if (rc != DM_OK) return rc;
-    const DmFuseSource* scan = seeded ? &h->src[h->n_src - 1] : h->src;
-    rc = dm_fuse_bbox_seeded_i64(scan, seeded ? 1 : h->n_src, h->cfg.b, 1, h->cfg.proj.map_res,
-                                 seeded ? world->box : nullptr, h->d_bbox, stream);
-    if (rc != DM_OK) return rc;
-  } else {
-    return rc;
-  }
-  DM_CUDA_OK(cudaMemcpyAsync(h->h_bbox, h->d_bbox, 5 * sizeof(int64_t), cudaMemcpyDeviceToHost, stream));
-  DM_CUDA_OK(cudaEventRecord(h->ev_bbox, stream));
-  h->prefilled_top = nullptr; h->prefilled_mask = nullptr; h->prefilled_cells = 0;
-  prefill_cells &= ~(int64_t)15;
-  if (prefill_topdown && prefill_mask && prefill_cells > 0) {
-    rc = dm_fuse_canvas_init_f32(prefill_topdown, prefill_mask, nullptr, prefill_cells, h->cfg.merge_fill_value, stream);
-    if (rc != DM_OK) return rc;
-    h->prefilled_top = prefill_topdown; h->prefilled_mask = prefill_mask; h->prefilled_cells = prefill_cells;
-  }
-  return shape ? dm_builder_plot_wait(h, shape) : DM_OK;  // shape == NULL: the caller waits later (dm_builder_plot_wait)
+  if (world && !height_map_ok(world)) return DM_EINVAL;
+  const DmValueMapRef wv = world ? value_ref(*world) : DmValueMapRef{};
+  return builder_plot(h, depth, nullptr, nullptr, pose, sin_yaw, cos_yaw, local_topdown, local_mask, nullptr,
+                      world ? &wv : nullptr, shape, prefill_topdown, nullptr, prefill_mask, prefill_cells,
+                      static_cast<cudaStream_t>(stream_));
 }
 
 extern "C" int dm_builder_plot_wait(DmBuilder* h, DmMergeShape* shape) {
@@ -329,27 +413,8 @@ extern "C" int dm_builder_plot_wait(DmBuilder* h, DmMergeShape* shape) {
 
 extern "C" int dm_builder_merge(DmBuilder* h, const DmMapRef* out, void* stream_) {
   DM_TRACE();
-  if (!h || h->C != 0 || !out || !out->topdown || !out->mask || out->h <= 0 || out->w <= 0 || h->n_src <= 0)
-    return DM_EINVAL;
-  const DmBuilderCfg& c = h->cfg;
-  DmFuseTarget tgt;
-  tgt.Mh = out->h; tgt.Mw = out->w; tgt.flip_h = c.proj.flip_h; tgt.map_res = c.proj.map_res;
-  tgt.width_offset = out->width_offset; tgt.height_offset = out->height_offset;
-  tgt.fill_value = c.merge_fill_value; tgt.reduction = c.merge_reduction;
-  // the prefill covers the first prefilled_cells cells (a multiple of 16: the tail below starts 16-byte aligned) of the
-  // canvases the caller guessed; a map that outgrew the guess gets its tail filled here
-  const int64_t n_cells = (int64_t)c.b * out->h * out->w;
-  const bool prefilled = out->topdown == h->prefilled_top && out->mask == h->prefilled_mask && h->prefilled_cells > 0;
-  if (prefilled && n_cells > h->prefilled_cells) {
-    const int rf = dm_fuse_canvas_init_f32(out->topdown + h->prefilled_cells, out->mask + h->prefilled_cells, nullptr,
-                                           n_cells - h->prefilled_cells, c.merge_fill_value, stream_);
-    if (rf != DM_OK) return rf;
-  }
-  const int rc = fuse_scatter_track(h->src, h->n_src, c.b, 1, &tgt, out->topdown, out->mask, nullptr, out->box,
-                                    out->plane_box, prefilled ? 1 : 0, stream_);
-  h->prefilled_top = nullptr; h->prefilled_mask = nullptr; h->prefilled_cells = 0;
-  h->n_src = 0;
-  return rc;
+  if (!h || h->C != 0 || !out || !height_map_ok(out) || h->n_src <= 0) return DM_EINVAL;
+  return builder_merge(h, value_ref(*out), stream_);
 }
 
 extern "C" int dm_builder_step_fixed(DmBuilder* h, const float* depth, const float* pose, const float* sin_yaw,
@@ -357,43 +422,12 @@ extern "C" int dm_builder_step_fixed(DmBuilder* h, const float* depth, const flo
                                      const DmMapRef* canvas, void* stream_) {
   DM_TRACE();
   if (!h || h->C != 0 || !depth || !pose || !sin_yaw || !cos_yaw || !local_topdown || !local_mask) return DM_EINVAL;
-  if (!canvas || !canvas->topdown || !canvas->mask || canvas->h <= 0 || canvas->w <= 0) return DM_EINVAL;
-  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  char* d_base = nullptr;
-  int fast = 0;
-  int rc = upload_params(h, pose, sin_yaw, cos_yaw, nullptr, stream, &d_base, &fast);
-  if (rc != DM_OK) return rc;
-  DmProjCfg pc = h->cfg.proj;
-  pc.fast_steps = fast;
-  pc.want_height = 0;
-  rc = dm_orth_project_f32(depth, nullptr, nullptr, reinterpret_cast<const DmProjSample*>(d_base), &pc, h->cfg.b,
-                           local_topdown, local_mask, nullptr, h->ws, h->ws_bytes, stream);
-  if (rc != DM_OK) return rc;
-  make_sources(h, d_base, local_topdown, local_mask, nullptr, nullptr);
-  const DmBuilderCfg& c = h->cfg;
-  DmFuseTarget tgt;
-  tgt.Mh = canvas->h; tgt.Mw = canvas->w; tgt.flip_h = c.proj.flip_h; tgt.map_res = c.proj.map_res;
-  tgt.width_offset = canvas->width_offset; tgt.height_offset = canvas->height_offset;
-  tgt.fill_value = c.merge_fill_value; tgt.reduction = c.merge_reduction;
-  rc = dm_fuse_inplace_f32(h->src, 1, c.b, 1, &tgt, canvas->topdown, canvas->mask, nullptr, stream);
-  h->n_src = 0;
-  return rc;
+  if (!canvas || !height_map_ok(canvas)) return DM_EINVAL;
+  return builder_step_fixed(h, depth, nullptr, nullptr, pose, sin_yaw, cos_yaw, local_topdown, local_mask, nullptr,
+                            value_ref(*canvas), static_cast<cudaStream_t>(stream_));
 }
 
 // ---- value maps (dm_builder_create_values) ----------------------------------------------------------------------
-
-// orth_project(value_map= / label_map=, get_height_map=True) of the step: local map, mask and its one height plane.
-static int project_values(DmBuilder* h, const float* depth, const float* values, const uint8_t* labels, char* d_base,
-                          int fast, float* topdown, uint8_t* mask, float* height, cudaStream_t stream) {
-  DmProjCfg pc = h->cfg.proj;
-  pc.fast_steps = fast;
-  const DmProjSample* samples = reinterpret_cast<const DmProjSample*>(d_base);
-  if (h->labels)
-    return dm_orth_project_labels_f32(depth, labels, nullptr, samples, &pc, h->cfg.b, topdown, mask, height, h->ws,
-                                      h->ws_bytes, stream);
-  return dm_orth_project_f32(depth, values, nullptr, samples, &pc, h->cfg.b, topdown, mask, height, h->ws, h->ws_bytes,
-                             stream);
-}
 
 static bool value_inputs_ok(const DmBuilder* h, const float* depth, const float* values, const uint8_t* labels,
                             const float* pose, const float* sin_yaw, const float* cos_yaw, const float* local_topdown,
@@ -417,57 +451,15 @@ extern "C" int dm_builder_plot_values(DmBuilder* h, const float* depth, const fl
   if (!value_inputs_ok(h, depth, values, labels, pose, sin_yaw, cos_yaw, local_topdown, local_mask, local_height))
     return DM_EINVAL;
   if (world && !value_map_ok(world)) return DM_EINVAL;
-  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  char* d_base = nullptr;
-  int fast = 0;
-  const float world_off[2] = {world ? world->width_offset : 0.0f, world ? world->height_offset : 0.0f};
-  int rc = upload_params(h, pose, sin_yaw, cos_yaw, world ? world_off : nullptr, stream, &d_base, &fast);
-  if (rc != DM_OK) return rc;
-  rc = project_values(h, depth, values, labels, d_base, fast, local_topdown, local_mask, local_height, stream);
-  if (rc != DM_OK) return rc;
-  make_sources(h, d_base, local_topdown, local_mask, local_height, world);
-  // pass 1 (maps.py:2146-2179): a tracked world map only seeds the box; the local map is scanned
-  const bool seeded = world && world->box;
-  const DmFuseSource* scan = seeded ? &h->src[h->n_src - 1] : h->src;
-  rc = dm_fuse_bbox_seeded_i64(scan, seeded ? 1 : h->n_src, h->cfg.b, h->C, h->cfg.proj.map_res,
-                               seeded ? world->box : nullptr, h->d_bbox, stream);
-  if (rc != DM_OK) return rc;
-  DM_CUDA_OK(cudaMemcpyAsync(h->h_bbox, h->d_bbox, 5 * sizeof(int64_t), cudaMemcpyDeviceToHost, stream));
-  DM_CUDA_OK(cudaEventRecord(h->ev_bbox, stream));
-  h->prefilled_top = nullptr; h->prefilled_height = nullptr; h->prefilled_mask = nullptr; h->prefilled_cells = 0;
-  prefill_cells &= ~(int64_t)15;
-  if (prefill_topdown && prefill_height && prefill_mask && prefill_cells > 0) {
-    rc = dm_fuse_canvas_init_f32(prefill_topdown, prefill_mask, prefill_height, prefill_cells, h->cfg.merge_fill_value,
-                                 stream);
-    if (rc != DM_OK) return rc;
-    h->prefilled_top = prefill_topdown; h->prefilled_height = prefill_height; h->prefilled_mask = prefill_mask;
-    h->prefilled_cells = prefill_cells;
-  }
-  return shape ? dm_builder_plot_wait(h, shape) : DM_OK;
+  return builder_plot(h, depth, values, labels, pose, sin_yaw, cos_yaw, local_topdown, local_mask, local_height, world,
+                      shape, prefill_topdown, prefill_height, prefill_mask, prefill_cells,
+                      static_cast<cudaStream_t>(stream_));
 }
 
 extern "C" int dm_builder_merge_values(DmBuilder* h, const DmValueMapRef* out, void* stream_) {
   DM_TRACE();
   if (!h || h->C == 0 || !out || !value_map_ok(out) || h->n_src <= 0) return DM_EINVAL;
-  const DmBuilderCfg& c = h->cfg;
-  DmFuseTarget tgt;
-  tgt.Mh = out->h; tgt.Mw = out->w; tgt.flip_h = c.proj.flip_h; tgt.map_res = c.proj.map_res;
-  tgt.width_offset = out->width_offset; tgt.height_offset = out->height_offset;
-  tgt.fill_value = c.merge_fill_value; tgt.reduction = c.merge_reduction;
-  const int64_t n_cells = (int64_t)c.b * h->C * out->h * out->w;  // 64-bit: b * C * h * w passes 2^31 at scale
-  const bool prefilled = out->topdown == h->prefilled_top && out->height == h->prefilled_height &&
-                         out->mask == h->prefilled_mask && h->prefilled_cells > 0;
-  if (prefilled && n_cells > h->prefilled_cells) {
-    const int64_t p = h->prefilled_cells;
-    const int rf = dm_fuse_canvas_init_f32(out->topdown + p, out->mask + p, out->height + p, n_cells - p,
-                                           c.merge_fill_value, stream_);
-    if (rf != DM_OK) return rf;
-  }
-  const int rc = fuse_scatter_track(h->src, h->n_src, c.b, h->C, &tgt, out->topdown, out->mask, out->height, out->box,
-                                    out->plane_box, prefilled ? 1 : 0, stream_);
-  h->prefilled_top = nullptr; h->prefilled_height = nullptr; h->prefilled_mask = nullptr; h->prefilled_cells = 0;
-  h->n_src = 0;
-  return rc;
+  return builder_merge(h, *out, stream_);
 }
 
 extern "C" int dm_builder_step_fixed_values(DmBuilder* h, const float* depth, const float* values,
@@ -478,20 +470,6 @@ extern "C" int dm_builder_step_fixed_values(DmBuilder* h, const float* depth, co
   if (!value_inputs_ok(h, depth, values, labels, pose, sin_yaw, cos_yaw, local_topdown, local_mask, local_height))
     return DM_EINVAL;
   if (!canvas || !value_map_ok(canvas)) return DM_EINVAL;
-  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  char* d_base = nullptr;
-  int fast = 0;
-  int rc = upload_params(h, pose, sin_yaw, cos_yaw, nullptr, stream, &d_base, &fast);
-  if (rc != DM_OK) return rc;
-  rc = project_values(h, depth, values, labels, d_base, fast, local_topdown, local_mask, local_height, stream);
-  if (rc != DM_OK) return rc;
-  make_sources(h, d_base, local_topdown, local_mask, local_height, nullptr);
-  const DmBuilderCfg& c = h->cfg;
-  DmFuseTarget tgt;
-  tgt.Mh = canvas->h; tgt.Mw = canvas->w; tgt.flip_h = c.proj.flip_h; tgt.map_res = c.proj.map_res;
-  tgt.width_offset = canvas->width_offset; tgt.height_offset = canvas->height_offset;
-  tgt.fill_value = c.merge_fill_value; tgt.reduction = c.merge_reduction;
-  rc = dm_fuse_inplace_f32(h->src, 1, c.b, h->C, &tgt, canvas->topdown, canvas->mask, canvas->height, stream);
-  h->n_src = 0;
-  return rc;
+  return builder_step_fixed(h, depth, values, labels, pose, sin_yaw, cos_yaw, local_topdown, local_mask, local_height,
+                            *canvas, static_cast<cudaStream_t>(stream_));
 }

@@ -933,11 +933,10 @@ def _fuse_source(m: TopdownMap, target: MapProjector, b: int, C: int, n_total: i
   src.steps, src.width_offset, src.height_offset = base, base + 4 * n_step_words, base + 4 * (n_step_words + b)
   # a map this module wrote carries, per plane, the rectangle that holds its valid cells: the passes scan that instead
   # of the whole plane (a grown world map is mostly empty canvas)
-  tb = getattr(m, "_tracked_box", None)
-  if (tb is not None and tb.plane_box is not None and m.mask is tb.mask and tb.mask._version == tb.mask_version
-      and tb.plane_box.device == dev and tuple(m.mask.shape) == (b, C, h, w)):
-    src.plane_box = tb.plane_box.data_ptr()
-    keep.append(tb.plane_box)
+  planes = _tracked_planes(m, dev, b * C)
+  if planes is not None:
+    src.plane_box = planes.data_ptr()
+    keep.append(planes)
   return src
 
 
@@ -1048,6 +1047,16 @@ def _tracked_box_valid(m: TopdownMap, target: MapProjector, dev: torch.device) -
           and float(target.map_res) == tb.key[2])
 
 
+def _tracked_planes(m: TopdownMap, dev: torch.device, n_planes: int) -> Optional[torch.Tensor]:
+  """The per-plane rectangles m carries (_TrackedBox.plane_box) while they still describe its mask: the same mask
+  tensor at the same version, rectangles on `dev`, one row for each of n_planes planes.  Else None."""
+  tb = getattr(m, "_tracked_box", None)
+  if (tb is None or tb.plane_box is None or m.mask is not tb.mask or tb.mask._version != tb.mask_version
+      or tb.plane_box.device != dev or tb.plane_box.shape[0] != n_planes):
+    return None
+  return tb.plane_box
+
+
 def merge_into_canvas(world: TopdownMap, new_map: TopdownMap, canvas_shape: Tuple[int, int],
                       map_projector: MapProjector, fill_value: Optional[float] = None,
                       reduction: Optional[Reduction] = None) -> TopdownMap:
@@ -1102,7 +1111,10 @@ def merge_into_canvas(world: TopdownMap, new_map: TopdownMap, canvas_shape: Tupl
 # ======== MapBuilder (maps.py:2289-2550) ==========================================================
 
 class _NativeBuilder():
-  """Owner of one DmBuilder handle (csrc/dm_builder.cu): a MapBuilder's step configuration frozen into C."""
+  """Owner of one DmBuilder handle (csrc/dm_builder.cu): a MapBuilder's step configuration frozen into C.  A height-map
+  handle (C = 0) takes dm_builder_plot_prefill / _merge / _step_fixed and DmMapRef, a value-map handle the *_values
+  entries and DmValueMapRef; the methods below are the one place that tells the two apart.  A map's canvases travel as
+  (topdown, mask), with a value map's heights third."""
 
   def __init__(self, proj: MapProjector, key: tuple, dev: torch.device):
     (b, H, W, _, plot_global, woff, hoff, Mw, Mh, pitch, camh, res, _, _, tdmin, tdmax, thmax, clip, flip, fill,
@@ -1132,6 +1144,8 @@ class _NativeBuilder():
     self.fill = get(fill, NINF)                       # maps.py:2246: get(fill_value, proj.fill_value, NINF)
     cfg.merge_fill_value = self.fill
     cfg.merge_reduction = red
+    self.C = C
+    self.dtypes = (torch.float32, torch.bool) + ((torch.float32,) if C else ())  # of the canvases
     self._lib = nat.lib()
     handle = nat.ctypes.c_void_p()
     with torch.cuda.device(dev):
@@ -1141,6 +1155,56 @@ class _NativeBuilder():
         nat.check(self._lib.dm_builder_create_values(cfg, int(kind == "labels"), dev.index, nat.ctypes.byref(handle)),
                   "dm_builder_create_values")
     self.handle = handle
+
+  def canvases(self, m: TopdownMap) -> tuple:
+    return (m.topdown_map, m.mask) + ((m.height_map,) if self.C else ())
+
+  def map_ref(self, canvases, h: int, w: int, width_offset: float, height_offset: float, box=None, planes=None):
+    """The DmMapRef / DmValueMapRef of (h, w) `canvases` with these offsets and tracked boxes (None: not tracked)."""
+    top, mask = canvases[0].data_ptr(), canvases[1].data_ptr()
+    if self.C == 0:
+      return nat.DmMapRef(top, mask, h, w, width_offset, height_offset, nat.ptr(box), nat.ptr(planes))
+    return nat.DmValueMapRef(top, canvases[2].data_ptr(), mask, h, w, width_offset, height_offset, nat.ptr(box),
+                             nat.ptr(planes))
+
+  def inputs(self, depth, values, labels, pose, sin, cos, local) -> tuple:
+    """The leading arguments of plot() and step_fixed(): the frame, the poses with the sin / cos of their yaws, and
+    the local map's canvases (a value map's with its one height plane)."""
+    if self.C == 0:
+      return (depth.data_ptr(), pose.data_ptr(), sin.data_ptr(), cos.data_ptr(), local[0].data_ptr(),
+              local[1].data_ptr())
+    return (depth.data_ptr(), nat.ptr(values), nat.ptr(labels), pose.data_ptr(), sin.data_ptr(), cos.data_ptr(),
+            local[0].data_ptr(), local[1].data_ptr(), local[2].data_ptr())
+
+  def plot(self, inputs: tuple, world, spec: Optional[list], n_guess: int, stream: int) -> None:
+    """Queues the projection, the bounding box's reduction and copy, and the fill of the first n_guess cells of the
+    speculative canvases `spec` (None: none); wait() blocks for the box."""
+    top, mask, *height = [nat.ptr(t) for t in spec] if spec is not None else [None] * len(self.dtypes)
+    lib = nat.lib()
+    if self.C == 0:
+      nat.check(lib.dm_builder_plot_prefill(self.handle, *inputs, world, None, top, mask, n_guess, stream),
+                "dm_builder_plot_prefill")
+    else:
+      nat.check(lib.dm_builder_plot_values(self.handle, *inputs, world, None, top, *height, mask, n_guess, stream),
+                "dm_builder_plot_values")
+
+  def wait(self) -> "nat.DmMergeShape":
+    shape = nat.DmMergeShape()
+    nat.check(nat.lib().dm_builder_plot_wait(self.handle, shape), "dm_builder_plot_wait")
+    return shape
+
+  def merge(self, out, stream: int) -> None:
+    if self.C == 0:
+      nat.check(nat.lib().dm_builder_merge(self.handle, out, stream), "dm_builder_merge")
+    else:
+      nat.check(nat.lib().dm_builder_merge_values(self.handle, out, stream), "dm_builder_merge_values")
+
+  def step_fixed(self, inputs: tuple, canvas, stream: int) -> None:
+    if self.C == 0:
+      nat.check(nat.lib().dm_builder_step_fixed(self.handle, *inputs, canvas, stream), "dm_builder_step_fixed")
+    else:
+      nat.check(nat.lib().dm_builder_step_fixed_values(self.handle, *inputs, canvas, stream),
+                "dm_builder_step_fixed_values")
 
   def close(self):
     """Destroys the handle (dm_builder_destroy synchronises with the work it queued)."""
@@ -1231,11 +1295,8 @@ class MapBuilder():
     red = utils._reduction_code(self.proj.reduction, fused=False)
     proj = world.proj if world.proj is not None else self.proj
     tb = getattr(world, "_tracked_box", None)
-    planes = box = None
-    if (tb is not None and tb.plane_box is not None and tb.mask is mask and tb.mask._version == tb.mask_version
-        and tb.plane_box.device == dev and tuple(tb.plane_box.shape) == (b * C, 4)):
-      planes = tb.plane_box
-      box = tb.box if _tracked_box_valid(world, proj, dev) else None
+    planes = _tracked_planes(world, dev, b * C)
+    box = tb.box if planes is not None and _tracked_box_valid(world, proj, dev) else None
     track = planes is not None and fill == fill and red < 2   # the rectangles assume "mask = beats the merge's fill"
     if not in_place:
       copy = lambda t, dt: utils.to_4D_image(t).to(device=dev, dtype=dt).clone(memory_format=torch.contiguous_format)
@@ -1376,16 +1437,18 @@ class MapBuilder():
     return "values", int(value_map.shape[1]), value_map, None
 
   def _native_step(self, depth_map, value_map, cam_pose, center_mode, kwargs) -> Optional[TopdownMap]:
-    """MapBuilder.step for the case dm_builder_* covers; None when the call needs the general path."""
+    """MapBuilder.step for the case dm_builder_* covers; None when the call needs the general path.  One sequence for
+    height maps (C = 0: one plane) and value maps (C planes, their heights as C planes of the world map and one plane
+    of the local map)."""
     proj = self.proj
     if (CenterMode(center_mode) is not CenterMode.none or not set(kwargs) <= self._NATIVE_KW or not proj.to_global
         or not torch.is_tensor(depth_map) or not depth_map.is_cuda or depth_map.dtype is not torch.float32
         or depth_map.dim() != 4 or depth_map.shape[1] != 1 or not depth_map.is_contiguous()):
       return None
-    inputs = self._native_values(depth_map, value_map, kwargs)
-    if inputs is None:
+    picked = self._native_values(depth_map, value_map, kwargs)
+    if picked is None:
       return None
-    kind, C, values, labels = inputs
+    kind, C, values, labels = picked
     kwargs = {k: v for k, v in kwargs.items() if k not in ("label_map", "num_classes")}
     get_kw = lambda name: get(kwargs.get(name), getattr(proj, name))
     scalars = [proj.cam_pitch, proj.cam_height, proj.map_res, get_kw("width_offset"), get_kw("height_offset"),
@@ -1413,207 +1476,96 @@ class MapBuilder():
            float(proj.map_res), proj.hfov, proj.vfov, proj.trunc_depth_min, proj.trunc_depth_max,
            proj.trunc_height_max, proj.clip_border, bool(proj.flip_h), fill, red, kind, C)
     nb = self._native_handle(key, dev)
-    if C > 0:
-      return self._native_value_step(nb, depth_map, values, labels, C, cam_pose, kwargs, have_world, woff, hoff, Mw, Mh)
+    n = max(C, 1)   # planes per environment
     pose = prm.per_sample(cam_pose, b, (3,), "cam_pose").contiguous()
     # utils.py:325-326 with the reference's own torch-CPU ops (the last ulp of sin / cos matters)
     sin, cos = prm.yaw_sin_cos(pose)
-    local_top = torch.empty((b, 1, Mh, Mw), dtype=torch.float32, device=dev)
-    local_mask = torch.empty((b, 1, Mh, Mw), dtype=torch.bool, device=dev)
-    lib = nat.lib()
+    local = (torch.empty((b, n, Mh, Mw), dtype=torch.float32, device=dev),
+             torch.empty((b, n, Mh, Mw), dtype=torch.bool, device=dev))
+    if C:
+      local += (torch.empty((b, 1, Mh, Mw), dtype=torch.float32, device=dev),)   # one height plane for all C channels
+    inputs = nb.inputs(depth_map, values, labels, pose, sin, cos, local)
     stream = nat.stream_ptr(dev)
     def make_local():
-      """The local map as plot() describes it (maps.py:2459-2469); offsets as compute_center_offsets returns them.
+      """The local map as plot() describes it (maps.py:2459-2469); offsets as compute_center_offsets returns them, and
+      a value map's height map is the stride-0 expand orth_project returns.
       Built AFTER the step's kernels are queued: host bookkeeping belongs behind GPU work, not in front of it."""
       local_kw = {k: v for k, v in kwargs.items() if k in _CTOR_ARGS}
       local_kw["width_offset"] = torch.tensor([woff], dtype=torch.float32)
       local_kw["height_offset"] = torch.tensor([hoff], dtype=torch.float32)
-      return TopdownMap(topdown_map=local_top, mask=local_mask, height_map=local_top,
-                        map_projector=proj.clone(cam_pose=cam_pose, **local_kw), is_height_map=True)
+      top, mask = local[:2]
+      height = torch.broadcast_to(local[2], top.shape) if C else top
+      return TopdownMap(topdown_map=top, mask=mask, height_map=height,
+                        map_projector=proj.clone(cam_pose=cam_pose, **local_kw), is_height_map=C == 0)
+    def world_map(canvases, map_projector):
+      return TopdownMap(topdown_map=canvases[0], mask=canvases[1], height_map=canvases[2] if C else canvases[0],
+                        map_projector=map_projector, is_height_map=C == 0)
     target = proj.clone(cam_pose=cam_pose)
     with torch.cuda.device(dev):
       if self._fixed is not None:
         Hc, Wc = self._fixed
-        if not have_world:
-          topdown = torch.empty((b, 1, Hc, Wc), dtype=torch.float32, device=dev)
-          mask = torch.empty((b, 1, Hc, Wc), dtype=torch.bool, device=dev)
-          nat.check(lib.dm_fuse_canvas_init_f32(topdown.data_ptr(), mask.data_ptr(), None, topdown.numel(),
-                                                get(fill, NINF), stream), "dm_fuse_canvas_init_f32")
-          self._owned = mask
+        if have_world:
+          canvases = nb.canvases(world)
         else:
-          topdown, mask = world.topdown_map, world.mask
-        canvas = nat.DmMapRef(topdown.data_ptr(), mask.data_ptr(), Hc, Wc, Wc / 2., Hc / 2., None, None)
-        nat.check(lib.dm_builder_step_fixed(nb.handle, depth_map.data_ptr(), pose.data_ptr(), sin.data_ptr(),
-                                            cos.data_ptr(), local_top.data_ptr(), local_mask.data_ptr(), canvas,
-                                            stream), "dm_builder_step_fixed")
-        self._world_map = TopdownMap(
-          topdown_map=topdown, mask=mask, height_map=topdown, is_height_map=True,
-          map_projector=target.clone(to_global=True, width_offset=Wc / 2., height_offset=Hc / 2., map_width=Wc,
-                                     map_height=Hc))
+          canvases = [torch.empty((b, n, Hc, Wc), dtype=dt, device=dev) for dt in nb.dtypes]
+          top, mask, height = canvases[0], canvases[1], canvases[2] if C else None
+          nat.check(nat.lib().dm_fuse_canvas_init_f32(top.data_ptr(), mask.data_ptr(), nat.ptr(height), top.numel(),
+                                                      nb.fill, stream), "dm_fuse_canvas_init_f32")
+          self._owned = canvases[1]
+        nb.step_fixed(inputs, nb.map_ref(canvases, Hc, Wc, Wc / 2., Hc / 2.), stream)
+        self._world_map = world_map(canvases, target.clone(to_global=True, width_offset=Wc / 2., height_offset=Hc / 2.,
+                                                           map_width=Wc, map_height=Hc))
         return make_local()
       wref = None
       if have_world:
         box = world._tracked_box.box if _tracked_box_valid(world, target, dev) else None
-        tb = getattr(world, "_tracked_box", None)
-        planes = None
-        if (tb is not None and tb.plane_box is not None and world.mask is tb.mask
-            and tb.mask._version == tb.mask_version and tb.plane_box.device == dev):
-          planes = tb.plane_box
-        wref = nat.DmMapRef(world.topdown_map.data_ptr(), world.mask.data_ptr(), world.mask.shape[-2],
-                            world.mask.shape[-1], float(world.proj.width_offset), float(world.proj.height_offset),
-                            nat.ptr(box), nat.ptr(planes))
-      shape = nat.DmMergeShape()
+        wref = nb.map_ref(nb.canvases(world), world.mask.shape[-2], world.mask.shape[-1],
+                          float(world.proj.width_offset), float(world.proj.height_offset), box,
+                          _tracked_planes(world, dev, b * n))
       # Everything the merge needs that does not depend on the bounding box is set up BEFORE the call that waits for it:
       # the GPU idles from the moment the box arrives until the merge kernels are queued.  The new canvas is as a rule
       # in the size class of the old one (the map grows by a few cells per step), so canvases of that class are taken
       # from the allocator ahead of the sync and only replaced when the box asks for more.
       track = nb.fill == nb.fill
       next_box = torch.empty((5,), dtype=torch.int64, device=dev) if track else None
-      next_planes = torch.empty((b, 4), dtype=torch.int32, device=dev) if track else None
-      spec_top = spec_mask = None
+      next_planes = torch.empty((b * n, 4), dtype=torch.int32, device=dev) if track else None
+      spec = None
       if have_world and world.mask.numel() >= (1 << 18):
         cap = _canvas_cap(world.mask.numel())
-        spec_top = torch.empty((cap,), dtype=torch.float32, device=dev)
-        spec_mask = torch.empty((cap,), dtype=torch.bool, device=dev)
+        spec = [torch.empty((cap,), dtype=dt, device=dev) for dt in nb.dtypes]
       # ... and their fill is queued behind the box's copy: it runs while the host waits for the box
-      # (prefilled: the old map's cells + 2 % — the map grows by a row or a column now and then; dm_builder_merge fills
+      # (prefilled: the old map's cells + 2 % — the map grows by a row or a column now and then; the merge fills
       # whatever tail the new map has beyond that, and the rest of the size class stays untouched)
-      n_guess = 0 if spec_top is None else min(spec_top.numel(), world.mask.numel() + world.mask.numel() // 50 + 4096)
-      nat.check(lib.dm_builder_plot_prefill(nb.handle, depth_map.data_ptr(), pose.data_ptr(), sin.data_ptr(),
-                                            cos.data_ptr(), local_top.data_ptr(), local_mask.data_ptr(), wref, None,
-                                            nat.ptr(spec_top), nat.ptr(spec_mask), n_guess, stream),
-                "dm_builder_plot_prefill")
-      local = make_local()  # while the projection, the box reduction and the prefill run
-      nat.check(lib.dm_builder_plot_wait(nb.handle, shape), "dm_builder_plot_wait")
-      if shape.n_valid == 0:  # maps.py:2217-2225
-        self._world_map = TopdownMap(topdown_map=local.topdown_map, mask=local.mask, height_map=local.height_map,
-                                     map_projector=target)
-        self._owned = None
-        return local
-      mh, mw = shape.map_height, shape.map_width
-      n_new = b * mh * mw
-      if spec_top is not None and (1 << 18) <= n_new <= spec_top.numel():
-        topdown = spec_top[:n_new].view(b, 1, mh, mw)
-        mask = spec_mask[:n_new].view(b, 1, mh, mw)
-      else:
-        topdown = _alloc_canvas((b, 1, mh, mw), torch.float32, dev)
-        mask = _alloc_canvas((b, 1, mh, mw), torch.bool, dev)
-      spec_top = spec_mask = None
-      out = nat.DmMapRef(topdown.data_ptr(), mask.data_ptr(), mh, mw, shape.width_offset, shape.height_offset,
-                         nat.ptr(next_box), nat.ptr(next_planes))
-      nat.check(lib.dm_builder_merge(nb.handle, out, stream), "dm_builder_merge")
-    new_proj = target.clone(width_offset=torch.tensor([shape.width_offset], dtype=torch.float32),
-                            height_offset=torch.tensor([shape.height_offset], dtype=torch.float32),
-                            map_width=mw, map_height=mh)
-    merged = TopdownMap(topdown_map=topdown, mask=mask, height_map=topdown, map_projector=new_proj,
-                        is_height_map=True)
-    if track:
-      merged._tracked_box = _TrackedBox(next_box, mask, new_proj, next_planes)
-    # (the scatter pass still reads the old world map and the local map on the stream: torch's caching allocator
-    # hands freed blocks to later work of the same stream only, so dropping the old map here is safe)
-    self._world_map, self._owned = merged, mask
-    return local
-
-  def _native_value_step(self, nb: "_NativeBuilder", depth_map, values, labels, C: int, cam_pose, kwargs,
-                         have_world: bool, woff: float, hoff: float, Mw: int, Mh: int) -> TopdownMap:
-    """_native_step for value maps (dm_builder_plot_values / _merge_values / _step_fixed_values): the same sequence as
-    the height-map step with (b, C, h, w) maps, their height planes, and (b * C, 4) plane boxes."""
-    proj, world = self.proj, self._world_map
-    dev = depth_map.device
-    b = depth_map.shape[0]
-    cam_pose = get(cam_pose, proj.cam_pose, np.array([0., 0., 0.], dtype=np.float32))
-    pose = prm.per_sample(cam_pose, b, (3,), "cam_pose").contiguous()
-    sin, cos = prm.yaw_sin_cos(pose)  # utils.py:325-326 with the reference's own torch-CPU ops
-    local_top = torch.empty((b, C, Mh, Mw), dtype=torch.float32, device=dev)
-    local_mask = torch.empty((b, C, Mh, Mw), dtype=torch.bool, device=dev)
-    local_height = torch.empty((b, 1, Mh, Mw), dtype=torch.float32, device=dev)
-    lib = nat.lib()
-    stream = nat.stream_ptr(dev)
-    inputs = (depth_map.data_ptr(), nat.ptr(values), nat.ptr(labels), pose.data_ptr(), sin.data_ptr(), cos.data_ptr(),
-              local_top.data_ptr(), local_mask.data_ptr(), local_height.data_ptr())
-    def make_local():
-      """The local map as plot() describes it: the height map is the stride-0 expand orth_project returns."""
-      local_kw = {k: v for k, v in kwargs.items() if k in _CTOR_ARGS}
-      local_kw["width_offset"] = torch.tensor([woff], dtype=torch.float32)
-      local_kw["height_offset"] = torch.tensor([hoff], dtype=torch.float32)
-      return TopdownMap(topdown_map=local_top, mask=local_mask, height_map=torch.broadcast_to(local_height, local_top.shape),
-                        map_projector=proj.clone(cam_pose=cam_pose, **local_kw), is_height_map=False)
-    target = proj.clone(cam_pose=cam_pose)
-    fill = nb.fill
-    with torch.cuda.device(dev):
-      if self._fixed is not None:
-        Hc, Wc = self._fixed
-        if not have_world:
-          topdown = torch.empty((b, C, Hc, Wc), dtype=torch.float32, device=dev)
-          mask = torch.empty((b, C, Hc, Wc), dtype=torch.bool, device=dev)
-          height = torch.empty_like(topdown)
-          nat.check(lib.dm_fuse_canvas_init_f32(topdown.data_ptr(), mask.data_ptr(), height.data_ptr(), topdown.numel(),
-                                                fill, stream), "dm_fuse_canvas_init_f32")
-          self._owned = mask
-        else:
-          topdown, mask, height = world.topdown_map, world.mask, world.height_map
-        canvas = nat.DmValueMapRef(topdown.data_ptr(), height.data_ptr(), mask.data_ptr(), Hc, Wc, Wc / 2., Hc / 2.,
-                                   None, None)
-        nat.check(lib.dm_builder_step_fixed_values(nb.handle, *inputs, canvas, stream), "dm_builder_step_fixed_values")
-        self._world_map = TopdownMap(
-          topdown_map=topdown, mask=mask, height_map=height, is_height_map=False,
-          map_projector=target.clone(to_global=True, width_offset=Wc / 2., height_offset=Hc / 2., map_width=Wc,
-                                     map_height=Hc))
-        return make_local()
-      wref = None
-      if have_world:
-        box = world._tracked_box.box if _tracked_box_valid(world, target, dev) else None
-        tb = getattr(world, "_tracked_box", None)
-        planes = None
-        if (tb is not None and tb.plane_box is not None and world.mask is tb.mask
-            and tb.mask._version == tb.mask_version and tb.plane_box.device == dev):
-          planes = tb.plane_box
-        wref = nat.DmValueMapRef(world.topdown_map.data_ptr(), world.height_map.data_ptr(), world.mask.data_ptr(),
-                                 world.mask.shape[-2], world.mask.shape[-1], float(world.proj.width_offset),
-                                 float(world.proj.height_offset), nat.ptr(box), nat.ptr(planes))
-      shape = nat.DmMergeShape()
-      track = fill == fill
-      next_box = torch.empty((5,), dtype=torch.int64, device=dev) if track else None
-      next_planes = torch.empty((b * C, 4), dtype=torch.int32, device=dev) if track else None
-      spec = None  # canvases of the old map's size class, filled while the host waits for the box (see _native_step)
-      if have_world and world.mask.numel() >= (1 << 18):
-        cap = _canvas_cap(world.mask.numel())
-        spec = (torch.empty((cap,), dtype=torch.float32, device=dev), torch.empty((cap,), dtype=torch.float32, device=dev),
-                torch.empty((cap,), dtype=torch.bool, device=dev))
       n_guess = 0 if spec is None else min(spec[0].numel(), world.mask.numel() + world.mask.numel() // 50 + 4096)
-      nat.check(lib.dm_builder_plot_values(nb.handle, *inputs, wref, None, *[nat.ptr(t) for t in (spec or (None,) * 3)],
-                                           n_guess, stream), "dm_builder_plot_values")
-      local = make_local()
-      nat.check(lib.dm_builder_plot_wait(nb.handle, shape), "dm_builder_plot_wait")
+      nb.plot(inputs, wref, spec, n_guess, stream)
+      local_map = make_local()  # while the projection, the box reduction and the prefill run
+      shape = nb.wait()
       if shape.n_valid == 0:  # maps.py:2217-2225
-        self._world_map = TopdownMap(topdown_map=local.topdown_map, mask=local.mask, height_map=local.height_map,
-                                     map_projector=target)
+        self._world_map = TopdownMap(topdown_map=local_map.topdown_map, mask=local_map.mask,
+                                     height_map=local_map.height_map, map_projector=target)
         self._owned = None
-        return local
+        return local_map
       mh, mw = shape.map_height, shape.map_width
-      n_new = b * C * mh * mw
+      n_new = b * n * mh * mw
       if spec is not None and (1 << 18) <= n_new <= spec[0].numel():
-        topdown, height, mask = (t[:n_new].view(b, C, mh, mw) for t in spec)
+        canvases = [t[:n_new].view(b, n, mh, mw) for t in spec]
       else:
         # the map outgrew the guess: the speculative canvases go back to the allocator BEFORE the new ones are taken,
-        # so that three C-channel canvases of the old class are not held next to the old map and the new one
+        # so that canvases of the old class are not held next to the old map and the new one
         # (the prefill queued on them is ordered before any later use of their blocks on this stream)
         spec = None
-        topdown = _alloc_canvas((b, C, mh, mw), torch.float32, dev)
-        height = _alloc_canvas((b, C, mh, mw), torch.float32, dev)
-        mask = _alloc_canvas((b, C, mh, mw), torch.bool, dev)
-      spec = None
-      out = nat.DmValueMapRef(topdown.data_ptr(), height.data_ptr(), mask.data_ptr(), mh, mw, shape.width_offset,
-                              shape.height_offset, nat.ptr(next_box), nat.ptr(next_planes))
-      nat.check(lib.dm_builder_merge_values(nb.handle, out, stream), "dm_builder_merge_values")
+        canvases = [_alloc_canvas((b, n, mh, mw), dt, dev) for dt in nb.dtypes]
+      nb.merge(nb.map_ref(canvases, mh, mw, shape.width_offset, shape.height_offset, next_box, next_planes), stream)
     new_proj = target.clone(width_offset=torch.tensor([shape.width_offset], dtype=torch.float32),
                             height_offset=torch.tensor([shape.height_offset], dtype=torch.float32),
                             map_width=mw, map_height=mh)
-    merged = TopdownMap(topdown_map=topdown, mask=mask, height_map=height, map_projector=new_proj, is_height_map=False)
+    merged = world_map(canvases, new_proj)
     if track:
-      merged._tracked_box = _TrackedBox(next_box, mask, new_proj, next_planes)
-    self._world_map, self._owned = merged, mask
-    return local
+      merged._tracked_box = _TrackedBox(next_box, merged.mask, new_proj, next_planes)
+    # (the scatter pass still reads the old world map and the local map on the stream: torch's caching allocator
+    # hands freed blocks to later work of the same stream only, so dropping the old map here is safe)
+    self._world_map, self._owned = merged, merged.mask
+    return local_map
 
   def _native_world_ok(self, world: TopdownMap, b: int, dev: torch.device, C: int = 0) -> bool:
     """The world map is one the C step can take as it is: a contiguous (b, 1, h, w) float32 height map + bool mask

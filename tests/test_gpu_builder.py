@@ -205,10 +205,10 @@ def test_prefilled_canvases_and_their_tail(monkeypatch):
   """The C step fills canvases of the old map's size class before the bounding box is known (the old map's cells + 2 %)
   and dm_builder_merge fills whatever tail the new map has beyond that.  With a generous size class (patched to 2 x) and
   a fast walk the new map regularly lands between the guess and the class: same world maps as the general path, which
-  never speculates."""
+  never speculates.  Height maps, then class ids of a few classes (values, heights and mask canvases)."""
   from dungeon_maps_b200 import maps as dmaps
   monkeypatch.setattr(dmaps, "_canvas_cap", lambda n: 2 * n)
-  b, T, H, W = 8, 8, 120, 160
+  b, T, H, W, C = 8, 8, 120, 160, 3
   poses = _walk(b, T, seed=23, half=12.0)
   def make(native):
     proj = dmap.MapProjector(width=W, height=H, hfov=HFOV, cam_pose=[0., 0., 0.], width_offset=0., height_offset=0.,
@@ -216,18 +216,22 @@ def test_prefilled_canvases_and_their_tail(monkeypatch):
                              trunc_depth_min=0.15, trunc_depth_max=5.05, clip_border=3, fill_value=dmap.NINF,
                              to_global=True, device="cuda")
     return dmap.MapBuilder(map_projector=proj, native_step=native)
-  nb, gb = make(True), make(False)
-  kw = dict(to_global=False, width_offset=100., height_offset=0., map_width=200, map_height=200)
-  grew = 0
-  for t in range(T):
-    depth = synth.room_depth(b, H, W, HFOV, PITCH, 0.88, poses[t].cuda(), seed=23, half=14.0, device="cuda")
-    before = 0 if nb.world_map is None or nb.world_map.is_empty else nb.world_map.mask.numel()
-    nb.step(depth, cam_pose=poses[t], **kw)
-    gb.step(depth, cam_pose=poses[t], **kw)
-    after = nb.world_map.mask.numel()
-    if before >= (1 << 18) and before + before // 50 + 4096 < after <= 2 * before:
-      grew += 1
-    _same_map(nb.world_map, gb.world_map, f"step {t} world")
-  assert nb._handles, "the native path was not taken"
-  assert grew > 0, "no step exercised the tail fill: make the walk faster"
+  for labels in (False, True):
+    nb, gb = make(True), make(False)
+    grew = 0
+    for t in range(T):
+      depth = synth.room_depth(b, H, W, HFOV, PITCH, 0.88, poses[t].cuda(), seed=23, half=14.0, device="cuda")
+      kw = dict(to_global=False, width_offset=100., height_offset=0., map_width=200, map_height=200)
+      if labels:
+        kw.update(label_map=synth.block_labels(b, C, H, W, seed=300 + t, device="cuda"), num_classes=C)
+      before = 0 if nb.world_map is None or nb.world_map.is_empty else nb.world_map.mask.numel()
+      nb.step(depth, cam_pose=poses[t], **kw)
+      gb.step(depth, cam_pose=poses[t], **kw)
+      after = nb.world_map.mask.numel()
+      if before >= (1 << 18) and before + before // 50 + 4096 < after <= 2 * before:
+        grew += 1
+      _same_map(nb.world_map, gb.world_map, f"labels={labels} step {t} world")
+    assert nb._handles, "the native path was not taken"
+    assert nb.world_map.is_height_map != labels
+    assert grew > 0, f"labels={labels}: no step exercised the tail fill: make the walk faster"
   assert_workspaces_clean()

@@ -223,11 +223,14 @@ def test_mixed_paths():
   poses = _walk(b, T, seed=19)
   nb, gb = _builder(True, fill=0.), _builder(False, fill=0.)
   c_steps = []   # (step, world map the C step started from) of every step the C step took
-  c_step = nb._native_value_step
+  c_step = nb._native_step
   def spy(*args, **kwargs):
-    c_steps.append((t, nb.world_map))
-    return c_step(*args, **kwargs)
-  nb._native_value_step = spy
+    started_from = nb.world_map
+    local = c_step(*args, **kwargs)
+    if local is not None:
+      c_steps.append((t, started_from))
+    return local
+  nb._native_step = spy
   for t in range(T):
     depth = _depth(b, poses[t], 19)
     kw = dict(LOCAL, **_inputs("onehot", b, C, t))

@@ -48,8 +48,13 @@ def test_create_values_refuses_null_pointers():
   handle = ctypes.c_void_p()
   assert lib.dm_builder_create_values(None, 0, 0, ctypes.byref(handle)) == -1
   assert lib.dm_builder_create_values(_cfg(4), 0, 0, None) == -1
-  # the height-map entry keeps refusing value channels, and the value entries refuse a missing handle
+  # the height-map entry keeps refusing value channels, and the step entries of both kinds refuse a missing handle
   assert lib.dm_builder_create(_cfg(4), 0, ctypes.byref(handle)) == -1
   assert lib.dm_builder_merge_values(None, None, None) == -1
   assert lib.dm_builder_plot_values(None, *([None] * 14), 0, None) == -1
   assert lib.dm_builder_step_fixed_values(None, *([None] * 11)) == -1
+  assert lib.dm_builder_plot(None, *([None] * 9)) == -1
+  assert lib.dm_builder_plot_prefill(None, *([None] * 10), 0, None) == -1
+  assert lib.dm_builder_plot_wait(None, None) == -1
+  assert lib.dm_builder_merge(None, None, None) == -1
+  assert lib.dm_builder_step_fixed(None, *([None] * 8)) == -1
