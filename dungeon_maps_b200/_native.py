@@ -92,6 +92,7 @@ class DmMergeShape(ctypes.Structure):
 STEP_WORDS = ctypes.sizeof(DmStep) // 4          # 16
 PROJ_SAMPLE_WORDS = 48                           # DmProjSample: 2 steps + 2 offsets + pad
 FLOW_SAMPLE_WORDS = 48                           # DmFlowSample: 3 steps
+EGO_SAMPLE_WORDS = 20                            # DM_EGO_SAMPLE_WORDS: 1 step + source and window offsets
 
 _SIGNATURES = {
   "dm_abi_version": (ctypes.c_int, []),
@@ -131,6 +132,8 @@ _SIGNATURES = {
   "dm_pack_proj_samples": (ctypes.c_int, [POINTER(DmPoseCfg), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int32,
                                           c_int32, c_void_p, POINTER(c_int32)]),
   "dm_pack_flow_samples": (ctypes.c_int, [POINTER(DmPoseCfg), c_void_p, c_void_p, c_void_p, c_int32, c_void_p]),
+  "dm_pack_ego_samples": (ctypes.c_int, [POINTER(DmPoseCfg), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                         c_void_p, c_int32, c_void_p]),
   "dm_builder_create": (ctypes.c_int, [POINTER(DmBuilderCfg), c_int32, POINTER(c_void_p)]),
   "dm_builder_destroy": (None, [c_void_p]),
   "dm_builder_plot": (ctypes.c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
@@ -165,6 +168,9 @@ _SIGNATURES = {
                                          c_int32, c_float, c_void_p, c_void_p]),
   "dm_crop_nearest_u8": (ctypes.c_int, [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_int32, c_int32,
                                         c_void_p, c_void_p]),
+  "dm_crop_egocentric_f32": (ctypes.c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int32, c_int32, c_int32, c_int32,
+                                            c_float, c_int32, c_void_p, c_int32, c_int32, c_float, c_void_p, c_void_p,
+                                            c_void_p, c_void_p]),
 }
 EXPORTS = tuple(_SIGNATURES)
 

@@ -281,6 +281,31 @@ def flow_samples(pose, pitch, cam_h, n_points: int) -> torch.Tensor:
                     local_to_camera(pitch, cam_h, n_points)), dim=1)
 
 
+_ego_cfgs = {}
+
+
+def ego_samples(pose, src_woff, src_hoff, woff, hoff, n_points: int) -> torch.Tensor:
+  """(b, 20) float32 words of TopdownMap.select_egocentric (DM_EGO_SAMPLE_WORDS): local_to_global(pose, n_points) as a
+  DmStep, then the source map's offsets, then the window's.  Packed in C from torch's sin / cos of the yaws."""
+  fused = int(fused_for(n_points))
+  cfg = _ego_cfgs.get(fused)
+  if cfg is None:  # the packer reads the yaw terms and `fused` only
+    cfg = nat.DmPoseCfg()
+    skew, skew_sq, _ = _skew_terms([0., 1., 0.])
+    cfg.yaw_skew[:] = skew.reshape(-1).tolist()
+    cfg.yaw_skew_sq[:] = skew_sq.reshape(-1).tolist()
+    cfg.fused = fused
+    _ego_cfgs[fused] = cfg
+  b = pose.shape[0]
+  pose = pose.contiguous()
+  sin, cos = yaw_sin_cos(pose)
+  cols = [t.contiguous() for t in (src_woff, src_hoff, woff, hoff)]
+  out = torch.empty((b, nat.EGO_SAMPLE_WORDS), dtype=torch.float32)
+  nat.check(nat.lib().dm_pack_ego_samples(cfg, pose.data_ptr(), sin.data_ptr(), cos.data_ptr(),
+                                          *[t.data_ptr() for t in cols], b, out.data_ptr()), "dm_pack_ego_samples")
+  return out
+
+
 class DeviceBlock:
   """A parameter block uploaded by dm_upload_params: a raw device pointer into the library's ring of slots, valid for
   the work queued on the current stream before the 64th upload after it (every caller hands it to the very next C

@@ -136,6 +136,14 @@ __device__ __forceinline__ void quantize_f(float x, float z, float woff, float h
   *zf = floorf(__fadd_rn(zb, 0.5f));
 }
 
+// maps.py:1021-1087 map_dequantize of the bins (xb, zb), given as floats.
+__device__ __forceinline__ void dequantize_f(float xb, float zb, float woff, float hoff, float res, int Mh,
+                                             int flip_h, float* x, float* z) {
+  if (flip_h) zb = __fsub_rn((float)(Mh - 1), zb);  // maps.py:1081-1084
+  *z = __fmul_rn(__fsub_rn(zb, hoff), res);
+  *x = __fmul_rn(__fsub_rn(xb, woff), res);
+}
+
 // Tensor.to(int64) on x86: cvttss2si semantics.
 __device__ __forceinline__ long long f2i64(float v) {
   if (!(v >= -9223372036854775808.0f && v < 9223372036854775808.0f)) return (long long)0x8000000000000000ULL;

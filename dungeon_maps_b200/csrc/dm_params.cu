@@ -91,3 +91,23 @@ extern "C" int dm_pack_flow_samples(const DmPoseCfg* cfg, const float* pose, con
   }
   return DM_OK;
 }
+
+extern "C" int dm_pack_ego_samples(const DmPoseCfg* cfg, const float* pose, const float* sin_yaw, const float* cos_yaw,
+                                   const float* src_width_offset, const float* src_height_offset,
+                                   const float* width_offset, const float* height_offset, int32_t b, float* out) {
+  if (!cfg || !pose || !sin_yaw || !cos_yaw || !src_width_offset || !src_height_offset || !width_offset ||
+      !height_offset || !out || b < 0)
+    return DM_EINVAL;
+  for (int i = 0; i < b; ++i) {
+    float* sp = out + (size_t)i * DM_EGO_SAMPLE_WORDS;
+    float Ry[9];
+    yaw_matrix(*cfg, pose[3 * i + 2], sin_yaw[i], cos_yaw[i], Ry);
+    const float ty[3] = {pose[3 * i + 0], 0.0f, pose[3 * i + 1]};  // maps.py:889-891
+    put_step(sp, DM_STEP_ROT_THEN_ADD, Ry, ty, cfg->fused);           // local_to_global_space
+    sp[16] = src_width_offset[i];
+    sp[17] = src_height_offset[i];
+    sp[18] = width_offset[i];
+    sp[19] = height_offset[i];
+  }
+  return DM_OK;
+}

@@ -171,10 +171,7 @@ dequantize_kernel(const float* __restrict__ xb, const float* __restrict__ zb, co
                   float* __restrict__ x, float* __restrict__ z) {
   DM_GRID_STRIDE(i, total) {
     const int s = (int)(i / n);
-    float zz = zb[i];
-    if (flip_h) zz = __fsub_rn((float)(Mh - 1), zz);  // maps.py:1081-1084
-    z[i] = __fmul_rn(__fsub_rn(zz, hoff[s]), res);
-    x[i] = __fmul_rn(__fsub_rn(xb[i], woff[s]), res);
+    dequantize_f(xb[i], zb[i], woff[s], hoff[s], res, Mh, flip_h, &x[i], &z[i]);
   }
 }
 
@@ -273,6 +270,47 @@ crop_kernel(const T* __restrict__ image, const float* __restrict__ center, int b
       v = (X >= 1 && X <= w && Y >= 1 && Y <= h) ? image[(sc * h + (Y - 1)) * w + (X - 1)] : fill;
     }
     out[i] = v;
+  }
+}
+
+// TopdownMap.select_egocentric: cell (r, c) of sample s's crop_h x crop_w window is map_dequantize(c, r) with the
+// window's offsets, local_to_global_space with the sample's pose, map_quantize with the source's offsets, and a read
+// of the source there (the fills outside it).  One thread per (sample, cell): the coordinates once, then the C planes.
+// samples: DM_EGO_SAMPLE_WORDS floats per sample, [DmStep | source woff, hoff | window woff, hoff].
+// height: plane stride hplane (0: one plane shared by the C channels, written once), NULL for height maps.
+__global__ void __launch_bounds__(kThreads)
+crop_egocentric_kernel(const float* __restrict__ top, const float* __restrict__ height, long long hplane,
+                       const uint8_t* __restrict__ mask, int b, int C, int Hs, int Ws, float res, int flip_h,
+                       const float* __restrict__ samples, int ch_, int cw_, float fill, float* __restrict__ out_top,
+                       float* __restrict__ out_height, uint8_t* __restrict__ out_mask) {
+  const long long per = (long long)ch_ * cw_;
+  const long long plane = (long long)Hs * Ws;
+  const long long total = (long long)b * per;
+  const int Ch = hplane ? C : 1;  // height planes per sample, in and out
+  DM_GRID_STRIDE(i, total) {
+    const int s = (int)(i / per);
+    const int o = (int)(i - s * per);
+    const int r = o / cw_, c = o - r * cw_;
+    const float* w = samples + (long long)s * DM_EGO_SAMPLE_WORDS;
+    float lx, lz;
+    dequantize_f((float)c, (float)r, w[18], w[19], res, ch_, flip_h, &lx, &lz);
+    const V3 g = apply_step(*reinterpret_cast<const DmStep*>(w), V3{lx, 0.0f, lz});
+    float xf, zf;
+    quantize_f(g.x, g.z, w[16], w[17], res, Hs, flip_h, &xf, &zf);
+    const bool in = xf >= 0.0f && xf < (float)Ws && zf >= 0.0f && zf < (float)Hs;
+    const long long cell = in ? (long long)zf * Ws + (long long)xf : 0;
+    const long long src = (long long)s * C * plane + cell;
+    const long long dst = (long long)s * C * per + o;
+    for (int k = 0; k < C; ++k) {
+      out_top[dst + k * per] = in ? top[src + k * plane] : fill;
+      out_mask[dst + k * per] = in ? mask[src + k * plane] : (uint8_t)0;
+    }
+    if (out_height) {
+      const long long hsrc = (long long)s * Ch * plane + cell;
+      const long long hdst = (long long)s * Ch * per + o;
+      for (int k = 0; k < Ch; ++k)
+        out_height[hdst + k * per] = in ? height[hsrc + k * plane] : -INFINITY;
+    }
   }
 }
 
@@ -415,6 +453,26 @@ extern "C" int dm_crop_nearest_u8(const uint8_t* image, const float* center, int
   // the reference crops masks with fill_value=False → border mode over a ring of zeros
   crop_kernel<uint8_t><<<grid_for(total), kThreads, 0, static_cast<cudaStream_t>(stream)>>>(
       image, center, b, c, h, w, crop_h, crop_w, 1, (uint8_t)0, (uint8_t)0, out);
+  DM_LAUNCHED();
+  return DM_OK;
+}
+
+extern "C" int dm_crop_egocentric_f32(const float* topdown, const float* height, int64_t height_plane_stride,
+                                      const uint8_t* mask, int32_t b, int32_t C, int32_t Hs, int32_t Ws, float map_res,
+                                      int32_t flip_h, const float* samples, int32_t crop_h, int32_t crop_w,
+                                      float fill_value, float* out_topdown, float* out_height, uint8_t* out_mask,
+                                      void* stream) {
+  DM_TRACE();
+  if (b <= 0 || C <= 0 || Hs <= 0 || Ws <= 0 || crop_h <= 0 || crop_w <= 0 || !(map_res > 0.0f)) return DM_EINVAL;
+  if ((long long)crop_h * crop_w >= (1ll << 31) || (long long)Hs * Ws >= (1ll << 31)) return DM_EINVAL;
+  if (!topdown || !mask || !samples || !out_topdown || !out_mask) return DM_EINVAL;
+  if (!height != !out_height) return DM_EINVAL;
+  if (height && height_plane_stride != 0 && height_plane_stride != (int64_t)Hs * Ws) return DM_EINVAL;
+  if (!aligned_to(samples, 4)) return DM_EINVAL;
+  const long long total = (long long)b * crop_h * crop_w;
+  crop_egocentric_kernel<<<grid_for(total), kThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+      topdown, height, height ? height_plane_stride : 0, mask, b, C, Hs, Ws, map_res, flip_h, samples, crop_h, crop_w,
+      fill_value, out_topdown, out_height, out_mask);
   DM_LAUNCHED();
   return DM_OK;
 }

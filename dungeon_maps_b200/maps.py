@@ -43,7 +43,8 @@ __all__ = [
   'height_map_to_point_cloud', 'image_to_camera_space', 'camera_to_image_space', 'camera_to_local_space',
   'local_to_camera_space', 'local_to_global_space', 'global_to_local_space', 'map_quantize',
   'map_dequantize', 'project', 'compute_center_offsets', 'MapProjector', 'TopdownMap', 'crop_topdown_map',
-  'fuse_topdown_maps', 'merge_into_canvas', 'MapBuilder', 'release_workspaces', 'Reduction', 'CameraIntrinsics', 'NINF', 'Float3D',
+  'crop_egocentric_map', 'fuse_topdown_maps', 'merge_into_canvas', 'MapBuilder', 'release_workspaces', 'Reduction',
+  'CameraIntrinsics', 'NINF', 'Float3D',
 ]
 
 
@@ -836,6 +837,14 @@ class TopdownMap():
     return crop_topdown_map(self, center=center, crop_width=crop_width, crop_height=crop_height,
                             fill_value=fill_value, _validate_args=True)
 
+  def select_egocentric(self, crop_width: int, crop_height: int, cam_pose: Optional[torch.Tensor] = None,
+                        width_offset: Optional[torch.Tensor] = None, height_offset: Optional[torch.Tensor] = None,
+                        fill_value: Optional[float] = None) -> "TopdownMap":
+    """A crop_width × crop_height window per environment in its camera frame (not in the reference);
+    see crop_egocentric_map."""
+    return crop_egocentric_map(self, crop_width=crop_width, crop_height=crop_height, cam_pose=cam_pose,
+                               width_offset=width_offset, height_offset=height_offset, fill_value=fill_value)
+
   def merge(self, *sources: List["TopdownMap"]) -> "TopdownMap":
     raise NotImplementedError
 
@@ -895,6 +904,79 @@ def crop_topdown_map(source: TopdownMap, center: torch.Tensor, crop_width: int, 
                         map_height=crop_height)
   return TopdownMap(topdown_map=topdown_map, mask=mask, height_map=height_map,
                     is_height_map=source.is_height_map, map_projector=new_proj)
+
+
+def crop_egocentric_map(source: TopdownMap, crop_width: int, crop_height: int, cam_pose: Optional[torch.Tensor] = None,
+                        width_offset: Optional[torch.Tensor] = None, height_offset: Optional[torch.Tensor] = None,
+                        fill_value: Optional[float] = None) -> TopdownMap:
+  """The crop_height × crop_width window of a global-frame map that every environment sees in its own camera frame:
+  centred on the agent and turned to its heading, the observation a policy reads each step (not in the reference).
+  Cell (r, c) of environment i is, by definition, the composition of this module's public functions
+      (lx, lz) = map_dequantize(c, r, width_offset[i], height_offset[i], map_res, crop_height, flip_h)
+      (gx, gz) = local_to_global_space((lx, 0, lz), cam_pose[i])        # crop_height * crop_width points per sample
+      (X, Z)   = map_quantize(gx, gz, source offsets[i], map_res, source map_height, flip_h)
+  read from the source at (Z, X), bit for bit; cells outside the source get what a merge leaves in a cell nothing
+  reached: `get(fill_value, proj.fill_value, NINF)` (heights of a value map: -inf; mask: False).  The window has the
+  source's map_res and flip_h; with flip_h the camera's forward direction (+z local) points up.
+
+  cam_pose (1 or b rows of x, z, yaw) defaults to source.proj.cam_pose (a MapBuilder's world map carries the pose of
+  its latest step); width_offset / height_offset (1 or b values) to crop_width / 2 and crop_height / 2, which puts the
+  camera where CenterMode.camera puts it in a local-frame plot; height_offset=0 puts the agent on the bottom row.
+  Poses and offsets are host values uploaded with the parameter block: a CUDA pose tensor is copied to the host, which
+  synchronises with its stream.  One kernel launch (csrc/dm_points.cu crop_egocentric_kernel), no host sync otherwise.
+
+  The result's projector is source.proj.clone(cam_pose=, to_global=False, width_offset=, height_offset=,
+  map_width=crop_width, map_height=crop_height), so its get_camera() is the agent's cell.  A height map stays a height
+  map; a height source that is one plane expanded over the channels (a value map's local map) gives one plane,
+  expanded the same way.  ValueError for an empty or local-frame source, a crop size below 1, and a pose or offset
+  count other than 1 or b; all before any device work."""
+  if source is None or source.is_empty:
+    raise ValueError("select_egocentric needs a map: the source is empty")
+  proj = source.proj
+  if proj is None or not proj.to_global:
+    raise ValueError("select_egocentric reads a global-frame map (proj.to_global); the source is in a local frame")
+  crop_width, crop_height = int(crop_width), int(crop_height)
+  if crop_width < 1 or crop_height < 1:
+    raise ValueError(f"crop size must be at least 1 x 1, got {crop_width} x {crop_height}")
+  top = utils.to_4D_image(source.topdown_map)
+  b, C, Hs, Ws = top.shape
+  pose_host = prm.host_f32(get(cam_pose, proj.cam_pose, [0., 0., 0.]), (3,))
+  pose = prm.per_sample(pose_host, b, (3,), "cam_pose")
+  woff = get(width_offset, crop_width / 2.)
+  hoff = get(height_offset, crop_height / 2.)
+  cols = [prm.per_sample(get(proj.width_offset, 0.), b, (), "source width_offset"),
+          prm.per_sample(get(proj.height_offset, 0.), b, (), "source height_offset"),
+          prm.per_sample(woff, b, (), "width_offset"), prm.per_sample(hoff, b, (), "height_offset")]
+  dev = _pick_device(proj.device, source.mask, top)
+  samples = prm.upload(prm.ego_samples(pose, *cols, crop_height * crop_width), dev)
+  top = top.to(device=dev, dtype=torch.float32).contiguous()
+  mask = utils.to_4D_image(source.mask).to(device=dev, dtype=torch.bool).expand(b, C, Hs, Ws).contiguous()
+  out_top = torch.empty((b, C, crop_height, crop_width), dtype=torch.float32, device=dev)
+  out_mask = torch.empty((b, C, crop_height, crop_width), dtype=torch.bool, device=dev)
+  height = out_height = None
+  plane_stride = 0
+  if not source.is_height_map:
+    hm = utils.to_4D_image(source.height_map).to(device=dev, dtype=torch.float32).expand(b, C, Hs, Ws)
+    shared = hm.stride(1) == 0 and C > 1   # one plane for the C channels, as crop_topdown_map keeps it
+    height = (hm[:, :1] if shared else hm).contiguous()
+    plane_stride = 0 if shared else Hs * Ws
+    out_height = torch.empty((b, 1 if shared else C, crop_height, crop_width), dtype=torch.float32, device=dev)
+  fill = get(fill_value, proj.fill_value, NINF)
+  with torch.cuda.device(dev):
+    rc = nat.lib().dm_crop_egocentric_f32(top.data_ptr(), nat.ptr(height), plane_stride, mask.data_ptr(), b, C, Hs, Ws,
+                                          float(proj.map_res), int(bool(proj.flip_h)), samples.data_ptr(),
+                                          crop_height, crop_width, fill, out_top.data_ptr(), nat.ptr(out_height),
+                                          out_mask.data_ptr(), nat.stream_ptr(dev))
+  nat.check(rc, "dm_crop_egocentric_f32")
+  if source.is_height_map:
+    out_height = out_top
+  elif out_height.shape[1] != C:
+    out_height = out_height.expand(b, C, crop_height, crop_width)
+  new_proj = proj.clone(cam_pose=pose_host, to_global=False,
+                        width_offset=prm.host_f32(woff), height_offset=prm.host_f32(hoff), map_width=crop_width,
+                        map_height=crop_height)
+  return TopdownMap(topdown_map=out_top, mask=out_mask, height_map=out_height, is_height_map=source.is_height_map,
+                    map_projector=new_proj)
 
 
 def _fuse_source(m: TopdownMap, target: MapProjector, b: int, C: int, n_total: int, dev: torch.device,

@@ -312,6 +312,16 @@ int dm_pack_proj_samples(const DmPoseCfg* cfg, const float* pose, const float* s
 /* camera_affine_grid (maps.py:428-446): to_local, transition by trans_pose, to_camera. */
 int dm_pack_flow_samples(const DmPoseCfg* cfg, const float* pose, const float* sin_yaw, const float* cos_yaw,
                          int32_t b, DmFlowSample* out);
+/* TopdownMap.select_egocentric: DM_EGO_SAMPLE_WORDS floats per sample, out (b * DM_EGO_SAMPLE_WORDS):
+ *   words 0-15  DmStep local_to_global_space(pose) = rot(yaw) + (x, 0, z);
+ *   words 16-17 the source map's width / height offsets;
+ *   words 18-19 the window's width / height offsets.
+ * Only cfg->yaw_skew, yaw_skew_sq and fused are read; fused = 9 * crop_h * crop_w >= 400 (the window's cells are the
+ * points the composition rotates per sample).  All arrays (b,) except pose (b, 3). */
+#define DM_EGO_SAMPLE_WORDS 20
+int dm_pack_ego_samples(const DmPoseCfg* cfg, const float* pose, const float* sin_yaw, const float* cos_yaw,
+                        const float* src_width_offset, const float* src_height_offset, const float* width_offset,
+                        const float* height_offset, int32_t b, float* out);
 
 /* ---- MapBuilder.step with the host side in C (maps.py:2357-2508) ----------------------------------------------
  * The plot → merge loop of b environments for height maps (value_map None) and a world map in the global frame —
@@ -473,6 +483,25 @@ int dm_crop_nearest_f32(const float* image, const float* center, int32_t b, int3
                         float* out, void* stream);
 int dm_crop_nearest_u8(const uint8_t* image, const float* center, int32_t b, int32_t c, int32_t h,
                        int32_t w, int32_t crop_h, int32_t crop_w, uint8_t* out, void* stream);
+
+/* TopdownMap.select_egocentric: a crop_h x crop_w window of a global-frame map per sample, in the sample's camera
+ * frame (not in the reference; defined by its public functions).  Output cell (r, c) of sample s:
+ *   (lx, lz) = map_dequantize(c, r, window offsets, map_res, crop_h, flip_h)
+ *   (gx, gz) = local_to_global_space((lx, 0, lz), pose)      (the DmStep of the sample block)
+ *   (X, Z)   = map_quantize(gx, gz, source offsets, map_res, Hs, flip_h)
+ *   out = source[s, k, Z, X] inside the source, else fill_value / -inf (height) / 0 (mask).
+ * Source: topdown (b, C, Hs, Ws) f32, mask (b, C, Hs, Ws) u8, height f32 (NULL for height maps) with
+ * height_plane_stride Hs * Ws ((b, C, Hs, Ws)) or 0 ((b, 1, Hs, Ws) shared by the C channels).
+ * samples: device, b * DM_EGO_SAMPLE_WORDS floats from dm_pack_ego_samples.
+ * Output: out_topdown / out_mask (b, C, crop_h, crop_w), out_height (b, C or 1, crop_h, crop_w) as the source's
+ * heights, NULL exactly when height is NULL.  One launch, no host synchronisation.
+ * DM_EINVAL, before any CUDA call, for null tensors, b, C, Hs, Ws, crop_h or crop_w <= 0, map_res not > 0, a window or
+ * source plane of 2^31 cells or more, height and out_height not both given or both NULL, another plane stride, and
+ * unaligned samples. */
+int dm_crop_egocentric_f32(const float* topdown, const float* height, int64_t height_plane_stride, const uint8_t* mask,
+                           int32_t b, int32_t C, int32_t Hs, int32_t Ws, float map_res, int32_t flip_h,
+                           const float* samples, int32_t crop_h, int32_t crop_w, float fill_value, float* out_topdown,
+                           float* out_height, uint8_t* out_mask, void* stream);
 
 /* Library/ABI introspection. */
 int dm_abi_version(void);
