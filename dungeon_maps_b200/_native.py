@@ -171,6 +171,8 @@ _SIGNATURES = {
   "dm_crop_egocentric_f32": (ctypes.c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int32, c_int32, c_int32, c_int32,
                                             c_float, c_int32, c_void_p, c_int32, c_int32, c_float, c_void_p, c_void_p,
                                             c_void_p, c_void_p]),
+  "dm_geodesic_distance_i32": (ctypes.c_int, [c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32,
+                                              c_void_p, c_void_p]),
 }
 EXPORTS = tuple(_SIGNATURES)
 

@@ -43,8 +43,8 @@ __all__ = [
   'height_map_to_point_cloud', 'image_to_camera_space', 'camera_to_image_space', 'camera_to_local_space',
   'local_to_camera_space', 'local_to_global_space', 'global_to_local_space', 'map_quantize',
   'map_dequantize', 'project', 'compute_center_offsets', 'MapProjector', 'TopdownMap', 'crop_topdown_map',
-  'crop_egocentric_map', 'fuse_topdown_maps', 'merge_into_canvas', 'MapBuilder', 'release_workspaces', 'Reduction',
-  'CameraIntrinsics', 'NINF', 'Float3D',
+  'crop_egocentric_map', 'geodesic_distance', 'fuse_topdown_maps', 'merge_into_canvas', 'MapBuilder',
+  'release_workspaces', 'Reduction', 'CameraIntrinsics', 'NINF', 'Float3D',
 ]
 
 
@@ -845,6 +845,15 @@ class TopdownMap():
     return crop_egocentric_map(self, crop_width=crop_width, crop_height=crop_height, cam_pose=cam_pose,
                                width_offset=width_offset, height_offset=height_offset, fill_value=fill_value)
 
+  def geodesic_distance(self, traversable: torch.Tensor, sources=None) -> torch.Tensor:
+    """geodesic_distance over this map's grid (not in the reference).  `sources` defaults to the agent's cell as
+    get_camera() defines it, computed on the host from the projector's pose and offsets (no sync when they are host
+    values, as a MapBuilder world map's and a select_egocentric window's are): the distance from the agent to every
+    cell in one call."""
+    if sources is None:
+      sources = _camera_cells(self.proj, _geodesic_grid(traversable)[0])
+    return geodesic_distance(traversable, sources)
+
   def merge(self, *sources: List["TopdownMap"]) -> "TopdownMap":
     raise NotImplementedError
 
@@ -977,6 +986,100 @@ def crop_egocentric_map(source: TopdownMap, crop_width: int, crop_height: int, c
                         map_height=crop_height)
   return TopdownMap(topdown_map=out_top, mask=out_mask, height_map=out_height, is_height_map=source.is_height_map,
                     map_projector=new_proj)
+
+
+def _geodesic_grid(traversable) -> Tuple[int, int, int]:
+  """(b, H, W) of a traversable grid, checked in every respect but its device."""
+  if not torch.is_tensor(traversable) or traversable.dtype is not torch.bool:
+    raise ValueError("traversable must be a bool tensor, got "
+                     f"{traversable.dtype if torch.is_tensor(traversable) else type(traversable).__name__}")
+  if not (traversable.dim() == 3 or (traversable.dim() == 4 and traversable.shape[1] == 1)):
+    raise ValueError(f"traversable must be (b, H, W) or (b, 1, H, W), got {tuple(traversable.shape)}")
+  b, H, W = traversable.shape[0], traversable.shape[-2], traversable.shape[-1]
+  if b < 1 or H < 1 or W < 1:
+    raise ValueError(f"traversable must not be empty, got {tuple(traversable.shape)}")
+  if 7 * H * W > 2 ** 31 - 1:
+    raise ValueError(f"a {H} x {W} grid is too large: its largest distance 7 * H * W does not fit in int32")
+  return b, H, W
+
+
+def geodesic_distance(traversable: torch.Tensor, sources) -> torch.Tensor:
+  """Shortest-path distance, through traversable cells, from the sources of each environment to every cell of its map
+  (not in the reference): the distance field a planner steps down, on the device, for a whole batch at once.
+
+  traversable: CUDA bool (b, H, W) or (b, 1, H, W).  sources: a bool mask of the same shape on the same device, or
+  integer cells [x, z] = [column, row] (the convention of get_coords / get_camera) of shape (b, n, 2) or (b, 2), on
+  that device or on the host (host cells are uploaded through the parameter ring).  Cells outside the map are ignored.
+  Returns int32 (b, H, W).
+
+  Definition: the cells are the nodes of a graph.  An edge runs from u to an 8-neighbour v when T[v] holds and the
+  step is orthogonal, or diagonal with both cells that share an edge with u and v traversable (no corner cutting).  An
+  orthogonal step costs 5, a diagonal one 7.  dist[v] = 0 for a source; otherwise the least total cost of a path from
+  any source of the environment, or -1 when there is none.  The distance in metres is dist * map_res / 5.
+  - Integer costs make the result exact and independent of evaluation order, so it is compared bit for bit.
+  - A 5 / 7 chamfer stays within about 2 % of the Euclidean length of straight paths.
+  - Edges depend on the traversability of the destination only: a source cell that is an obstacle still reaches its
+    free neighbours, so an object's class plane can be the goal as it is.
+  Deriving `traversable` stays with the caller.  For a height world map `m` of a MapBuilder, with heights above the
+  floor: `free = m.mask & (m.height_map <= obstacle_height)`, and `free | ~m.mask` when unknown cells count as free.
+
+  One library call on the current stream (csrc/dm_geodesic.cu, one cooperative launch) and no host sync.  ValueError,
+  before any device work, for another shape, dtype or device, zero source cells, and grids whose largest distance
+  7 * H * W does not fit in int32."""
+  b, H, W = _geodesic_grid(traversable)
+  mask = cells = None
+  if torch.is_tensor(sources) and sources.dtype is torch.bool:
+    if sources.shape != traversable.shape:
+      raise ValueError(f"a source mask must have traversable's shape {tuple(traversable.shape)}, got "
+                       f"{tuple(sources.shape)}")
+    mask = sources
+  else:
+    cells = sources if torch.is_tensor(sources) else torch.from_numpy(np.asarray(sources))
+    if cells.dtype is torch.bool or cells.is_floating_point() or cells.is_complex():
+      raise ValueError(f"source cells must be integers (or a bool mask), got {cells.dtype}")
+    if cells.dim() == 2:
+      cells = cells.unsqueeze(1)
+    if cells.dim() != 3 or cells.shape[0] != b or cells.shape[2] != 2 or cells.shape[1] < 1:
+      raise ValueError(f"source cells must be ({b}, n, 2) with n >= 1 or ({b}, 2), got {tuple(sources.shape)}")
+  dev = traversable.device
+  if not traversable.is_cuda:
+    raise ValueError(f"traversable must be on a CUDA device, got {dev}")
+  if mask is not None and mask.device != dev:
+    raise ValueError(f"the source mask must be on {dev}, got {mask.device}")
+  if cells is not None and cells.is_cuda and cells.device != dev:
+    raise ValueError(f"the source cells must be on {dev} or the host, got {cells.device}")
+  n = 0
+  if cells is not None:
+    n = cells.shape[1]
+    cells = cells.to(torch.int64).contiguous()
+    if not cells.is_cuda:
+      cells = prm.upload(cells, dev) if cells.numel() * 8 <= prm._UPLOAD_MAX else \
+          cells.pin_memory().to(dev, non_blocking=True)
+  trav = traversable.reshape(b, H, W).contiguous()
+  mask = None if mask is None else mask.reshape(b, H, W).contiguous()
+  out = torch.empty((b, H, W), dtype=torch.int32, device=dev)
+  with torch.cuda.device(dev):
+    rc = nat.lib().dm_geodesic_distance_i32(trav.data_ptr(), nat.ptr(mask), nat.ptr(cells), n, b, H, W,
+                                            out.data_ptr(), nat.stream_ptr(dev))
+  nat.check(rc, "dm_geodesic_distance_i32")
+  return out
+
+
+def _camera_cells(proj: MapProjector, b: int) -> torch.Tensor:
+  """TopdownMap.get_camera() of b environments, (b, 2) int64 [x, z], from the projector's host values: the local
+  origin, moved by local_to_global_space for a global-frame map ((0, 0, 0) rotated is +-0, so it lands on the pose's
+  x, z exactly), then map_quantize in the same float32 operations."""
+  zero = torch.zeros((b,), dtype=torch.float32)
+  x = z = zero
+  if proj.to_global:
+    pose = prm.per_sample(prm.host_f32(get(proj.cam_pose, [0., 0., 0.]), (3,)), b, (3,), "cam_pose")
+    x, z = pose[:, 0] + zero, pose[:, 1] + zero
+  res = torch.tensor(float(proj.map_res), dtype=torch.float32)
+  xb = x / res + prm.per_sample(get(proj.width_offset, 0.), b, (), "width_offset")
+  zb = z / res + prm.per_sample(get(proj.height_offset, 0.), b, (), "height_offset")
+  if proj.flip_h:
+    zb = torch.tensor(float(proj.map_height - 1), dtype=torch.float32) - zb
+  return torch.stack((torch.floor(xb + 0.5), torch.floor(zb + 0.5)), dim=-1).to(torch.int64)
 
 
 def _fuse_source(m: TopdownMap, target: MapProjector, b: int, C: int, n_total: int, dev: torch.device,

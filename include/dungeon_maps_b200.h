@@ -503,6 +503,21 @@ int dm_crop_egocentric_f32(const float* topdown, const float* height, int64_t he
                            const float* samples, int32_t crop_h, int32_t crop_w, float fill_value, float* out_topdown,
                            float* out_height, uint8_t* out_mask, void* stream);
 
+/* geodesic_distance: per-environment shortest-path distances over an 8-connected grid (not in the reference).
+ * traversable (b, H, W) u8 0 / 1; the sources are EITHER source_mask (b, H, W) u8 (source_cells NULL, n_cells 0) OR
+ * source_cells (b, n_cells, 2) int64 [x, z] = [column, row] (source_mask NULL, n_cells >= 1; cells outside the map are
+ * ignored).  An edge runs from u to an 8-neighbour v when v is traversable and, for a diagonal step, both cells that
+ * share an edge with u and with v are traversable (no corner cutting); an orthogonal step costs 5, a diagonal one 7.
+ * Edges depend on the destination only: a source that is an obstacle still reaches its free neighbours.
+ * dist (b, H, W) int32: 0 on sources, else the least path cost from any source of the environment, -1 without a path.
+ * Exact (integer costs), whatever the evaluation order.  One cooperative launch, no host synchronisation; the kernel
+ * stops after H * W + 2 rounds, a count it provably never needs, and then raises the status word dm_device_status
+ * reports as DM_ETIMEOUT (dist is undefined).  DM_EINVAL, before any CUDA call, for null traversable or dist, b, H or
+ * W <= 0, both source forms or neither, n_cells out of the rule above, 7 * H * W > INT32_MAX (the largest distance),
+ * and 2^31 tiles of 32 x 32 or more. */
+int dm_geodesic_distance_i32(const uint8_t* traversable, const uint8_t* source_mask, const int64_t* source_cells,
+                             int32_t n_cells, int32_t b, int32_t H, int32_t W, int32_t* dist, void* stream);
+
 /* Library/ABI introspection. */
 int dm_abi_version(void);
 /* sizeof() of a struct of this header as the library was compiled, for bindings to check their mirror against:
