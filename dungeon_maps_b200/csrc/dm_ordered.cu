@@ -44,8 +44,9 @@ ordered_fold_kernel(const unsigned long long* __restrict__ keys, const unsigned 
       acc = reduction == 4 ? __fmul_rn(acc, v) : __fadd_rn(acc, v);
       ++hits;
     }
-    // scatter_mean: the sum (canvas included) divided by the number of hits (canvas excluded), at least 1
-    if (reduction == 3) acc = __fdiv_rn(acc, (float)hits);
+    // scatter_mean: the sum (canvas included) divided by the number of hits (canvas excluded), at least 1.
+    // torch_scatter counts with float32 ones, so its count stops at 2^24 (2^24 + 1 rounds back to 2^24).
+    if (reduction == 3) acc = __fdiv_rn(acc, hits < (1ll << 24) ? (float)hits : 16777216.0f);
     if (mask_or) {
       float dlt = fabsf(__fsub_rn(acc, canvas[k]));
       if (dlt != dlt) dlt = 0.0f;

@@ -297,7 +297,8 @@ int dmo_scatter(const float* values, const int64_t* coords, const uint8_t* valid
                 float* canvas, uint8_t* mask) {
   /* reduction (utils.py:44-76): 0 max, 1 min, 2 sum, 3 mean, 4 prod; hits are applied in index order like
    * torch_scatter's CPU loops.  mean (torch_scatter.scatter_mean with out=): the starting canvas takes part in
-   * the sum, not in the count; count is clamped to >= 1. */
+   * the sum, not in the count; count is clamped to >= 1.  torch_scatter counts with a scatter_add_ of float32 ones:
+   * that count stops at 2^24 (2^24 + 1 rounds back to 2^24), so the divisor is min(count, 2^24). */
   const int64_t M = (int64_t)Mh * Mw;
   float* before = (float*)malloc(sizeof(float) * (size_t)M);
   int32_t* count = (int32_t*)malloc(sizeof(int32_t) * (size_t)M);
@@ -318,7 +319,8 @@ int dmo_scatter(const float* values, const int64_t* coords, const uint8_t* valid
       else if (better(v, *t, reduction)) *t = v;
     }
     if (reduction == 3)
-      for (int64_t i = 0; i < M; ++i) cv[i] = cv[i] / (float)(count[i] < 1 ? 1 : count[i]);
+      for (int64_t i = 0; i < M; ++i)
+        cv[i] = cv[i] / (count[i] < 1 ? 1.0f : count[i] < (1 << 24) ? (float)count[i] : 16777216.0f);
     for (int64_t i = 0; i < M; ++i) {
       float d = fabsf(cv[i] - before[i]);
       if (isnan(d)) d = 0.0f;
