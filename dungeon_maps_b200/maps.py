@@ -43,8 +43,8 @@ __all__ = [
   'height_map_to_point_cloud', 'image_to_camera_space', 'camera_to_image_space', 'camera_to_local_space',
   'local_to_camera_space', 'local_to_global_space', 'global_to_local_space', 'map_quantize',
   'map_dequantize', 'project', 'compute_center_offsets', 'MapProjector', 'TopdownMap', 'crop_topdown_map',
-  'crop_egocentric_map', 'geodesic_distance', 'fuse_topdown_maps', 'merge_into_canvas', 'MapBuilder',
-  'release_workspaces', 'Reduction', 'CameraIntrinsics', 'NINF', 'Float3D',
+  'crop_egocentric_map', 'geodesic_distance', 'connected_components', 'fuse_topdown_maps', 'merge_into_canvas',
+  'MapBuilder', 'release_workspaces', 'Reduction', 'CameraIntrinsics', 'NINF', 'Float3D',
 ]
 
 
@@ -1063,6 +1063,64 @@ def geodesic_distance(traversable: torch.Tensor, sources) -> torch.Tensor:
                                             out.data_ptr(), nat.stream_ptr(dev))
   nat.check(rc, "dm_geodesic_distance_i32")
   return out
+
+
+def connected_components(mask: torch.Tensor, connectivity: int = 8, return_sizes: bool = False):
+  """Connected-component labels of every H x W plane of a mask (not in the reference): frontier clusters, object
+  instances of a class plane, obstacle blobs, on the device for a whole batch at once.
+
+  mask: CUDA bool (b, H, W) or (b, C, H, W); each plane is labelled on its own, so the C class planes of a semantic map
+  are C separate problems.  Non-contiguous views (world.mask[:, 0], an expanded plane) are made contiguous.
+  connectivity: 4 (orthogonal neighbours) or 8 (orthogonal and diagonal neighbours).  8-connectivity has no corner rule:
+  two cells that touch only at a corner are joined even when both cells beside that corner are background, so it is
+  not geodesic_distance's reachability, which forbids corner cutting.  For "reachable from the agent" use
+  `geodesic_distance(free, sources) >= 0`.
+
+  Returns (labels, counts), or (labels, counts, sizes) with return_sizes=True:
+  - labels: int32 with the shape of mask.  0 on background; the components of each plane are numbered 1..K in raster
+    order of their first cell (the smallest row * W + col).  That is exactly scipy.ndimage.label(plane, structure)
+    with structure = generate_binary_structure(2, 1) for connectivity=4 and np.ones((3, 3)) for connectivity=8.
+  - counts: int32 (b,) or (b, C) on the device: K per plane.
+  - sizes: int32 with the shape of mask: the cell count of each cell's component, 0 on background.  It filters by size
+    without a host sync, where a per-component table would need K on the host.
+
+  Frontier clusters of a MapBuilder world map `m` (seen free cells next to unseen ones), dropping clusters below k
+  cells:
+    seen = m.mask[:, 0]
+    free = seen & (m.height_map[:, 0] <= obstacle_height)
+    unseen_near = torch.nn.functional.max_pool2d((~seen).float()[:, None], 3, 1, 1)[:, 0] > 0
+    frontier = free & unseen_near
+    labels, counts, sizes = connected_components(frontier, return_sizes=True)
+    labels = labels * (sizes >= k)
+
+  One library call on the current stream (csrc/dm_components.cu: a block-based union-find in a few kernels and a cub
+  scan), no host sync, mask never written.  ValueError, before any device work, for a non-tensor or non-bool mask, a
+  rank other than 3 or 4, an empty dimension, a mask off CUDA, connectivity not 4 or 8, and more than 2^31 - 1 cells."""
+  if not torch.is_tensor(mask) or mask.dtype is not torch.bool:
+    raise ValueError("mask must be a bool tensor, got "
+                     f"{mask.dtype if torch.is_tensor(mask) else type(mask).__name__}")
+  if mask.dim() not in (3, 4):
+    raise ValueError(f"mask must be (b, H, W) or (b, C, H, W), got {tuple(mask.shape)}")
+  if mask.numel() == 0:
+    raise ValueError(f"mask must not be empty, got {tuple(mask.shape)}")
+  if mask.numel() > 2 ** 31 - 1:
+    raise ValueError(f"a mask of {mask.numel()} cells is too large: at most 2^31 - 1 cells are labelled in one call")
+  if isinstance(connectivity, bool) or connectivity not in (4, 8):
+    raise ValueError(f"connectivity must be 4 or 8, got {connectivity!r}")
+  if not mask.is_cuda:
+    raise ValueError(f"mask must be on a CUDA device, got {mask.device}")
+  H, W = mask.shape[-2], mask.shape[-1]
+  dev = mask.device
+  m = mask.contiguous()
+  labels = torch.empty(mask.shape, dtype=torch.int32, device=dev)
+  counts = torch.empty(mask.shape[:-2], dtype=torch.int32, device=dev)
+  sizes = torch.empty(mask.shape, dtype=torch.int32, device=dev) if return_sizes else None
+  with torch.cuda.device(dev):
+    rc = nat.lib().dm_connected_components_i32(m.data_ptr(), m.numel() // (H * W), H, W, int(connectivity),
+                                               labels.data_ptr(), counts.data_ptr(), nat.ptr(sizes),
+                                               nat.stream_ptr(dev))
+  nat.check(rc, "dm_connected_components_i32")
+  return (labels, counts, sizes) if return_sizes else (labels, counts)
 
 
 def _camera_cells(proj: MapProjector, b: int) -> torch.Tensor:

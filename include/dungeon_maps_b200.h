@@ -518,6 +518,19 @@ int dm_crop_egocentric_f32(const float* topdown, const float* height, int64_t he
 int dm_geodesic_distance_i32(const uint8_t* traversable, const uint8_t* source_mask, const int64_t* source_cells,
                              int32_t n_cells, int32_t b, int32_t H, int32_t W, int32_t* dist, void* stream);
 
+/* connected_components: per-plane connected-component labels of masks (not in the reference).
+ * mask (n_planes, H, W) u8, nonzero = foreground; each H x W plane is labelled on its own.  connectivity 4 (orthogonal
+ * neighbours) or 8 (orthogonal and diagonal neighbours, no corner rule).
+ * labels (n_planes, H, W) int32: 0 on background; the components of a plane are numbered 1..K in raster order of their
+ * first cell (the smallest row * W + col), exactly as scipy.ndimage.label numbers them.  counts (n_planes) int32: K.
+ * sizes (n_planes, H, W) int32, or NULL when not wanted: the cell count of each cell's component, 0 on background.
+ * Deterministic whatever order the atomics run in.  Several kernels and a cub scan on `stream`, stream-ordered scratch
+ * (cudaMallocAsync, 4 B a cell), no host synchronisation, no device-to-host copy; mask is never written.  DM_EINVAL,
+ * before any CUDA call, for null mask, labels or counts, n_planes, H or W <= 0, connectivity not 4 or 8, and
+ * n_planes * H * W > INT32_MAX. */
+int dm_connected_components_i32(const uint8_t* mask, int32_t n_planes, int32_t H, int32_t W, int32_t connectivity,
+                                int32_t* labels, int32_t* counts, int32_t* sizes, void* stream);
+
 /* Library/ABI introspection. */
 int dm_abi_version(void);
 /* sizeof() of a struct of this header as the library was compiled, for bindings to check their mirror against:
