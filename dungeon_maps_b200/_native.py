@@ -175,6 +175,7 @@ _SIGNATURES = {
                                               c_void_p, c_void_p]),
   "dm_connected_components_i32": (ctypes.c_int, [c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p,
                                                  c_void_p, c_void_p]),
+  "dm_distance_transform_f32": (ctypes.c_int, [c_void_p, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p]),
 }
 EXPORTS = tuple(_SIGNATURES)
 

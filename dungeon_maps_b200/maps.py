@@ -43,8 +43,8 @@ __all__ = [
   'height_map_to_point_cloud', 'image_to_camera_space', 'camera_to_image_space', 'camera_to_local_space',
   'local_to_camera_space', 'local_to_global_space', 'global_to_local_space', 'map_quantize',
   'map_dequantize', 'project', 'compute_center_offsets', 'MapProjector', 'TopdownMap', 'crop_topdown_map',
-  'crop_egocentric_map', 'geodesic_distance', 'connected_components', 'fuse_topdown_maps', 'merge_into_canvas',
-  'MapBuilder', 'release_workspaces', 'Reduction', 'CameraIntrinsics', 'NINF', 'Float3D',
+  'crop_egocentric_map', 'geodesic_distance', 'connected_components', 'distance_transform', 'fuse_topdown_maps',
+  'merge_into_canvas', 'MapBuilder', 'release_workspaces', 'Reduction', 'CameraIntrinsics', 'NINF', 'Float3D',
 ]
 
 
@@ -1121,6 +1121,68 @@ def connected_components(mask: torch.Tensor, connectivity: int = 8, return_sizes
                                                nat.stream_ptr(dev))
   nat.check(rc, "dm_connected_components_i32")
   return (labels, counts, sizes) if return_sizes else (labels, counts)
+
+
+def distance_transform(mask: torch.Tensor, return_indices: bool = False):
+  """Exact Euclidean distance transform of every H x W plane of a mask (not in the reference): the clearance of each
+  cell from the nearest obstacle, and the nearest free cell to a goal, on the device for a whole batch at once.
+
+  mask: CUDA bool (b, H, W) or (b, C, H, W); each plane is transformed on its own.  Non-contiguous views
+  (world.mask[:, 0], an expanded plane) are made contiguous.
+
+  Returns dist, or (dist, nearest) with return_indices=True:
+  - dist: float32 with the shape of mask.  0 on False cells; on True cells the Euclidean distance in cells (centre to
+    centre) to the nearest False cell of the same plane; in metres, dist * map_res.  That is exactly
+    scipy.ndimage.distance_transform_edt(plane).astype(np.float32).
+  - nearest: int32 of shape (*mask.shape, 2) holding [x, z] = [column, row], the cell convention of get_coords /
+    get_camera / geodesic_distance's source cells.  It is not scipy's return_indices layout, which is (2, H, W) in
+    [row, column] order.  On a True cell: a False cell at exactly the returned distance; on a False cell: the cell
+    itself.  When several False cells are equally near, it is one of them, fixed: the same input gives the same bits
+    on every call, and a plane's result does not depend on the other planes.  It need not be scipy's choice.
+  A plane with no False cell has no nearest one: dist is +inf and nearest is -1 on every cell of it (scipy instead
+  measures to a phantom cell outside the plane).
+
+  Obstacle inflation for a MapBuilder world map `m` and an agent of radius r metres: the cells where the agent's centre
+  keeps more than r from every obstacle, and the geodesic field over them:
+    seen = m.mask[:, 0]
+    obstacle = seen & (m.height_map[:, 0] > obstacle_height)
+    free = seen & ~obstacle
+    traversable = free & (distance_transform(~obstacle) * map_res > r)
+    dist_to_agent = m.geodesic_distance(traversable)
+
+  Goal snapping, the free cell nearest to goal cell (x, z) of environment i (an object goal on an obstacle, a frontier
+  cell):
+    d, nearest = distance_transform(~free, return_indices=True)
+    x_free, z_free = nearest[i, z, x]
+
+  One library call on the current stream (csrc/dm_distance.cu: the separable exact transform in two kernels), no host
+  sync, mask never written.  ValueError, before any device work, for a non-tensor or non-bool mask, a rank other than 3
+  or 4, an empty dimension, a mask off CUDA, H or W above 32768 (the squared distance must fit in int32), and more than
+  2^31 - 1 cells."""
+  if not torch.is_tensor(mask) or mask.dtype is not torch.bool:
+    raise ValueError("mask must be a bool tensor, got "
+                     f"{mask.dtype if torch.is_tensor(mask) else type(mask).__name__}")
+  if mask.dim() not in (3, 4):
+    raise ValueError(f"mask must be (b, H, W) or (b, C, H, W), got {tuple(mask.shape)}")
+  if mask.numel() == 0:
+    raise ValueError(f"mask must not be empty, got {tuple(mask.shape)}")
+  H, W = mask.shape[-2], mask.shape[-1]
+  if H > 32768 or W > 32768:
+    raise ValueError(f"a {H} x {W} plane is too large: H and W must be at most 32768 so that the squared distance fits "
+                     "in int32")
+  if mask.numel() > 2 ** 31 - 1:
+    raise ValueError(f"a mask of {mask.numel()} cells is too large: at most 2^31 - 1 cells are transformed in one call")
+  if not mask.is_cuda:
+    raise ValueError(f"mask must be on a CUDA device, got {mask.device}")
+  dev = mask.device
+  m = mask.contiguous()
+  dist = torch.empty(mask.shape, dtype=torch.float32, device=dev)
+  nearest = torch.empty((*mask.shape, 2), dtype=torch.int32, device=dev) if return_indices else None
+  with torch.cuda.device(dev):
+    rc = nat.lib().dm_distance_transform_f32(m.data_ptr(), m.numel() // (H * W), H, W, dist.data_ptr(),
+                                             nat.ptr(nearest), nat.stream_ptr(dev))
+  nat.check(rc, "dm_distance_transform_f32")
+  return (dist, nearest) if return_indices else dist
 
 
 def _camera_cells(proj: MapProjector, b: int) -> torch.Tensor:

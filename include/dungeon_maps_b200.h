@@ -531,6 +531,21 @@ int dm_geodesic_distance_i32(const uint8_t* traversable, const uint8_t* source_m
 int dm_connected_components_i32(const uint8_t* mask, int32_t n_planes, int32_t H, int32_t W, int32_t connectivity,
                                 int32_t* labels, int32_t* counts, int32_t* sizes, void* stream);
 
+/* distance_transform: per-plane exact Euclidean distance transform of masks (not in the reference).
+ * mask (n_planes, H, W) u8; each H x W plane is transformed on its own.
+ * dist (n_planes, H, W) float32: 0 on zero cells; on nonzero cells the Euclidean distance in cells (centre to centre)
+ * to the nearest zero cell of the plane, rounded as (float)sqrt((double)d2) from the exact integer squared distance d2,
+ * which is exactly scipy.ndimage.distance_transform_edt(plane).astype(float32).
+ * nearest (n_planes, H, W, 2) int32, or NULL when not wanted: [x, z] = [column, row] of a zero cell at exactly that
+ * distance (the cell itself on zero cells); on ties one fixed such cell, the same on every call and whatever the other
+ * planes hold.
+ * A plane without a zero cell gets dist = +inf and nearest = -1 on every cell.  Two kernels on `stream`, stream-ordered
+ * scratch (cudaMallocAsync, 2 B a cell), no atomics, no host synchronisation, no device-to-host copy; mask is never
+ * written.  DM_EINVAL, before any CUDA call, for null mask or dist, n_planes, H or W <= 0, H or W > 32768 (d2 must fit
+ * int32) and n_planes * H * W > INT32_MAX. */
+int dm_distance_transform_f32(const uint8_t* mask, int32_t n_planes, int32_t H, int32_t W, float* dist,
+                              int32_t* nearest, void* stream);
+
 /* Library/ABI introspection. */
 int dm_abi_version(void);
 /* sizeof() of a struct of this header as the library was compiled, for bindings to check their mirror against:
