@@ -43,7 +43,7 @@ __all__ = [
   'height_map_to_point_cloud', 'image_to_camera_space', 'camera_to_image_space', 'camera_to_local_space',
   'local_to_camera_space', 'local_to_global_space', 'global_to_local_space', 'map_quantize',
   'map_dequantize', 'project', 'compute_center_offsets', 'MapProjector', 'TopdownMap', 'crop_topdown_map',
-  'crop_egocentric_map', 'geodesic_distance', 'connected_components', 'distance_transform', 'fuse_topdown_maps',
+  'crop_egocentric_map', 'score_poses', 'geodesic_distance', 'connected_components', 'distance_transform', 'fuse_topdown_maps',
   'merge_into_canvas', 'MapBuilder', 'release_workspaces', 'Reduction', 'CameraIntrinsics', 'NINF', 'Float3D',
 ]
 
@@ -986,6 +986,110 @@ def crop_egocentric_map(source: TopdownMap, crop_width: int, crop_height: int, c
                         map_height=crop_height)
   return TopdownMap(topdown_map=out_top, mask=out_mask, height_map=out_height, is_height_map=source.is_height_map,
                     map_projector=new_proj)
+
+
+def score_poses(source: TopdownMap, planes: torch.Tensor, window: torch.Tensor, cam_poses,
+                width_offset=None, height_offset=None) -> torch.Tensor:
+  """How well a local window matches the planes of a global-frame map at each of n candidate poses, for every
+  environment at once (not in the reference): correlative scan matching, to correct noisy odometry before a merge.
+
+  source: a global-frame TopdownMap; only its projector (map_res, flip_h, per-environment width_offset /
+  height_offset) and its b x Hs x Ws size are read.  planes: CUDA bool (b, Hs, Ws) or (b, C, Hs, Ws) on the source's
+  grid, what to match against (world obstacle cells, world free cells, ...).  window: CUDA bool (b, h, w), shared by
+  every plane, or (b, C, h, w), one per plane (4-D planes only): the local observation, e.g. the local map's obstacle
+  cells.  cam_poses: float (n, 3), shared by the environments, or (b, n, 3), rows [x, z, yaw], n >= 1.
+  width_offset / height_offset (1 or b values): the window's origin, by default w / 2 and h / 2 as in
+  crop_egocentric_map; a config-4 local map (to_global=False, width_offset=MW / 2, height_offset=0) passes its own.
+  Returns int32 (b, n) for 3-D planes and (b, C, n) for 4-D planes.
+
+  Definition, exact:
+      score[i, c, k] = sum over (r, col) of window[i, c or 0, r, col]  AND
+          crop_egocentric_map(TopdownMap(mask=planes) with source.proj, w, h, cam_pose=cam_poses[i, k],
+                              width_offset, height_offset).mask[i, c, r, col]
+  i.e. window cell (r, col) goes through map_dequantize with the window offsets, local_to_global_space with candidate
+  k (h * w points, so the fused or naive rotation is chosen as for the crop), map_quantize with the source offsets, and
+  a read of the plane there; cells that land outside the source count as False.  Integer counts: the result does not
+  depend on evaluation order.  The best pose is the caller's choice, scores.argmax(-1) (the first maximum).
+
+  Noisy-odometry recipe for a height-map MapBuilder `builder` with config-4 local maps (to_global=False,
+  width_offset=MW / 2, height_offset=0), odometry poses `odom` (b, 3) on the host:
+    world = builder.world_map
+    seen = world.mask[:, 0]
+    obstacle = seen & (world.height_map[:, 0] > obstacle_height)
+    planes = torch.stack((obstacle, seen & ~obstacle), dim=1)                # world obstacle and free cells
+    local = builder.plot(depth, cam_pose=odom, **config4)                    # orth_project in the camera frame
+    window = local.mask[:, 0] & (local.height_map[:, 0] > obstacle_height)   # local obstacle cells
+    cands = (odom[:, None, :] + lattice[None]).to(torch.float32)             # (b, n, 3): (dx, dz, dyaw) offsets
+    s = score_poses(world, planes, window, cands, width_offset=MW / 2, height_offset=0.)
+    best = (s[:, 0] - s[:, 1]).argmax(-1)        # obstacle hits minus local obstacles on known free cells
+    pose = cands[torch.arange(b), best.cpu()]    # reading the winner back: the caller's one host sync
+    builder.step(depth, cam_pose=pose, **config4)
+  The read-back is the only sync the recipe adds; the growing-map MapBuilder.step already syncs once per step for
+  its bounding box.
+
+  cam_poses, like crop_egocentric_map's pose and the offsets, are host values packed into one block per (environment,
+  candidate); a CUDA cam_poses tensor is copied to the host, which synchronises with its stream.  Blocks up to 64 KiB
+  go through the parameter ring, larger ones through a pinned non-blocking copy: no host sync otherwise.  One library
+  call on the current stream (csrc/dm_match.cu: a compaction and a scoring kernel); planes and window are never
+  written.  ValueError, before any device work, for an empty or local-frame source; planes or window not bool or of
+  the wrong rank; planes whose batch or Hs x Ws differs from the source; a window not (b, h, w) or (b, C, h, w), or
+  with an empty dimension; cam_poses not (n, 3) or (b, n, 3) or with n < 1; an offset count other than 1 or b; b * n,
+  h * w or Hs * Ws of 2^31 or more; and planes or window off CUDA or on different devices."""
+  if source is None or source.is_empty:
+    raise ValueError("score_poses needs a map: the source is empty")
+  proj = source.proj
+  if proj is None or not proj.to_global:
+    raise ValueError("score_poses reads a global-frame map (proj.to_global); the source is in a local frame")
+  b, _, Hs, Ws = utils.to_4D_image(source.topdown_map).shape
+  for name, t in (("planes", planes), ("window", window)):
+    if not torch.is_tensor(t) or t.dtype is not torch.bool:
+      raise ValueError(f"{name} must be a bool tensor, got {t.dtype if torch.is_tensor(t) else type(t).__name__}")
+  if planes.dim() not in (3, 4):
+    raise ValueError(f"planes must be (b, Hs, Ws) or (b, C, Hs, Ws), got {tuple(planes.shape)}")
+  C = planes.shape[1] if planes.dim() == 4 else 1
+  if planes.shape[0] != b or tuple(planes.shape[-2:]) != (Hs, Ws) or C < 1:
+    raise ValueError(f"planes must be ({b}, [C,] {Hs}, {Ws}) like the source map, got {tuple(planes.shape)}")
+  per_plane = window.dim() == 4
+  if not (window.dim() == 3 or (per_plane and planes.dim() == 4 and window.shape[1] == C)) or window.shape[0] != b:
+    raise ValueError(f"window must be ({b}, h, w)" + (f" or ({b}, {C}, h, w)" if planes.dim() == 4 else "") +
+                     f", got {tuple(window.shape)}")
+  h, w = window.shape[-2], window.shape[-1]
+  if h < 1 or w < 1:
+    raise ValueError(f"window must not be empty, got {tuple(window.shape)}")
+  pose_shape = tuple(cam_poses.shape) if torch.is_tensor(cam_poses) else np.shape(cam_poses)
+  if not (len(pose_shape) == 2 or (len(pose_shape) == 3 and pose_shape[0] == b)) or pose_shape[-1] != 3 or \
+     pose_shape[-2] < 1:
+    raise ValueError(f"cam_poses must be (n, 3) or ({b}, n, 3) with n >= 1, got {pose_shape}")
+  n = pose_shape[-2]
+  for what, cells in (("b * n", b * n), ("h * w", h * w), ("Hs * Ws", Hs * Ws)):
+    if cells >= 2 ** 31:
+      raise ValueError(f"{what} = {cells} is too large: it must stay below 2^31")
+  cols = [prm.per_sample(get(proj.width_offset, 0.), b, (), "source width_offset"),
+          prm.per_sample(get(proj.height_offset, 0.), b, (), "source height_offset"),
+          prm.per_sample(get(width_offset, w / 2.), b, (), "width_offset"),
+          prm.per_sample(get(height_offset, h / 2.), b, (), "height_offset")]
+  dev = planes.device
+  if not planes.is_cuda:
+    raise ValueError(f"planes must be on a CUDA device, got {dev}")
+  if window.device != dev:
+    raise ValueError(f"window must be on {dev}, got {window.device}")
+  if torch.is_tensor(cam_poses) and cam_poses.is_cuda and cam_poses.device != dev:
+    raise ValueError(f"cam_poses must be on {dev} or the host, got {cam_poses.device}")
+  poses = prm.host_f32(cam_poses, (3,))
+  poses = poses.reshape(-1, n, 3).expand(b, n, 3).reshape(b * n, 3)
+  cols = [c[:, None].expand(b, n).reshape(b * n) for c in cols]
+  samples = prm.ego_samples(poses, *cols, h * w)
+  pl = planes.reshape(b, C, Hs, Ws).contiguous()
+  win = window.contiguous()
+  out = torch.empty((b, C, n), dtype=torch.int32, device=dev)
+  with torch.cuda.device(dev):
+    block = prm.upload(samples, dev) if samples.numel() * 4 <= prm._UPLOAD_MAX else \
+        samples.pin_memory().to(dev, non_blocking=True)
+    rc = nat.lib().dm_score_poses_i32(pl.data_ptr(), b, C, Hs, Ws, float(proj.map_res), int(bool(proj.flip_h)),
+                                      win.data_ptr(), C if per_plane else 1, h, w, block.data_ptr(), n,
+                                      out.data_ptr(), nat.stream_ptr(dev))
+  nat.check(rc, "dm_score_poses_i32")
+  return out if planes.dim() == 4 else out.view(b, n)
 
 
 def _geodesic_grid(traversable) -> Tuple[int, int, int]:

@@ -546,6 +546,24 @@ int dm_connected_components_i32(const uint8_t* mask, int32_t n_planes, int32_t H
 int dm_distance_transform_f32(const uint8_t* mask, int32_t n_planes, int32_t H, int32_t W, float* dist,
                               int32_t* nearest, void* stream);
 
+/* score_poses: per-environment match counts of a window against the planes of a global-frame map at candidate poses
+ * (not in the reference; defined by its public functions).  For window cell (r, c) and candidate k of environment i:
+ *   (lx, lz) = map_dequantize(c, r, window offsets, map_res, h, flip_h)
+ *   (gx, gz) = local_to_global_space((lx, 0, lz), pose k)       (the DmStep of block i * n + k)
+ *   (X, Z)   = map_quantize(gx, gz, source offsets, map_res, Hs, flip_h)
+ * which is cell (r, c) of dm_crop_egocentric_f32 with that block, and
+ *   scores[i, p, k] = #{(r, c) : window[i, p or 0, r, c] != 0, (X, Z) inside the source, planes[i, p, Z, X] != 0}.
+ * planes (b, C, Hs, Ws) u8; window (b, window_planes, h, w) u8 with window_planes 1 (shared by the C planes) or C (one
+ * per plane).  samples: device, b * n * DM_EGO_SAMPLE_WORDS floats from dm_pack_ego_samples, environment-major (block
+ * i * n + k), each block with its own offsets.  scores (b, C, n) int32, every entry written.  Exact integer counts,
+ * independent of evaluation order.  Two kernels on `stream` (counted as one launch), stream-ordered scratch
+ * (cudaMallocAsync, 4 B per window cell), no atomics, no host synchronisation; planes, window and samples are never
+ * written.  DM_EINVAL, before any CUDA call, for null pointers, b, C, Hs, Ws, h, w or n <= 0, window_planes not 1 or
+ * C, map_res not > 0, b * n, h * w or Hs * Ws of 2^31 or more, and unaligned samples. */
+int dm_score_poses_i32(const uint8_t* planes, int32_t b, int32_t C, int32_t Hs, int32_t Ws, float map_res,
+                       int32_t flip_h, const uint8_t* window, int32_t window_planes, int32_t h, int32_t w,
+                       const float* samples, int32_t n, int32_t* scores, void* stream);
+
 /* Library/ABI introspection. */
 int dm_abi_version(void);
 /* sizeof() of a struct of this header as the library was compiled, for bindings to check their mirror against:
