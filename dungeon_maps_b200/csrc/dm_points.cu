@@ -349,6 +349,7 @@ extern "C" int dm_depth_to_points_f32(const float* depth, const uint8_t* valid_i
                                       uint8_t* valid_out, void* stream) {
   DM_TRACE();
   if (frames < 0 || H <= 0 || W <= 0) return DM_EINVAL;
+  if ((long long)H * W >= (1ll << 31)) return DM_EINVAL;  // the kernel steps through a frame with int
   const long long total = (long long)frames * H * W;
   if (total == 0) return DM_OK;
   if (!depth || !points || !valid_out) return DM_EINVAL;
@@ -434,6 +435,7 @@ extern "C" int dm_crop_nearest_f32(const float* image, const float* center, int3
                                    float* out, void* stream) {
   DM_TRACE();
   if (b < 0 || c < 0 || h <= 0 || w <= 0 || crop_h < 0 || crop_w < 0) return DM_EINVAL;
+  if ((long long)crop_h * crop_w >= (1ll << 31) || (long long)h * w >= (1ll << 31)) return DM_EINVAL;
   const long long total = (long long)b * c * crop_h * crop_w;
   if (total == 0) return DM_OK;
   if (!image || !center || !out) return DM_EINVAL;
@@ -447,6 +449,7 @@ extern "C" int dm_crop_nearest_u8(const uint8_t* image, const float* center, int
                                   int32_t w, int32_t crop_h, int32_t crop_w, uint8_t* out, void* stream) {
   DM_TRACE();
   if (b < 0 || c < 0 || h <= 0 || w <= 0 || crop_h < 0 || crop_w < 0) return DM_EINVAL;
+  if ((long long)crop_h * crop_w >= (1ll << 31) || (long long)h * w >= (1ll << 31)) return DM_EINVAL;
   const long long total = (long long)b * c * crop_h * crop_w;
   if (total == 0) return DM_OK;
   if (!image || !center || !out) return DM_EINVAL;

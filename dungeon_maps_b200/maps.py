@@ -534,15 +534,25 @@ def global_to_local_space(points: torch.Tensor, cam_pose: torch.Tensor,
   return _run_steps(points, _pick_device(device, points), [st])
 
 
-def _coords_pair(x_coords, z_coords, dev):
+def _coords_pair(x_coords, z_coords, width_offset, height_offset, dev):
+  """(b, n) float32 coordinates on `dev`, the output shape, and the (b,) offsets.  Like the transforms, one coordinate
+  set is broadcast over b offsets (TopdownMap.get_camera / get_origin of a batched map)."""
   x = utils.to_tensor(x_coords).to(device=dev, dtype=torch.float32)
   z = utils.to_tensor(z_coords).to(device=dev, dtype=torch.float32)
   x, z = torch.broadcast_tensors(x, z)
   shape = x.shape
   if x.dim() < 2:
     x, z = x.reshape(1, -1), z.reshape(1, -1)
+    shape = x.shape
   b = x.shape[0]
-  return x.reshape(b, -1).contiguous(), z.reshape(b, -1).contiguous(), shape, b
+  x, z = x.reshape(b, -1), z.reshape(b, -1)
+  if b == 1:
+    b = max(prm.host_f32(width_offset).shape[0], prm.host_f32(height_offset).shape[0])
+    x, z = x.expand(b, -1), z.expand(b, -1)
+    shape = (b,) + tuple(shape[1:])
+  woff = prm.upload(prm.per_sample(width_offset, b).contiguous(), dev)
+  hoff = prm.upload(prm.per_sample(height_offset, b).contiguous(), dev)
+  return x.contiguous(), z.contiguous(), shape, woff, hoff
 
 
 def map_quantize(x_coords: torch.Tensor, z_coords: torch.Tensor, width_offset: torch.Tensor,
@@ -551,20 +561,17 @@ def map_quantize(x_coords: torch.Tensor, z_coords: torch.Tensor, width_offset: t
                  _validate_args: bool = True) -> Tuple[torch.Tensor, torch.Tensor]:
   """World x, z → integer map bins, rounding half up (maps.py:944-1019)."""
   dev = _pick_device(device, x_coords, z_coords)
-  x, z, shape, b = _coords_pair(x_coords, z_coords, dev)
   if flip_h:
     assert map_height is not None
-  woff = prm.upload(prm.per_sample(width_offset, b).contiguous(), dev)
-  hoff = prm.upload(prm.per_sample(height_offset, b).contiguous(), dev)
+  x, z, shape, woff, hoff = _coords_pair(x_coords, z_coords, width_offset, height_offset, dev)
   xb = torch.empty(x.shape, dtype=torch.int64, device=dev)
   zb = torch.empty(x.shape, dtype=torch.int64, device=dev)
   with torch.cuda.device(dev):
-    rc = nat.lib().dm_map_quantize_f32(x.data_ptr(), z.data_ptr(), woff.data_ptr(), hoff.data_ptr(), b,
+    rc = nat.lib().dm_map_quantize_f32(x.data_ptr(), z.data_ptr(), woff.data_ptr(), hoff.data_ptr(), x.shape[0],
                                        x.shape[1], map_res, int(map_height or 0), int(bool(flip_h)),
                                        xb.data_ptr(), zb.data_ptr(), nat.stream_ptr(dev))
   nat.check(rc, "dm_map_quantize_f32")
-  out_shape = shape if len(shape) >= 2 else (1, xb.numel())
-  return xb.reshape(out_shape), zb.reshape(out_shape)
+  return xb.reshape(shape), zb.reshape(shape)
 
 
 def map_dequantize(x_coords: torch.Tensor, z_coords: torch.Tensor, width_offset: torch.Tensor,
@@ -573,20 +580,17 @@ def map_dequantize(x_coords: torch.Tensor, z_coords: torch.Tensor, width_offset:
                    _validate_args: bool = True) -> Tuple[torch.Tensor, torch.Tensor]:
   """Inverse of map_quantize (maps.py:1021-1087)."""
   dev = _pick_device(device, x_coords, z_coords)
-  xb, zb, shape, b = _coords_pair(x_coords, z_coords, dev)
   if flip_h:
     assert map_height is not None
-  woff = prm.upload(prm.per_sample(width_offset, b).contiguous(), dev)
-  hoff = prm.upload(prm.per_sample(height_offset, b).contiguous(), dev)
+  xb, zb, shape, woff, hoff = _coords_pair(x_coords, z_coords, width_offset, height_offset, dev)
   x = torch.empty_like(xb)
   z = torch.empty_like(zb)
   with torch.cuda.device(dev):
-    rc = nat.lib().dm_map_dequantize_f32(xb.data_ptr(), zb.data_ptr(), woff.data_ptr(), hoff.data_ptr(), b,
+    rc = nat.lib().dm_map_dequantize_f32(xb.data_ptr(), zb.data_ptr(), woff.data_ptr(), hoff.data_ptr(), xb.shape[0],
                                          xb.shape[1], map_res, int(map_height or 0), int(bool(flip_h)),
                                          x.data_ptr(), z.data_ptr(), nat.stream_ptr(dev))
   nat.check(rc, "dm_map_dequantize_f32")
-  out_shape = shape if len(shape) >= 2 else (1, x.numel())
-  return x.reshape(out_shape), z.reshape(out_shape)
+  return x.reshape(shape), z.reshape(shape)
 
 
 def project(coords: torch.Tensor, values: torch.Tensor, masks: torch.Tensor, canvas: torch.Tensor,

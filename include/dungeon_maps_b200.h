@@ -445,7 +445,7 @@ int dm_image_camera_f32(const float* points, int64_t n, float fx, float fy, floa
                         int32_t flip_h, int32_t height, int32_t to_image, float* out, void* stream);
 
 /* depth_map_to_point_cloud maps.py:462-545: depth (b*c, H, W) → points (b*c, H, W, 3) and
- * valid (b*c, H, W) u8. valid_in may be NULL. */
+ * valid (b*c, H, W) u8. valid_in may be NULL.  DM_EINVAL for a frame of 2^31 pixels or more. */
 int dm_depth_to_points_f32(const float* depth, const uint8_t* valid_in, int64_t frames, int32_t H,
                            int32_t W, float fx, float fy, float cx, float cy, int32_t flip_h,
                            int32_t has_tmin, float tmin, int32_t has_tmax, float tmax,
@@ -477,7 +477,7 @@ int dm_scatter_f32(const float* values, const int64_t* coords, const uint8_t* va
  * image_sample utils.py:613-652 (pad 1, grid_sample nearest, align_corners).
  * image (b, c, h, w) f32 → out (b, c, crop_h, crop_w); center (b, 2) f32 device.
  * border = 1: padding_mode 'border' with pad value `fill` (fill_value given);
- * border = 0: zeros. */
+ * border = 0: zeros.  DM_EINVAL for a crop or an image plane of 2^31 cells or more. */
 int dm_crop_nearest_f32(const float* image, const float* center, int32_t b, int32_t c, int32_t h,
                         int32_t w, int32_t crop_h, int32_t crop_w, int32_t border, float fill,
                         float* out, void* stream);
