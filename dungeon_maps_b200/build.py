@@ -15,7 +15,8 @@ CSRC = os.path.join(HERE, "csrc")
 # $DM_B200_LIB points the binding at another build of the same ABI (kernel experiments, scripts/exp_build.sh)
 LIB = os.environ.get("DM_B200_LIB") or os.path.join(HERE, "libdungeon_maps_b200.so")
 SOURCES = ["dm_api.cu", "dm_project.cu", "dm_labels.cu", "dm_flow.cu", "dm_fuse.cu", "dm_points.cu", "dm_builder.cu", "dm_params.cu", "dm_ordered.cu",
-           "dm_geodesic.cu", "dm_components.cu", "dm_distance.cu", "dm_match.cu"]
+           "dm_geodesic.cu", "dm_components.cu", "dm_distance.cu", "dm_match.cu",
+           "dm_visibility.cu"]
 NVCC_FLAGS = [
   "-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "--fmad=false",
   "-Xcompiler", "-fPIC", "-Xcompiler", "-ffp-contract=off", "-shared", "-cudart", "static",

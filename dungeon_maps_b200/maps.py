@@ -43,7 +43,8 @@ __all__ = [
   'height_map_to_point_cloud', 'image_to_camera_space', 'camera_to_image_space', 'camera_to_local_space',
   'local_to_camera_space', 'local_to_global_space', 'global_to_local_space', 'map_quantize',
   'map_dequantize', 'project', 'compute_center_offsets', 'MapProjector', 'TopdownMap', 'crop_topdown_map',
-  'crop_egocentric_map', 'score_poses', 'geodesic_distance', 'connected_components', 'distance_transform', 'fuse_topdown_maps',
+  'crop_egocentric_map', 'score_poses', 'geodesic_distance', 'connected_components', 'distance_transform',
+  'visible_cells', 'count_visible', 'fuse_topdown_maps',
   'merge_into_canvas', 'MapBuilder', 'release_workspaces', 'Reduction', 'CameraIntrinsics', 'NINF', 'Float3D',
 ]
 
@@ -858,6 +859,21 @@ class TopdownMap():
       sources = _camera_cells(self.proj, _geodesic_grid(traversable)[0])
     return geodesic_distance(traversable, sources)
 
+  def visible_cells(self, blocking: torch.Tensor, radius: int, origins=None) -> torch.Tensor:
+    """visible_cells over this map's grid (not in the reference).  `origins` defaults to the agent's cell as
+    get_camera() defines it, computed on the host from the projector as for geodesic_distance, so the call does not
+    sync: the region the agent sees from where it stands, (b, 1, 2r + 1, 2r + 1)."""
+    if origins is None:
+      origins = _camera_cells(self.proj, _sight_grid(blocking)[0])
+    return visible_cells(blocking, origins, radius)
+
+  def count_visible(self, blocking: torch.Tensor, targets: torch.Tensor, radius: int, origins=None) -> torch.Tensor:
+    """count_visible over this map's grid (not in the reference).  `origins` defaults to the agent's cell as in
+    visible_cells: (b, 1), or (b, C, 1) for 4-D targets."""
+    if origins is None:
+      origins = _camera_cells(self.proj, _sight_grid(blocking)[0])
+    return count_visible(blocking, targets, origins, radius)
+
   def merge(self, *sources: List["TopdownMap"]) -> "TopdownMap":
     raise NotImplementedError
 
@@ -1111,6 +1127,31 @@ def _geodesic_grid(traversable) -> Tuple[int, int, int]:
   return b, H, W
 
 
+def _cells(cells, b: int, what: str, alternative: str = "") -> torch.Tensor:
+  """Integer cells [x, z] of shape (b, n, 2) or (b, 2) as a (b, n, 2) tensor where they are, checked in every respect
+  but their device."""
+  t = cells if torch.is_tensor(cells) else torch.from_numpy(np.asarray(cells))
+  if t.dtype is torch.bool or t.is_floating_point() or t.is_complex():
+    raise ValueError(f"{what} must be integers{alternative}, got {t.dtype}")
+  if t.dim() == 2:
+    t = t.unsqueeze(1)
+  if t.dim() != 3 or t.shape[0] != b or t.shape[2] != 2 or t.shape[1] < 1:
+    raise ValueError(f"{what} must be ({b}, n, 2) with n >= 1 or ({b}, 2), got {tuple(cells.shape)}")
+  return t
+
+
+def _device_cells(cells: torch.Tensor, dev: torch.device, what: str) -> torch.Tensor:
+  """Contiguous int64 cells on `dev`.  Host cells go through the parameter ring, or a pinned non-blocking copy when
+  larger: no host sync."""
+  if cells.is_cuda and cells.device != dev:
+    raise ValueError(f"the {what} must be on {dev} or the host, got {cells.device}")
+  cells = cells.to(torch.int64).contiguous()
+  if not cells.is_cuda:
+    cells = prm.upload(cells, dev) if cells.numel() * 8 <= prm._UPLOAD_MAX else \
+        cells.pin_memory().to(dev, non_blocking=True)
+  return cells
+
+
 def geodesic_distance(traversable: torch.Tensor, sources) -> torch.Tensor:
   """Shortest-path distance, through traversable cells, from the sources of each environment to every cell of its map
   (not in the reference): the distance field a planner steps down, on the device, for a whole batch at once.
@@ -1142,27 +1183,16 @@ def geodesic_distance(traversable: torch.Tensor, sources) -> torch.Tensor:
                        f"{tuple(sources.shape)}")
     mask = sources
   else:
-    cells = sources if torch.is_tensor(sources) else torch.from_numpy(np.asarray(sources))
-    if cells.dtype is torch.bool or cells.is_floating_point() or cells.is_complex():
-      raise ValueError(f"source cells must be integers (or a bool mask), got {cells.dtype}")
-    if cells.dim() == 2:
-      cells = cells.unsqueeze(1)
-    if cells.dim() != 3 or cells.shape[0] != b or cells.shape[2] != 2 or cells.shape[1] < 1:
-      raise ValueError(f"source cells must be ({b}, n, 2) with n >= 1 or ({b}, 2), got {tuple(sources.shape)}")
+    cells = _cells(sources, b, "source cells", " (or a bool mask)")
   dev = traversable.device
   if not traversable.is_cuda:
     raise ValueError(f"traversable must be on a CUDA device, got {dev}")
   if mask is not None and mask.device != dev:
     raise ValueError(f"the source mask must be on {dev}, got {mask.device}")
-  if cells is not None and cells.is_cuda and cells.device != dev:
-    raise ValueError(f"the source cells must be on {dev} or the host, got {cells.device}")
   n = 0
   if cells is not None:
     n = cells.shape[1]
-    cells = cells.to(torch.int64).contiguous()
-    if not cells.is_cuda:
-      cells = prm.upload(cells, dev) if cells.numel() * 8 <= prm._UPLOAD_MAX else \
-          cells.pin_memory().to(dev, non_blocking=True)
+    cells = _device_cells(cells, dev, "source cells")
   trav = traversable.reshape(b, H, W).contiguous()
   mask = None if mask is None else mask.reshape(b, H, W).contiguous()
   out = torch.empty((b, H, W), dtype=torch.int32, device=dev)
@@ -1291,6 +1321,136 @@ def distance_transform(mask: torch.Tensor, return_indices: bool = False):
                                              nat.ptr(nearest), nat.stream_ptr(dev))
   nat.check(rc, "dm_distance_transform_f32")
   return (dist, nearest) if return_indices else dist
+
+
+def _sight_grid(blocking) -> Tuple[int, int, int]:
+  """(b, H, W) of a blocking grid, checked in every respect but its size and device."""
+  if not torch.is_tensor(blocking) or blocking.dtype is not torch.bool:
+    raise ValueError("blocking must be a bool tensor, got "
+                     f"{blocking.dtype if torch.is_tensor(blocking) else type(blocking).__name__}")
+  if not (blocking.dim() == 3 or (blocking.dim() == 4 and blocking.shape[1] == 1)):
+    raise ValueError(f"blocking must be (b, H, W) or (b, 1, H, W), got {tuple(blocking.shape)}")
+  b, H, W = blocking.shape[0], blocking.shape[-2], blocking.shape[-1]
+  if b < 1 or H < 1 or W < 1:
+    raise ValueError(f"blocking must not be empty, got {tuple(blocking.shape)}")
+  return b, H, W
+
+
+def _sight_args(blocking, origins, radius, targets=None):
+  """Checked (blocking, targets, origins) as contiguous device tensors, and (b, C, n, H, W, radius)."""
+  b, H, W = _sight_grid(blocking)
+  if isinstance(radius, bool) or not isinstance(radius, (int, np.integer)) or not 0 <= radius <= 512:
+    raise ValueError(f"radius must be an int from 0 to 512 cells, got {radius!r}")
+  radius = int(radius)
+  cells = _cells(origins if torch.is_tensor(origins) else np.asarray(origins), b, "origins")
+  n, C = cells.shape[1], 0
+  if targets is not None:
+    if not torch.is_tensor(targets) or targets.dtype is not torch.bool:
+      raise ValueError("targets must be a bool tensor, got "
+                       f"{targets.dtype if torch.is_tensor(targets) else type(targets).__name__}")
+    if targets.dim() not in (3, 4):
+      raise ValueError(f"targets must be (b, H, W) or (b, C, H, W), got {tuple(targets.shape)}")
+    C = targets.shape[1] if targets.dim() == 4 else 1
+    if targets.shape[0] != b or tuple(targets.shape[-2:]) != (H, W) or C < 1:
+      raise ValueError(f"targets must be ({b}, [C,] {H}, {W}) like blocking, got {tuple(targets.shape)}")
+  for what, size in (("b * n", b * n), ("H * W", H * W), ("b * C * H * W", b * C * H * W)):
+    if size >= 2 ** 31:
+      raise ValueError(f"{what} = {size} is too large: it must stay below 2^31")
+  dev = blocking.device
+  if not blocking.is_cuda:
+    raise ValueError(f"blocking must be on a CUDA device, got {dev}")
+  if targets is not None and targets.device != dev:
+    raise ValueError(f"targets must be on {dev}, got {targets.device}")
+  cells = _device_cells(cells, dev, "origins")
+  tg = None if targets is None else targets.reshape(b, C, H, W).contiguous()
+  return blocking.reshape(b, H, W).contiguous(), tg, cells, (b, C, n, H, W, radius)
+
+
+def visible_cells(blocking: torch.Tensor, origins, radius: int) -> torch.Tensor:
+  """What can be seen from each of n cells of every environment within `radius` cells (not in the reference): the
+  visible region around the agent, for rewards and policy inputs, on the device for a whole batch at once.
+
+  blocking: CUDA bool (b, H, W) or (b, 1, H, W), the cells that block sight; non-contiguous views (world.mask[:, 0])
+  are made contiguous.  origins: integer cells [x, z] of shape (b, n, 2), or (b, 2) for n = 1 (the n dimension is
+  kept), on blocking's device or on the host (host cells are uploaded through the parameter ring, or a pinned
+  non-blocking copy when larger).  radius: an int from 0 to 512, in cells.
+  Returns bool (b, n, 2 * radius + 1, 2 * radius + 1): out[i, k, radius + dz, radius + dx] is True iff cell
+  origins[i, k] + (dx, dz) is visible; window cells outside the disk or the map are False.
+
+  Definition, exact and integer, in cells [x, z] = [column, row] (the convention of get_camera / get_coords /
+  geodesic_distance; map_res and flip_h play no part).  For an origin o = (ox, oz) and a target t = (ox + dx, oz + dz),
+  with ax = |dx|, az = |dz|, m = max(ax, az) and sx, sz the signs of dx and dz, the line is the cells p_i, i = 0..m:
+      p_i = (ox + sx * i, oz + sz * floor((2 * i * az + m) / (2 * m)))   when ax >= az,
+  and the same with the axes swapped otherwise (m = 0: just o).  That is Bresenham with halves rounded away from the
+  origin; p_0 = o, p_m = t, and each step moves the minor coordinate by at most 1.  t is visible from o when
+    1. dx^2 + dz^2 <= radius^2;
+    2. t lies inside the H x W map;
+    3. no intermediate cell p_i, 0 < i < m, is blocking;
+    4. no corner leak: for no diagonal step p_i -> p_i+1 are both side cells (x_i+1, z_i) and (x_i, z_i+1) blocking.
+  The origin and the target never block: a wall cell is itself visible (so a goal's class-plane cells count as seen),
+  and an agent standing on an inflated obstacle still sees around it.  Rule 4 is geodesic_distance's "no corner
+  cutting": without it, sight slips between the cells of a diagonal wall that touch only at a corner, which is how depth
+  projection draws diagonal walls.  An origin outside the map sees nothing.
+
+  Visible region of a height world map `m` of a MapBuilder, unknown cells letting sight through (the optimistic
+  choice; `obstacle | ~seen` gives the pessimistic one):
+    obstacle = m.mask[:, 0] & (m.height_map[:, 0] > obstacle_height)
+    window = m.visible_cells(obstacle, r)                        # (b, 1, 2r + 1, 2r + 1) around the agent's cell
+
+  One library call on the current stream (csrc/dm_visibility.cu, one kernel) and no host sync; blocking and origins are
+  never written.  ValueError, before any device work, for a blocking that is not a bool (b, H, W) or (b, 1, H, W)
+  tensor or is empty, origins not integer (b, n, 2) or (b, 2) with n >= 1, a radius that is not an int from 0 to 512,
+  b * n or H * W of 2^31 or more, a blocking off CUDA and origins on another CUDA device."""
+  blk, _, cells, (b, _, n, H, W, radius) = _sight_args(blocking, origins, radius)
+  side = 2 * radius + 1
+  dev = blk.device
+  out = torch.empty((b, n, side, side), dtype=torch.bool, device=dev)
+  with torch.cuda.device(dev):
+    rc = nat.lib().dm_line_of_sight_u8(blk.data_ptr(), b, H, W, cells.data_ptr(), n, radius, out.data_ptr(), None, 0,
+                                       None, nat.stream_ptr(dev))
+  nat.check(rc, "dm_line_of_sight_u8")
+  return out
+
+
+def count_visible(blocking: torch.Tensor, targets: torch.Tensor, origins, radius: int) -> torch.Tensor:
+  """How many cells of each target plane can be seen from each of n cells of every environment within `radius` cells
+  (not in the reference): a line-of-sight goal check, and the exploration utility of candidate viewpoints, on the
+  device for a whole batch at once.
+
+  blocking, origins, radius: as in visible_cells.  targets: CUDA bool (b, H, W) or (b, C, H, W) on blocking's device
+  and grid; each plane is counted on its own.  Returns int32 (b, n) for 3-D targets and (b, C, n) for 4-D targets:
+      count[i, c, k] = #{visible t from origins[i, k] : targets[i, c, t]}
+  which is (visible_cells(blocking, origins, radius) & the targets' windows).sum(), without the window in memory.
+  Visibility is exactly visible_cells': integer lines from the origin, no corner leak, counts compared bit for bit.
+
+  Recipes for a height world map `m` of a MapBuilder, with obstacle = m.mask[:, 0] & (m.height_map[:, 0] > h).  Unknown
+  cells let sight through in both, the optimistic choice; `obstacle | ~m.mask[:, 0]` gives the pessimistic one.
+  - Object-goal stop check, a cell of the goal's class plane within 1 m and in line of sight of the agent:
+      near = m.count_visible(obstacle, goal_plane, round(1.0 / map_res))[:, 0] > 0        # (b,)
+  - Exploration utility (next-best view): the unknown cells n candidate viewpoints would reveal, weighed against the
+    geodesic distance to them, all on the device:
+      cands = m.get_camera()[:, None, :] + lattice.to(device)              # (b, n, 2); lattice: (n, 2) cell offsets
+      gain = count_visible(obstacle, ~m.mask[:, 0], cands, r)              # (b, n)
+      dist = m.geodesic_distance(free)                                     # (b, H, W), -1 where unreachable
+      H, W = dist.shape[-2:]
+      x, z = cands[..., 0], cands[..., 1]
+      inside = (x >= 0) & (x < W) & (z >= 0) & (z < H)
+      d = dist.flatten(1).gather(1, z.clamp(0, H - 1) * W + x.clamp(0, W - 1))
+      score = torch.where(inside & (d >= 0), gain - lam * d, float("-inf"))
+      best = score.argmax(-1)
+
+  One library call on the current stream (csrc/dm_visibility.cu, a memset of the counts and one kernel) and no host
+  sync; blocking, targets and origins are never written.  ValueError, before any device work, for the cases of
+  visible_cells, targets that are not a bool (b, H, W) or (b, C, H, W) tensor on blocking's grid and device, and
+  b * C * H * W of 2^31 or more."""
+  blk, tg, cells, (b, C, n, H, W, radius) = _sight_args(blocking, origins, radius, targets)
+  dev = blk.device
+  out = torch.empty((b, C, n), dtype=torch.int32, device=dev)
+  with torch.cuda.device(dev):
+    rc = nat.lib().dm_line_of_sight_u8(blk.data_ptr(), b, H, W, cells.data_ptr(), n, radius, None, tg.data_ptr(), C,
+                                       out.data_ptr(), nat.stream_ptr(dev))
+  nat.check(rc, "dm_line_of_sight_u8")
+  return out if targets.dim() == 4 else out.view(b, n)
 
 
 def _camera_cells(proj: MapProjector, b: int) -> torch.Tensor:

@@ -564,6 +564,26 @@ int dm_score_poses_i32(const uint8_t* planes, int32_t b, int32_t C, int32_t Hs, 
                        int32_t flip_h, const uint8_t* window, int32_t window_planes, int32_t h, int32_t w,
                        const float* samples, int32_t n, int32_t* scores, void* stream);
 
+/* visible_cells / count_visible: per-environment line of sight over masks from many origins (not in the reference).
+ * blocking (b, H, W) u8, nonzero = blocks sight; origins: device, (b, n, 2) int64 [x, z] = [column, row].  For origin
+ * o and target t = o + (dx, dz), with ax = |dx|, az = |dz|, m = max(ax, az) and sx, sz the signs of dx, dz, the line is
+ * the cells p_i, i = 0..m, p_i = (ox + sx * i, oz + sz * floor((2 * i * az + m) / (2 * m))) when ax >= az and the same
+ * with the axes swapped otherwise (p_0 = o, p_m = t).  t is visible from o when dx^2 + dz^2 <= radius^2, t is inside the
+ * map, no p_i with 0 < i < m is blocking, and for no diagonal step p_i -> p_i+1 both side cells (x_i+1, z_i) and
+ * (x_i, z_i+1) are blocking (no corner leak).  The origin and the target never block.  An origin outside the map sees
+ * nothing.  Exactly one output:
+ *   visible (b, n, 2r+1, 2r+1) u8: visible[i, k, r + dz, r + dx] = 1 iff o_ik + (dx, dz) is visible (targets NULL,
+ *           C 0), indexed in 64 bits;
+ *   counts  (b, C, n) int32: #{visible t : targets[i, c, t] != 0}, with targets (b, C, H, W) u8 and C >= 1.
+ * Exact integers.  One kernel on `stream` (a memset of counts before it in count mode), no host synchronisation;
+ * blocking, origins and targets are never written.  DM_EINVAL, before any CUDA call, for null blocking or origins, both
+ * outputs or neither, targets without counts or the reverse, C not >= 1 with counts or not 0 without, b, H, W or
+ * n <= 0, radius < 0 or > 512 (the staged window must fit in shared memory), and b * n, H * W or b * C * H * W of
+ * 2^31 or more. */
+int dm_line_of_sight_u8(const uint8_t* blocking, int32_t b, int32_t H, int32_t W, const int64_t* origins, int32_t n,
+                        int32_t radius, uint8_t* visible, const uint8_t* targets, int32_t C, int32_t* counts,
+                        void* stream);
+
 /* Library/ABI introspection. */
 int dm_abi_version(void);
 /* sizeof() of a struct of this header as the library was compiled, for bindings to check their mirror against:
