@@ -178,6 +178,8 @@ _SIGNATURES = {
   "dm_distance_transform_f32": (ctypes.c_int, [c_void_p, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p]),
   "dm_score_poses_i32": (ctypes.c_int, [c_void_p, c_int32, c_int32, c_int32, c_int32, c_float, c_int32, c_void_p,
                                         c_int32, c_int32, c_int32, c_void_p, c_int32, c_void_p, c_void_p]),
+  "dm_geodesic_path_i32": (ctypes.c_int, [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_void_p, c_int32, c_int32,
+                                          c_void_p, c_void_p, c_void_p]),
   "dm_line_of_sight_u8": (ctypes.c_int, [c_void_p, c_int32, c_int32, c_int32, c_void_p, c_int32, c_int32, c_void_p,
                                          c_void_p, c_int32, c_void_p, c_void_p]),
 }

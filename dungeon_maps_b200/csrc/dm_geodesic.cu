@@ -164,6 +164,83 @@ __global__ void __launch_bounds__(kGeoThreads) geodesic_kernel(const GeoArgs a) 
   for (long long i = gtid; i < total; i += gstride)
     if (__ldcg(a.dist + i) == kInf) a.dist[i] = -1;
 }
+
+// geodesic_path (dm_geodesic_path_i32): the walk down a field D from a start s.  p_0 = s when s is inside the map and
+// D[s] >= 0 (else the path is empty); while D[p_k] > 0 and k + 1 < max_cells, p_k+1 is the first neighbour
+// q = p_k + (dx, dz), in the order (+1, 0), (0, +1), (-1, 0), (0, -1), (+1, +1), (-1, +1), (-1, -1), (+1, -1), inside
+// the map with D[q] >= 0, D[q] == D[p_k] - cost and an edge q -> p_k under geodesic_kernel's rule (T[p_k], and for a
+// diagonal step T of both side cells).  D strictly decreases along the walk, so it ends for any int32 field.
+//
+// One warp per (environment, start).  Lanes 0..7 own the 8 neighbours in the definition's order and load D and T of
+// theirs together through the read-only path (consecutive steps share most of their 3 x 3 neighbourhood, so they
+// mostly hit L1); the first qualifying neighbour is the lowest set bit of a ballot.  Lane k % 32 keeps cell k, and
+// each group of 32 cells is stored as one coalesced 256-byte row; the warp then fills the rest of the path with -1.
+constexpr int kPathThreads = 256;
+constexpr int kPathWarps = kPathThreads / 32;
+
+struct PathArgs {
+  const uint8_t* trav;       // (b, H, W)
+  const int32_t* dist;       // (b, H, W)
+  const long long* starts;   // (b, n, 2) [x, z]
+  int H, W, n, max_cells;
+  long long paths;           // b * n
+  int2* cells;               // (b, n, max_cells) [x, z]
+  int32_t* lengths;          // (b, n)
+};
+
+__global__ void __launch_bounds__(kPathThreads) geodesic_path_kernel(const PathArgs a) {
+  const int lane = threadIdx.x & 31;
+  const long long path = (long long)blockIdx.x * kPathWarps + (threadIdx.x >> 5);
+  if (path >= a.paths) return;                             // uniform in the warp
+  // lane j < 8 owns the j-th neighbour of the order above; lanes >= 8 only store
+  const int dx = (lane == 0 || lane == 4 || lane == 7) ? 1 : (lane == 2 || lane == 5 || lane == 6) ? -1 : 0;
+  const int dz = (lane == 1 || lane == 4 || lane == 5) ? 1 : (lane == 3 || lane == 6 || lane == 7) ? -1 : 0;
+  const bool diag = dx != 0 && dz != 0;
+  const int32_t cost = diag ? kDiag : kOrtho;
+  // a diagonal step needs T of its side cells (q.x, p.z) = p + (dx, 0) and (p.x, q.z) = p + (0, dz): lanes 0 / 2, 1 / 3
+  const unsigned sides = diag ? (1u << (dx > 0 ? 0 : 2)) | (1u << (dz > 0 ? 1 : 3)) : 0u;
+  const size_t plane = (size_t)(path / a.n) * a.H * a.W;
+  const int32_t* D = a.dist + plane;
+  const uint8_t* T = a.trav + plane;
+  int2* out = a.cells + path * a.max_cells;
+  const long long sx = a.starts[2 * path], sz = a.starts[2 * path + 1];
+  int len = 0;
+  const bool inside = sx >= 0 && sx < a.W && sz >= 0 && sz < a.H;
+  int32_t d = inside ? __ldg(D + sz * a.W + sx) : -1;
+  if (d >= 0) {
+    int x = (int)sx, z = (int)sz;
+    bool t = __ldg(T + sz * a.W + sx) != 0;
+    int2 mine = make_int2(-1, -1);                         // cell k of the walk, k % 32 == lane
+    int k = 0;
+    for (;;) {
+      if (lane == (k & 31)) mine = make_int2(x, z);
+      if ((k & 31) == 31) out[k - 31 + lane] = mine;
+      if (d == 0 || k + 1 >= a.max_cells || !t) break;     // a source, the capacity, or no edge into p_k
+      const int qx = x + dx, qz = z + dz;
+      int32_t dq = -1;
+      bool tq = false;
+      if (lane < 8 && qx >= 0 && qx < a.W && qz >= 0 && qz < a.H) {
+        const size_t g = (size_t)qz * a.W + qx;
+        dq = __ldg(D + g);
+        tq = __ldg(T + g) != 0;
+      }
+      const unsigned tb = __ballot_sync(0xffffffffu, tq);
+      const bool ok = dq >= 0 && dq == d - cost && (tb & sides) == sides;   // d > 0: d - cost cannot overflow
+      const unsigned win = __ballot_sync(0xffffffffu, ok);
+      if (!win) break;
+      const int w = __ffs(win) - 1;
+      x = __shfl_sync(0xffffffffu, qx, w);
+      z = __shfl_sync(0xffffffffu, qz, w);
+      d = __shfl_sync(0xffffffffu, dq, w);
+      t = (tb >> w) & 1u;
+      ++k;
+    }
+    len = k + 1;
+    if ((k & 31) != 31 && lane <= (k & 31)) out[(k & ~31) + lane] = mine;
+  }
+  for (long long i = len + lane; i < a.max_cells; i += 32) out[i] = make_int2(-1, -1);
+  if (lane == 0) a.lengths[path] = len;
+}
 }  // namespace
 }  // namespace dm
 
@@ -211,6 +288,32 @@ extern "C" int dm_geodesic_distance_i32(const uint8_t* traversable, const uint8_
                                                     dim3(kGeoThreads), params, 0, stream);
   DM_CUDA_OK(cudaFreeAsync(scratch, stream));
   DM_CUDA_OK(e);
+  DM_LAUNCHED();
+  return DM_OK;
+}
+
+extern "C" int dm_geodesic_path_i32(const uint8_t* traversable, const int32_t* dist, int32_t b, int32_t H, int32_t W,
+                                    const int64_t* starts, int32_t n, int32_t max_cells, int32_t* cells,
+                                    int32_t* lengths, void* stream_) {
+  DM_TRACE();
+  if (!traversable || !dist || !starts || !cells || !lengths) return DM_EINVAL;
+  if (b <= 0 || H <= 0 || W <= 0 || n <= 0) return DM_EINVAL;
+  const long long HW = (long long)H * W, paths = (long long)b * n;
+  if (HW >= (1ll << 31) || paths >= (1ll << 31)) return DM_EINVAL;
+  if (max_cells < 1 || max_cells > HW) return DM_EINVAL;
+  PathArgs a;
+  a.trav = traversable;
+  a.dist = dist;
+  a.starts = reinterpret_cast<const long long*>(starts);
+  a.H = H;
+  a.W = W;
+  a.n = n;
+  a.max_cells = max_cells;
+  a.paths = paths;
+  a.cells = reinterpret_cast<int2*>(cells);
+  a.lengths = lengths;
+  const long long blocks = (paths + kPathWarps - 1) / kPathWarps;
+  geodesic_path_kernel<<<(unsigned)blocks, kPathThreads, 0, static_cast<cudaStream_t>(stream_)>>>(a);
   DM_LAUNCHED();
   return DM_OK;
 }

@@ -43,7 +43,8 @@ __all__ = [
   'height_map_to_point_cloud', 'image_to_camera_space', 'camera_to_image_space', 'camera_to_local_space',
   'local_to_camera_space', 'local_to_global_space', 'global_to_local_space', 'map_quantize',
   'map_dequantize', 'project', 'compute_center_offsets', 'MapProjector', 'TopdownMap', 'crop_topdown_map',
-  'crop_egocentric_map', 'score_poses', 'geodesic_distance', 'connected_components', 'distance_transform',
+  'crop_egocentric_map', 'score_poses', 'geodesic_distance', 'geodesic_path', 'connected_components',
+  'distance_transform',
   'visible_cells', 'count_visible', 'fuse_topdown_maps',
   'merge_into_canvas', 'MapBuilder', 'release_workspaces', 'Reduction', 'CameraIntrinsics', 'NINF', 'Float3D',
 ]
@@ -859,6 +860,14 @@ class TopdownMap():
       sources = _camera_cells(self.proj, _geodesic_grid(traversable)[0])
     return geodesic_distance(traversable, sources)
 
+  def geodesic_path(self, traversable: torch.Tensor, dist: torch.Tensor, max_cells: int, starts=None):
+    """geodesic_path over this map's grid (not in the reference).  `starts` defaults to the agent's cell as
+    get_camera() defines it, computed on the host from the projector as for geodesic_distance, so the call does not
+    sync: the path from where the agent stands to the nearest goal of `dist`, (b, 1, max_cells, 2) and (b, 1)."""
+    if starts is None:
+      starts = _camera_cells(self.proj, _geodesic_grid(traversable)[0])
+    return geodesic_path(traversable, dist, starts, max_cells)
+
   def visible_cells(self, blocking: torch.Tensor, radius: int, origins=None) -> torch.Tensor:
     """visible_cells over this map's grid (not in the reference).  `origins` defaults to the agent's cell as
     get_camera() defines it, computed on the host from the projector as for geodesic_distance, so the call does not
@@ -1201,6 +1210,91 @@ def geodesic_distance(traversable: torch.Tensor, sources) -> torch.Tensor:
                                             out.data_ptr(), nat.stream_ptr(dev))
   nat.check(rc, "dm_geodesic_distance_i32")
   return out
+
+
+def geodesic_path(traversable: torch.Tensor, dist: torch.Tensor, starts, max_cells: int):
+  """The cells from each of n start cells of every environment down a geodesic distance field to a goal (not in the
+  reference): the path a planner follows and, from it, the next waypoint, on the device for a whole batch at once.
+
+  traversable: CUDA bool (b, H, W) or (b, 1, H, W), the grid `dist` was computed over.  dist: int32 (b, H, W) or
+  (b, 1, H, W) on the same grid and device, normally geodesic_distance(traversable, goals).  Non-contiguous views are
+  made contiguous.  starts: integer cells [x, z] = [column, row] of shape (b, n, 2), or (b, 2) for n = 1 (the n
+  dimension is kept), on traversable's device or on the host (host cells are uploaded through the parameter ring, or a
+  pinned non-blocking copy when larger).  max_cells: an int from 1 to H * W, the capacity of each path, start included.
+  Returns (cells, lengths):
+  - cells: int32 (b, n, max_cells, 2), [x, z] (int32 like distance_transform's nearest); entries past a path's length
+    are -1;
+  - lengths: int32 (b, n), the number of cells written.
+
+  Definition, for start s of environment i, with D = dist[i] and T = traversable[i]:
+    1. If s lies outside the H x W map, or D[s] < 0, the path is empty (length 0).
+    2. Otherwise p_0 = s.  While D[p_k] > 0 and k + 1 < max_cells, let d = D[p_k].  Try the 8 neighbours
+       q = p_k + (dx, dz) in the fixed order (dx, dz) = (+1, 0), (0, +1), (-1, 0), (0, -1), (+1, +1), (-1, +1),
+       (-1, -1), (+1, -1).  The first q that meets all of these becomes p_k+1:
+       - q is inside the map;
+       - D[q] >= 0;
+       - D[q] == d - c, where c = 5 for an orthogonal step and 7 for a diagonal one;
+       - the edge q -> p_k exists under geodesic_distance's rule: T[p_k], and for a diagonal step also T[(q.x, p_k.z)]
+         and T[(p_k.x, q.z)] (no corner cutting).
+    3. The walk stops when D[p_k] == 0 (a source), when no neighbour qualifies, or when max_cells cells are written.
+  Consequences:
+  - D strictly decreases along a walk, so a walk always ends.  It visits distinct cells, at most
+    min(max_cells, D[s] / 5 + 1) of them, for any int32 input, including a dist that is not a distance field: a larger
+    max_cells than H * W is never needed.
+  - When dist is geodesic_distance(traversable, goals), step 2 always finds a neighbour.  The path is then a shortest
+    path to a goal: its step costs sum to D[s].
+  - Every cell except the last is traversable.  The last cell may be a goal on an obstacle, such as an object's class
+    plane.
+  - The path reached a goal iff lengths > 0 and D at its last cell is 0:
+      last = cells.gather(2, (lengths - 1).clamp(min=0).long()[..., None, None].expand(-1, -1, 1, 2))[:, :, 0]
+      reached = (lengths > 0) & (dist.flatten(1).gather(1, (last[..., 1] * W + last[..., 0]).clamp(min=0).long()) == 0)
+  - A start on a non-traversable cell has D = -1 (unless it is a goal), so its path is empty.  Snap it to the nearest
+    traversable cell first: _, nearest = distance_transform(~traversable, return_indices=True), and the start (x, z) of
+    environment i becomes nearest[i, z, x].
+
+  Waypoint recipe: the farthest path index j such that path cells 0..j all lie in the radius-r window around the start
+  and are visible from it, for (b, n, 2) device starts, with no host sync:
+    side = 2 * r + 1
+    vis = visible_cells(~traversable, starts, r).flatten(2)                  # (b, n, side * side)
+    rel = cells.long() - starts[:, :, None, :] + r                           # window [column, row] of each path cell
+    ok = ((rel >= 0) & (rel < side)).all(-1)
+    ok &= torch.arange(max_cells, device=cells.device) < lengths[..., None]
+    seen = vis.gather(2, (rel[..., 1] * side + rel[..., 0]).clamp(0, side * side - 1)) & ok
+    j = seen.int().cumprod(-1).sum(-1) - 1                                   # (b, n), -1 for an empty path
+    waypoint = cells.gather(2, j.clamp(min=0).long()[..., None, None].expand(-1, -1, 1, 2))[:, :, 0]
+
+  One library call on the current stream (csrc/dm_geodesic.cu, one kernel) and no host sync; traversable, dist and
+  starts are never written.  ValueError, before any device work, for a traversable geodesic_distance refuses, a dist
+  that is not an int32 tensor of traversable's grid, starts not integer (b, n, 2) or (b, 2) with n >= 1, a max_cells
+  that is not an int from 1 to H * W, b * n of 2^31 or more, a traversable off CUDA, and dist or starts on another CUDA
+  device."""
+  b, H, W = _geodesic_grid(traversable)
+  if not torch.is_tensor(dist) or dist.dtype is not torch.int32 or \
+      tuple(dist.shape) not in ((b, H, W), (b, 1, H, W)):
+    raise ValueError(f"dist must be an int32 tensor of traversable's grid, ({b}, {H}, {W}) or ({b}, 1, {H}, {W}), got "
+                     f"{f'{dist.dtype} {tuple(dist.shape)}' if torch.is_tensor(dist) else type(dist).__name__}")
+  cells = _cells(starts if torch.is_tensor(starts) else np.asarray(starts), b, "starts")
+  n = cells.shape[1]
+  if isinstance(max_cells, bool) or not isinstance(max_cells, (int, np.integer)) or not 1 <= max_cells <= H * W:
+    raise ValueError(f"max_cells must be an int from 1 to H * W = {H * W}, got {max_cells!r}")
+  max_cells = int(max_cells)
+  if b * n >= 2 ** 31:
+    raise ValueError(f"b * n = {b * n} is too large: it must stay below 2^31")
+  dev = traversable.device
+  if not traversable.is_cuda:
+    raise ValueError(f"traversable must be on a CUDA device, got {dev}")
+  if dist.device != dev:
+    raise ValueError(f"dist must be on {dev}, got {dist.device}")
+  cells = _device_cells(cells, dev, "starts")
+  trav = traversable.reshape(b, H, W).contiguous()
+  d = dist.reshape(b, H, W).contiguous()
+  out = torch.empty((b, n, max_cells, 2), dtype=torch.int32, device=dev)
+  lengths = torch.empty((b, n), dtype=torch.int32, device=dev)
+  with torch.cuda.device(dev):
+    rc = nat.lib().dm_geodesic_path_i32(trav.data_ptr(), d.data_ptr(), b, H, W, cells.data_ptr(), n, max_cells,
+                                        out.data_ptr(), lengths.data_ptr(), nat.stream_ptr(dev))
+  nat.check(rc, "dm_geodesic_path_i32")
+  return out, lengths
 
 
 def connected_components(mask: torch.Tensor, connectivity: int = 8, return_sizes: bool = False):

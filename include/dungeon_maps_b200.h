@@ -518,6 +518,28 @@ int dm_crop_egocentric_f32(const float* topdown, const float* height, int64_t he
 int dm_geodesic_distance_i32(const uint8_t* traversable, const uint8_t* source_mask, const int64_t* source_cells,
                              int32_t n_cells, int32_t b, int32_t H, int32_t W, int32_t* dist, void* stream);
 
+/* geodesic_path: per-environment paths from n start cells down a distance field (not in the reference).
+ * traversable (b, H, W) u8 0 / 1 and dist (b, H, W) int32, normally dm_geodesic_distance_i32's output over that grid;
+ * starts: device, (b, n, 2) int64 [x, z] = [column, row].  For start s of environment i, with D = dist[i] and
+ * T = traversable[i]:
+ *   1. if s lies outside the H x W map or D[s] < 0, the path is empty (length 0);
+ *   2. otherwise p_0 = s.  While D[p_k] > 0 and k + 1 < max_cells, with d = D[p_k], the 8 neighbours
+ *      q = p_k + (dx, dz) are tried in the fixed order (dx, dz) = (+1, 0), (0, +1), (-1, 0), (0, -1), (+1, +1),
+ *      (-1, +1), (-1, -1), (+1, -1), and the first q with all of: q inside the map; D[q] >= 0; D[q] == d - c, c = 5
+ *      for an orthogonal step and 7 for a diagonal one; the edge q -> p_k of dm_geodesic_distance_i32 (T[p_k], and for
+ *      a diagonal step T[(q.x, p_k.z)] and T[(p_k.x, q.z)]) becomes p_k+1;
+ *   3. the walk stops when D[p_k] == 0, when no neighbour qualifies, or when max_cells cells are written.
+ * D strictly decreases along a walk, so it ends and visits distinct cells, at most min(max_cells, D[s] / 5 + 1) of
+ * them, for any int32 dist.  When dist is the distance field of traversable, step 2 always finds a neighbour and the
+ * path is a shortest path to a source: its step costs sum to D[s].
+ * cells (b, n, max_cells, 2) int32 [x, z]: p_0 .. p_{len-1}, then -1, indexed in 64 bits; lengths (b, n) int32: len.
+ * Every entry of both is written.  Exact integers.  One kernel on `stream`, no scratch, no atomics, no host
+ * synchronisation; traversable, dist and starts are never written.  DM_EINVAL, before any CUDA call, for a null
+ * pointer, b, H, W or n <= 0, H * W or b * n of 2^31 or more, and max_cells < 1 or > H * W. */
+int dm_geodesic_path_i32(const uint8_t* traversable, const int32_t* dist, int32_t b, int32_t H, int32_t W,
+                         const int64_t* starts, int32_t n, int32_t max_cells, int32_t* cells, int32_t* lengths,
+                         void* stream);
+
 /* connected_components: per-plane connected-component labels of masks (not in the reference).
  * mask (n_planes, H, W) u8, nonzero = foreground; each H x W plane is labelled on its own.  connectivity 4 (orthogonal
  * neighbours) or 8 (orthogonal and diagonal neighbours, no corner rule).
